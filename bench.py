@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                     [--workload all|c2|c2big|c3|c4|c5|c5loop|entropy|collide|dwa] [--loop-steps L]
+                    [--dump-outputs DIR]
 
 One "step" = one batched ErgodicControl::control() iteration (ONE fused CUDA kernel) over the
 workload's instances.  The PRIMARY line (`value`) is BASELINE.json configs[1] ("c2": Omni, 10x10 basis,
@@ -23,6 +24,10 @@ Timing (N = world size, launched by torchrun: one process per GPU):
   * e2e: the same metric through the host-buffer entry points with pinned host memory, copies inside the
     timed region.  N > 1: pinned x -> H2D -> control + fused gather -> wait -> D2H of the GATHERED twists.
 --impl reference times the reference's own CPU implementation (oracle/_ref) on all host cores.
+--dump-outputs DIR writes what the primary workload's timed path returned in its last timed step: u0.npy (first
+twists), metric.npy and ut.npy (the warm-started control signals of the controller that step used), float64.  N > 1:
+u0 holds the gathered rows of every rank, metric and ut rank 0's rows.  The inputs are seeded, so two builds run with
+the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -302,6 +307,7 @@ class Ctx:
             self.clocks.start()
         self._flush = None
         self._peak64 = None
+        self.outputs = None  # --dump-outputs: the arrays bench_solve kept from its last timed step
         try:
             self.peaks = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))
         except Exception:
@@ -361,8 +367,9 @@ def fp64_roofline(ctx, F, solves_per_launch, k_ms, key, N, M, note=None):
     return r
 
 
-def bench_solve(ctx, key, steps, warmup, with_cpu=True):
-    """one batched control() per step over this rank's instances; returns the result dict (rank 0) or None"""
+def bench_solve(ctx, key, steps, warmup, with_cpu=True, keep_outputs=False):
+    """one batched control() per step over this rank's instances; returns the result dict (rank 0) or None.
+    keep_outputs: rank 0 keeps in ctx.outputs what the last step of the run `value` reports returned"""
     torch, dist, eb = ctx.torch, ctx.dist, ctx.eb
     wl = WORKLOADS[key]
     world, rank = ctx.world, ctx.rank
@@ -421,6 +428,10 @@ def bench_solve(ctx, key, steps, warmup, with_cpu=True):
     def launch_total():
         return sum(c_.launch_count() for c_ in ctls)
 
+    def last_step_outputs(u0):
+        # read before any untimed call reuses u0d / metd or steps the controller again
+        return {"u0": u0.cpu().numpy(), "metric": metd.cpu().numpy(), "ut": ctls[(steps - 1) % n_rot].get_ut()}
+
     W = max(3, warmup)
     for i in range(max(W, n_rot)):  # every batch has built its phi_k (first call) before the clock starts
         step_dev(i)
@@ -447,6 +458,8 @@ def bench_solve(ctx, key, steps, warmup, with_cpu=True):
     for c_ in ctls:
         c_.check()
     t_ms = ea.elapsed_time(eb_)
+    if keep_outputs and pg is None and rank == 0:
+        ctx.outputs = last_step_outputs(u0d)
 
     # N > 1, beside the strict number: the same K steps with the gather PIPELINED -- nothing in step i + 1 of a rank
     # depends on other ranks' rows (independent instances), so the solve of step i + 1 is launched while the rows of
@@ -474,6 +487,8 @@ def bench_solve(ctx, key, steps, warmup, with_cpu=True):
         for c_ in ctls:
             c_.check()
         pipe_ms = pa.elapsed_time(pb)
+        if keep_outputs and rank == 0:
+            ctx.outputs = last_step_outputs(pg.gathered())
 
     gather_ok = None
     if pg is not None:
@@ -1109,6 +1124,22 @@ def primary_line(res):
     return line
 
 
+DUMP_BYTES = 60 * 10**6  # a dump stays under 64 MB, .npy headers included
+
+
+def dump_outputs(path, arrays):
+    """<path>/<name>.npy in float64.  Beyond DUMP_BYTES in all, every array keeps the same fraction of its rows, a
+    seeded sorted sample: the same rows in every run of the same arguments, and the same rows of arrays of equal length
+    (u0, metric and ut of one instance stay together)."""
+    os.makedirs(path, exist_ok=True)
+    arrays = {name: np.asarray(a, dtype=np.float64) for name, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > DUMP_BYTES:
+            a = a[np.sort(np.random.default_rng(0).choice(len(a), len(a) * DUMP_BYTES // total, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def run_ours(args):
     ctx = Ctx(args)
     order = ["c2", "c3", "c4", "c5", "c5loop", "entropy"] if args.workload == "all" else [args.workload]
@@ -1126,7 +1157,8 @@ def run_ours(args):
             elif key == "entropy":
                 r = bench_entropy(ctx, max(args.steps, 100) if args.workload == "all" else args.steps, args.warmup)
             else:
-                r = bench_solve(ctx, key, args.steps, args.warmup)
+                r = bench_solve(ctx, key, args.steps, args.warmup,
+                                keep_outputs=args.dump_outputs is not None and key == order[0])
         except SystemExit:
             raise
         except Exception as exc:  # a secondary must not take the primary line down with it
@@ -1137,6 +1169,8 @@ def run_ours(args):
         ctx.torch.cuda.empty_cache()
     stress = peer_stress(ctx) if (ctx.world > 1 and args.workload == "all") else None
     if ctx.rank == 0:
+        if args.dump_outputs is not None:
+            dump_outputs(args.dump_outputs, ctx.outputs)
         line = primary_line(results[0])
         if stress is not None:
             line["peer_stress"] = stress
@@ -1244,7 +1278,12 @@ def main():
     ap.add_argument("--loop-steps", type=int, default=1000, help="ticks of the configs[4] closed loop")
     ap.add_argument("--workload", default="all",
                     choices=["all"] + sorted(WORKLOADS) + ["c3", "c5loop", "collide", "dwa", "entropy"])
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the primary workload's outputs of its last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs is not None and (args.impl != "ours" or args.workload not in ["all"] + sorted(WORKLOADS)):
+        ap.error("--dump-outputs needs the GPU arm with a control() workload as the primary: all, "
+                 + ", ".join(sorted(WORKLOADS)))
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.impl == "reference":

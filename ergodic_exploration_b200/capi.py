@@ -165,6 +165,12 @@ SIGNATURES = {
     "eb_map_target_extent": (C.c_int, [_vp, _dp, _dp]),
     "eb_map_target_launch_count": (C.c_longlong, [_vp]),
     "eb_set_phik_dev": (C.c_int, [_vp, _vp, C.c_double, C.c_double]),
+    "eb_set_target_gaussians_batch": (C.c_int, [_vp, C.c_int, _vp, _vp, _vp]),
+    "eb_set_phik_batch_dev": (C.c_int, [_vp, _vp, _vp]),
+    "eb_get_phik_batch": (C.c_int, [_vp, _vp, _vp]),
+    "eb_config_target_batch_dev": (C.c_int, [_vp, _vp, _vp]),
+    "eb_control_batch_dev": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp]),
+    "eb_control_batch_host": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp]),
     "eb_model_controls": (C.c_int, [C.c_int]),
     "eb_rk4_solve_host": (C.c_int, [C.c_int, C.c_int, _vp, C.c_double, C.c_double, _vp, _vp, C.c_int, C.c_int, _vp]),
     "eb_rk4_solve_dev": (C.c_int, [C.c_int, C.c_int, _vp, C.c_double, C.c_double, _vp, _vp, C.c_int, C.c_int, _vp, _vp, _vp]),

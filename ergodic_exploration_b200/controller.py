@@ -294,7 +294,13 @@ class ErgodicControl:
 
     def control(self, grid, x, mem_idx=None, u0=None, metric=None):
         """One control() iteration for all instances.  Returns u0 (B, 3); pass
-        ``metric`` (B,) to also receive sum_k lamda_k (c_k - phi_k)^2."""
+        ``metric`` (B,) to also receive sum_k lamda_k (c_k - phi_k)^2.
+
+        ``grid``: one map for the whole batch (bounds or an object with them), or per-instance
+        bounds (B, 4) {xmin, xmax, ymin, ymax} (array or CUDA tensor), or None on a per-instance
+        controller: the frames of the last configure, no frame launch."""
+        if grid is None or (type(grid) is not tuple and np.ndim(grid) == 2):
+            return self._control_batch(grid, x, mem_idx, u0, metric)
         if type(grid) is tuple:  # a control loop passes the same bounds tuple every tick
             b = grid
         else:
@@ -321,6 +327,91 @@ class ErgodicControl:
                 idx_p = mem_idx.ctypes.data
             met_p = self._host_ptr(metric) if metric is not None else None
             st = self._lib.eb_control_host(self._h, *b, self._host_ptr(x), idx_p, self._host_ptr(u0), met_p)
+        if st != capi.EB_OK:
+            if st == capi.EB_ERR_INVALID_ARGUMENT:
+                raise ValueError(self._lib.eb_last_error().decode())
+            check(st)
+        return u0
+
+    # -- per-instance targets (one target and map frame per instance) -------------------
+    def _bounds_dev(self, bounds):
+        b = torch.as_tensor(bounds, dtype=torch.float64, device=f"cuda:{self.device}").contiguous()
+        if tuple(b.shape) != (self.batch, 4):
+            raise ValueError(f"per-instance bounds must be ({self.batch}, 4), got {tuple(b.shape)}")
+        return b
+
+    def setTargets(self, targets) -> None:
+        """Target::setTarget per instance: ``targets`` holds B Targets (or lists of Gaussians).
+        Does not rebuild phi_k by itself (configTargets / control with bounds does)."""
+        if len(targets) != self.batch:
+            raise ValueError(f"setTargets needs {self.batch} targets, got {len(targets)}")
+        gss = [t.gaussians if isinstance(t, Target) else list(t) for t in targets]
+        counts = np.array([len(g) for g in gss], dtype=np.int32)
+        max_n = max(1, int(counts.max()))
+        mu = np.zeros((self.batch, max_n, 2))
+        sg = np.ones((self.batch, max_n, 2))
+        for i, g in enumerate(gss):
+            for j, gi in enumerate(g):
+                mu[i, j] = gi.mu
+                sg[i, j] = gi.sigmas
+        st = self._lib.eb_set_target_gaussians_batch(self._h, max_n, counts.ctypes.data, mu.ctypes.data, sg.ctypes.data)
+        if st == capi.EB_ERR_INVALID_ARGUMENT:
+            raise ValueError(self._lib.eb_last_error().decode())
+        check(st)
+
+    def configTargets(self, bounds) -> np.ndarray:
+        """configTarget of every instance, bounds (B, 4) {xmin, xmax, ymin, ymax}.  Returns rebuilt (B,) bool.
+        A moved extent without Gaussians surfaces from the next check()."""
+        self._sync_stream()
+        b = self._bounds_dev(bounds)
+        rebuilt = torch.zeros(self.batch, dtype=torch.int32, device=b.device)
+        check(self._lib.eb_config_target_batch_dev(self._h, C.c_void_p(b.data_ptr()), C.c_void_p(rebuilt.data_ptr())))
+        return rebuilt.cpu().numpy().astype(bool)
+
+    def set_phik_batch(self, phik, extent) -> None:
+        """phi_k rows (B, K) and extents (B, 2) {lx, ly}, CUDA tensors (e.g. MapTarget.execute outputs);
+        the origins of the frames are kept."""
+        self._sync_stream()
+        assert _is_cuda_tensor(phik) and _is_cuda_tensor(extent), "set_phik_batch takes CUDA tensors"
+        assert phik.dtype == torch.float64 and phik.is_contiguous() and phik.numel() == self.batch * self.num_coeff
+        assert extent.dtype == torch.float64 and extent.is_contiguous() and extent.numel() == 2 * self.batch
+        check(self._lib.eb_set_phik_batch_dev(self._h, C.c_void_p(phik.data_ptr()), C.c_void_p(extent.data_ptr())))
+
+    def get_phik_batch(self):
+        """(phik (B, K), extent (B, 2)) of a per-instance controller"""
+        ph = np.empty((self.batch, self.num_coeff))
+        ext = np.empty((self.batch, 2))
+        st = self._lib.eb_get_phik_batch(self._h, ph.ctypes.data, ext.ctypes.data)
+        if st == capi.EB_ERR_INVALID_ARGUMENT:
+            raise ValueError(self._lib.eb_last_error().decode())
+        check(st)
+        return ph, ext
+
+    def _control_batch(self, bounds, x, mem_idx, u0, metric):
+        if _is_cuda_tensor(x):
+            self._sync_stream()
+            assert x.dtype == torch.float64 and x.is_contiguous() and x.numel() == 3 * self.batch
+            b = self._bounds_dev(bounds) if bounds is not None else None
+            if u0 is None:
+                u0 = torch.empty((self.batch, 3), dtype=torch.float64, device=x.device)
+            st = self._lib.eb_control_batch_dev(
+                self._h, C.c_void_p(b.data_ptr()) if b is not None else None, C.c_void_p(x.data_ptr()),
+                C.c_void_p(mem_idx.data_ptr()) if mem_idx is not None else None, C.c_void_p(u0.data_ptr()),
+                C.c_void_p(metric.data_ptr()) if metric is not None else None)
+        else:
+            x = _np_f64(x).reshape(self.batch, 3)
+            b = None
+            if bounds is not None:
+                b = bounds.cpu().numpy() if _is_cuda_tensor(bounds) else bounds
+                b = _np_f64(b, (self.batch, 4))
+            if u0 is None:
+                u0 = np.empty((self.batch, 3))
+            idx_p = None
+            if mem_idx is not None:
+                mem_idx = np.ascontiguousarray(mem_idx, dtype=np.int32)
+                idx_p = mem_idx.ctypes.data
+            st = self._lib.eb_control_batch_host(self._h, b.ctypes.data if b is not None else None, x.ctypes.data,
+                                                 idx_p, u0.ctypes.data, metric.ctypes.data if metric is not None else None)
         if st != capi.EB_OK:
             if st == capi.EB_ERR_INVALID_ARGUMENT:
                 raise ValueError(self._lib.eb_last_error().decode())

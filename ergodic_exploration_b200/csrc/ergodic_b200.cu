@@ -31,6 +31,7 @@
 #include "solve_kernel.cuh"
 #include "solve_kernel_v2.cuh"
 #include "solve_kernel_big.cuh"
+#include "target_batch.cuh"
 
 namespace
 {
@@ -570,6 +571,16 @@ struct eb_controller
   bool have_pose = false;
   bool keep_ck = true;  // store the c_k by-product of every control() (eb_get_ck)
   const struct PeerLaunch* peer = nullptr;  // set for the duration of eb_control_dev_gather
+  // per-instance targets (eb_*_batch calls): switched on by the first of them; the shared target calls refuse after it.
+  // Every stored row's cosines (d_hist_cos) are then kept valid for its instance's current frame.
+  bool per_inst = false;
+  bool frames_set = false;          // a configure or eb_set_phik_batch_dev has given every instance a frame
+  double* d_phik_b = nullptr;       // [B][K]
+  double* d_frames = nullptr;       // [B][eb::kFrDoubles]
+  double *d_gmu = nullptr, *d_gsig = nullptr;  // [B][gmax][2]
+  int* d_gcount = nullptr;          // [B]
+  int gmax = 0;
+  double* d_bounds = nullptr;       // [B][4] staging of eb_control_batch_host
 
   // device alias of a page-locked host buffer (nullptr for pageable memory);
   // looked up on every call -- a cached answer could outlive the allocation
@@ -631,7 +642,7 @@ inline bool use_v2(int nb)
   return !v1 && nb > (small ? 8 : 12) && nb <= 24;
 }
 
-template <int MODEL, int NB, bool V2>
+template <int MODEL, int NB, bool V2, bool PER_INST = false>
 struct SolveLaunch
 {
   static constexpr int kWide = []() constexpr {
@@ -657,9 +668,9 @@ struct SolveLaunch
     cudaGetDevice(&dev);
     auto kernel = [] {
       if constexpr (V2)
-        return eb::solve_kernel2<MODEL, NB, WARPS>;
+        return eb::solve_kernel2<MODEL, NB, WARPS, PER_INST>;
       else
-        return eb::solve_kernel<MODEL, NB, WARPS>;
+        return eb::solve_kernel<MODEL, NB, WARPS, PER_INST>;
     }();
     if (bytes > configured[dev & 63])
     {
@@ -715,7 +726,7 @@ struct SolveLaunch
 };
 
 // num_basis > 32: a CTA per instance (solve_kernel_big.cuh), persistent over the batch; one scratch row per CTA
-template <int MODEL>
+template <int MODEL, bool PER_INST>
 cudaError_t launch_solve_big(const eb::SolveParams& p, cudaStream_t s)
 {
   const size_t bytes = eb::solve_big_smem_bytes(p.nb, p.N);
@@ -724,13 +735,13 @@ cudaError_t launch_solve_big(const eb::SolveParams& p, cudaStream_t s)
   cudaGetDevice(&dev);
   if (bytes > configured[dev & 63])
   {
-    cudaError_t e = cudaFuncSetAttribute(eb::solve_kernel_big<MODEL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    cudaError_t e = cudaFuncSetAttribute(eb::solve_kernel_big<MODEL, PER_INST>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
     if (e != cudaSuccess) return e;
     configured[dev & 63] = bytes;
   }
   if (!p.big_scratch || p.big_rows < 1) return cudaErrorInvalidValue;
   const int grid = std::min(p.B, p.big_rows);
-  eb::solve_kernel_big<MODEL><<<grid, eb::kBigThreads, bytes, s>>>(p, p.big_scratch);
+  eb::solve_kernel_big<MODEL, PER_INST><<<grid, eb::kBigThreads, bytes, s>>>(p, p.big_scratch);
   return cudaGetLastError();
 }
 
@@ -750,26 +761,26 @@ int solve_big_resident(int nb, int N)
   return sms * std::max(1, per_sm);
 }
 
-template <int MODEL>
+template <int MODEL, bool PER_INST>
 cudaError_t launch_solve_m(const eb::SolveParams& p, int rounds, cudaStream_t s)
 {
   const int nb = p.nb;
-  if (nb > 32) return launch_solve_big<MODEL>(p, s);
-  if (nb <= 8) return SolveLaunch<MODEL, 8, false>::launch(p, rounds, s);
+  if (nb > 32) return launch_solve_big<MODEL, PER_INST>(p, s);
+  if (nb <= 8) return SolveLaunch<MODEL, 8, false, PER_INST>::launch(p, rounds, s);
   if (nb <= 12 && use_v2(nb))
-    return nb <= 10 ? SolveLaunch<MODEL, 10, true>::launch(p, rounds, s) : SolveLaunch<MODEL, 12, true>::launch(p, rounds, s);
-  if (nb <= 10) return SolveLaunch<MODEL, 10, false>::launch(p, rounds, s);
-  if (nb <= 12) return SolveLaunch<MODEL, 12, false>::launch(p, rounds, s);
+    return nb <= 10 ? SolveLaunch<MODEL, 10, true, PER_INST>::launch(p, rounds, s) : SolveLaunch<MODEL, 12, true, PER_INST>::launch(p, rounds, s);
+  if (nb <= 10) return SolveLaunch<MODEL, 10, false, PER_INST>::launch(p, rounds, s);
+  if (nb <= 12) return SolveLaunch<MODEL, 12, false, PER_INST>::launch(p, rounds, s);
   if (use_v2(nb))
   {
-    if (nb <= 16) return SolveLaunch<MODEL, 16, true>::launch(p, rounds, s);
-    if (nb <= 20) return SolveLaunch<MODEL, 20, true>::launch(p, rounds, s);
-    return SolveLaunch<MODEL, 24, true>::launch(p, rounds, s);
+    if (nb <= 16) return SolveLaunch<MODEL, 16, true, PER_INST>::launch(p, rounds, s);
+    if (nb <= 20) return SolveLaunch<MODEL, 20, true, PER_INST>::launch(p, rounds, s);
+    return SolveLaunch<MODEL, 24, true, PER_INST>::launch(p, rounds, s);
   }
-  if (nb <= 16) return SolveLaunch<MODEL, 16, false>::launch(p, rounds, s);
-  if (nb <= 20) return SolveLaunch<MODEL, 20, false>::launch(p, rounds, s);
-  if (nb <= 24) return SolveLaunch<MODEL, 24, false>::launch(p, rounds, s);
-  return SolveLaunch<MODEL, 32, false>::launch(p, rounds, s);
+  if (nb <= 16) return SolveLaunch<MODEL, 16, false, PER_INST>::launch(p, rounds, s);
+  if (nb <= 20) return SolveLaunch<MODEL, 20, false, PER_INST>::launch(p, rounds, s);
+  if (nb <= 24) return SolveLaunch<MODEL, 24, false, PER_INST>::launch(p, rounds, s);
+  return SolveLaunch<MODEL, 32, false, PER_INST>::launch(p, rounds, s);
 }
 
 // dynamic shared memory of the solve kernel instantiation that serves `nb` (same dispatch as launch_solve_m)
@@ -792,10 +803,14 @@ size_t solve_smem_for(int nb, int N)
   return SolveLaunch<0, 32, false>::smem(N);
 }
 
-cudaError_t launch_solve(const eb::SolveParams& p, int model, int rounds, cudaStream_t s)
+// per_inst: the kernels read each instance's frame and phi_k row (p.frames, p.phik [B][K])
+cudaError_t launch_solve(const eb::SolveParams& p, int model, int rounds, cudaStream_t s, bool per_inst)
 {
-  return model == EB_MODEL_OMNI ? launch_solve_m<eb::kModelOmni>(p, rounds, s) :
-                                  launch_solve_m<eb::kModelSimpleCart>(p, rounds, s);
+  if (per_inst)
+    return model == EB_MODEL_OMNI ? launch_solve_m<eb::kModelOmni, true>(p, rounds, s) :
+                                    launch_solve_m<eb::kModelSimpleCart, true>(p, rounds, s);
+  return model == EB_MODEL_OMNI ? launch_solve_m<eb::kModelOmni, false>(p, rounds, s) :
+                                  launch_solve_m<eb::kModelSimpleCart, false>(p, rounds, s);
 }
 
 eb_status ensure_hist(eb_controller* c, long long need)
@@ -820,7 +835,21 @@ eb_status ensure_hist(eb_controller* c, long long need)
   cudaFree(c->d_hist);
   c->d_hist = nh;
   c->hist_cap = cap;
-  if (replay_cos_cache())
+  if (replay_cos_cache() && c->per_inst)
+  {
+    // per-instance frames: the rows are kept valid as they are written, so they move with the buffer
+    double* nc = nullptr;
+    EB_CUDA(cudaMalloc(&nc, sizeof(double) * 2 * (size_t)c->B * (size_t)cap));
+    if (c->mem_count > 0 && c->d_hist_cos)
+    {
+      EB_CUDA(cudaMemcpyAsync(nc, c->d_hist_cos, sizeof(double) * 2 * (size_t)c->B * (size_t)c->mem_count,
+                              cudaMemcpyDeviceToDevice, c->stream));
+      EB_CUDA(cudaStreamSynchronize(c->stream));
+    }
+    cudaFree(c->d_hist_cos);
+    c->d_hist_cos = nc;
+  }
+  else if (replay_cos_cache())
   {
     cudaFree(c->d_hist_cos);  // re-derived from the rows on the next control() (cos_count = 0)
     c->d_hist_cos = nullptr;
@@ -863,8 +892,62 @@ eb_status check_fault(eb_controller* c)
     if (f & 2)  // buffer.cpp:84,103: memory_.at(i) throws std::out_of_range
       return fail(EB_ERR_OUT_OF_RANGE, "replay-buffer sample index outside [0, stored states)");
     if (f & 4) return fail(EB_ERR_CUDA, "control(): non-finite state or control signal (NaN / Inf guard)");
+    if (f & eb::kFaultTarget)
+      return fail(EB_ERR_INVALID_ARGUMENT, "per-instance target: an instance's map extent changed but it has no "
+                                           "Gaussians (eb_set_target_gaussians_batch), or its extent is not positive");
     return fail(EB_ERR_INVALID_ARGUMENT, "Invalid twist y-velocity must be 0.");  // cart.hpp:169
   }
+  return EB_OK;
+}
+
+// the shared target calls on a controller that holds per-instance targets
+eb_status refuse_per_inst(const char* call)
+{
+  return fail(EB_ERR_INVALID_ARGUMENT, std::string(call) + ": the controller holds one target per instance (it has "
+                                                           "taken an eb_*_batch target call); use the _batch calls");
+}
+
+// first per-instance call: phi_k rows and frames (all zero: lx = ly = 0, so the first configure rebuilds every instance)
+eb_status ensure_per_inst(eb_controller* c)
+{
+  if (c->per_inst) return EB_OK;
+  EB_CUDA(cudaSetDevice(c->cfg.device));
+  const size_t pb = sizeof(double) * (size_t)c->K * c->B, fb = sizeof(double) * eb::kFrDoubles * (size_t)c->B;
+  EB_CUDA(cudaMalloc(&c->d_phik_b, pb));
+  EB_CUDA(cudaMalloc(&c->d_frames, fb));
+  EB_CUDA(cudaMalloc(&c->d_gcount, sizeof(int) * (size_t)c->B));
+  EB_CUDA(cudaMalloc(&c->d_bounds, sizeof(double) * 4 * (size_t)c->B));
+  EB_CUDA(cudaMemsetAsync(c->d_phik_b, 0, pb, c->stream));
+  EB_CUDA(cudaMemsetAsync(c->d_frames, 0, fb, c->stream));
+  EB_CUDA(cudaMemsetAsync(c->d_gcount, 0, sizeof(int) * (size_t)c->B, c->stream));
+  c->per_inst = true;
+  return EB_OK;
+}
+
+// configTarget of every instance (bounds_dev [B][4]), or the frames of eb_set_phik_batch_dev (extent_dev [B][2])
+eb_status target_batch(eb_controller* c, const double* bounds_dev, const double* extent_dev, int* rebuilt_dev)
+{
+  eb::TargetBatchParams tp{};
+  tp.B = c->B;
+  tp.nb = c->nb;
+  tp.max_n = c->gmax;
+  tp.res = c->cfg.resolution;
+  tp.bounds = bounds_dev;
+  tp.extent = extent_dev;
+  tp.counts = c->d_gcount;
+  tp.mu = c->d_gmu;
+  tp.sigma = c->d_gsig;
+  tp.frames = c->d_frames;
+  tp.phik = c->d_phik_b;
+  tp.rebuilt = rebuilt_dev;
+  tp.hist = c->d_hist;
+  tp.hist_cos = c->d_hist_cos;
+  tp.mem_count = c->d_hist_cos ? c->mem_count : 0;
+  tp.fault = c->d_fault;
+  eb::target_batch_kernel<<<c->B, eb::kTbThreads, sizeof(double) * 6 * (size_t)c->gmax, c->stream>>>(tp);
+  EB_CUDA(cudaGetLastError());
+  c->launches += 1;
+  c->frames_set = true;
   return EB_OK;
 }
 }  // namespace
@@ -981,6 +1064,12 @@ void eb_destroy(eb_controller* c)
   cudaFree(c->d_phi_grid);
   cudaFree(c->d_gauss);
   cudaFree(c->d_big_scratch);
+  cudaFree(c->d_phik_b);
+  cudaFree(c->d_frames);
+  cudaFree(c->d_gmu);
+  cudaFree(c->d_gsig);
+  cudaFree(c->d_gcount);
+  cudaFree(c->d_bounds);
   eb_phik_plan_destroy(c->plan);
   delete c;
 }
@@ -1030,6 +1119,34 @@ eb_status eb_clone(const eb_controller* src, eb_controller** out)
   c->have_pose = src->have_pose;
   c->keep_ck = src->keep_ck;
   c->stream = src->stream;
+  if (src->per_inst)
+  {
+    if ((st = ensure_per_inst(c)) != EB_OK)
+    {
+      eb_destroy(c);
+      return st;
+    }
+    const size_t B = (size_t)src->B;
+    if ((e = cudaMemcpy(c->d_phik_b, src->d_phik_b, sizeof(double) * src->K * B, cudaMemcpyDeviceToDevice)) != cudaSuccess ||
+        (e = cudaMemcpy(c->d_frames, src->d_frames, sizeof(double) * eb::kFrDoubles * B, cudaMemcpyDeviceToDevice)) != cudaSuccess ||
+        (e = cudaMemcpy(c->d_gcount, src->d_gcount, sizeof(int) * B, cudaMemcpyDeviceToDevice)) != cudaSuccess)
+      return bail(e);
+    if (src->gmax > 0)
+    {
+      const size_t gb = sizeof(double) * 2 * (size_t)src->gmax * B;
+      if ((e = cudaMalloc(&c->d_gmu, gb)) != cudaSuccess || (e = cudaMalloc(&c->d_gsig, gb)) != cudaSuccess ||
+          (e = cudaMemcpy(c->d_gmu, src->d_gmu, gb, cudaMemcpyDeviceToDevice)) != cudaSuccess ||
+          (e = cudaMemcpy(c->d_gsig, src->d_gsig, gb, cudaMemcpyDeviceToDevice)) != cudaSuccess)
+        return bail(e);
+      c->gmax = src->gmax;
+    }
+    // the cosine rows (the shared path re-derives them; per-instance rows are only derived when a frame moves)
+    if (src->mem_count > 0 && src->d_hist_cos && c->d_hist_cos &&
+        (e = cudaMemcpy(c->d_hist_cos, src->d_hist_cos, sizeof(double) * 2 * B * (size_t)src->mem_count,
+                        cudaMemcpyDeviceToDevice)) != cudaSuccess)
+      return bail(e);
+    c->frames_set = src->frames_set;
+  }
   *out = c;
   return EB_OK;
 }
@@ -1061,6 +1178,7 @@ eb_status eb_set_keep_ck(eb_controller* c, int keep)
 eb_status eb_set_target_gaussians(eb_controller* c, int n, const double* mu, const double* sigma)
 {
   if (!c || n < 0 || (n > 0 && (!mu || !sigma))) return fail(EB_ERR_INVALID_ARGUMENT, "eb_set_target_gaussians: bad argument");
+  if (c->per_inst) return refuse_per_inst("eb_set_target_gaussians");
   c->gauss_mu.assign(mu, mu + 2 * (size_t)n);
   c->gauss_sigma.assign(sigma, sigma + 2 * (size_t)n);
   return EB_OK;
@@ -1070,6 +1188,7 @@ eb_status eb_config_target(eb_controller* c, double xmin, double xmax, double ym
 {
   EB_TRACE("eb_config_target");
   if (!c) return fail(EB_ERR_INVALID_ARGUMENT, "controller is NULL");
+  if (c->per_inst) return refuse_per_inst("eb_config_target");
   if (rebuilt) *rebuilt = 0;
   // translation from map to fourier domain (:366-367)
   c->map_pos[0] = xmin;
@@ -1137,6 +1256,7 @@ eb_status eb_config_target(eb_controller* c, double xmin, double xmax, double ym
 eb_status eb_set_phik(eb_controller* c, const double* phik, double lx, double ly)
 {
   if (!c || !phik) return fail(EB_ERR_INVALID_ARGUMENT, "eb_set_phik: NULL argument");
+  if (c->per_inst) return refuse_per_inst("eb_set_phik");
   EB_CUDA(cudaSetDevice(c->cfg.device));
   EB_CUDA(cudaMemcpyAsync(c->d_phik, phik, sizeof(double) * c->K, cudaMemcpyHostToDevice, c->stream));
   EB_CUDA(cudaStreamSynchronize(c->stream));
@@ -1148,6 +1268,7 @@ eb_status eb_set_phik(eb_controller* c, const double* phik, double lx, double ly
 eb_status eb_get_phik(const eb_controller* c, double* phik, double* lx, double* ly)
 {
   if (!c) return fail(EB_ERR_INVALID_ARGUMENT, "controller is NULL");
+  if (c->per_inst) return refuse_per_inst("eb_get_phik");
   EB_CUDA(cudaSetDevice(c->cfg.device));
   if (phik)
   {
@@ -1167,13 +1288,30 @@ static eb_status add_state_memory(eb_controller* c, const double* x, cudaMemcpyK
   eb_status st = ensure_hist(c, c->mem_count + 1);
   if (st != EB_OK) return st;
   const size_t row = (size_t)c->B * (size_t)c->mem_count;
+  if (c->per_inst && c->d_hist_cos)
+  {
+    // per-instance frames: the row and its cosines (each in its instance's frame) in one launch, always
+    const double* xd = x;
+    if (kind == cudaMemcpyHostToDevice)
+    {
+      EB_CUDA(cudaMemcpyAsync(c->d_x, x, sizeof(double) * 3 * c->B, kind, c->stream));
+      xd = c->d_x;
+    }
+    eb::add_state_kernel<<<(c->B + 255) / 256, 256, 0, c->stream>>>(xd, c->d_hist + 3 * row, c->d_hist_cos + 2 * row, c->B,
+                                                                    0.0, 0.0, 0.0, 0.0, c->d_frames);
+    EB_CUDA(cudaGetLastError());
+    if (kind == cudaMemcpyHostToDevice) EB_CUDA(cudaStreamSynchronize(c->stream));
+    c->launches += 1;
+    c->mem_count++;
+    return EB_OK;
+  }
   const double key[4] = { c->map_pos[0], c->map_pos[1], 1.0 / c->lx, 1.0 / c->ly };
   if (kind == cudaMemcpyDeviceToDevice && c->d_hist_cos && c->cos_count == c->mem_count && c->lx > 0.0 && c->ly > 0.0 &&
       std::memcmp(key, c->cos_key, sizeof(key)) == 0)
   {
     // the cosine rows are up to date for the current frame: the new row and its cosines in ONE launch
     eb::add_state_kernel<<<(c->B + 255) / 256, 256, 0, c->stream>>>(x, c->d_hist + 3 * row, c->d_hist_cos + 2 * row, c->B,
-                                                                    key[0], key[1], key[2], key[3]);
+                                                                    key[0], key[1], key[2], key[3], nullptr);
     EB_CUDA(cudaGetLastError());
     c->launches += 1;
     c->cos_count++;
@@ -1205,14 +1343,25 @@ eb_status eb_add_state_memory_dev(eb_controller* c, const double* x_dev)
   return add_state_memory(c, x_dev, cudaMemcpyDeviceToDevice);
 }
 
+static eb_status solve_step(eb_controller* c, const double* x_dev, const int* mem_idx_dev, double* u0_dev,
+                            double* metric_dev);
+
 eb_status eb_control_dev(eb_controller* c, double xmin, double xmax, double ymin, double ymax, const double* x_dev,
                          const int* mem_idx_dev, double* u0_dev, double* metric_dev)
 {
   EB_TRACE("eb_control_dev");
   if (!c || !x_dev || !u0_dev) return fail(EB_ERR_INVALID_ARGUMENT, "eb_control_dev: NULL argument");
+  if (c->per_inst) return refuse_per_inst("eb_control_dev");
   EB_CUDA(cudaSetDevice(c->cfg.device));
   eb_status st = eb_config_target(c, xmin, xmax, ymin, ymax, nullptr);  // :230
   if (st != EB_OK) return st;
+  return solve_step(c, x_dev, mem_idx_dev, u0_dev, metric_dev);
+}
+
+// one solve launch over the batch, after the target is configured (shared frame, or per-instance frames and rows)
+static eb_status solve_step(eb_controller* c, const double* x_dev, const int* mem_idx_dev, double* u0_dev,
+                            double* metric_dev)
+{
   // pose_ = x (:227)
   c->have_pose = true;  // the kernel records x as pose_ (for optTraj)
 
@@ -1260,13 +1409,17 @@ eb_status eb_control_dev(eb_controller* c, double xmin, double xmax, double ymin
   p.hist = c->d_hist;
   if (p.M > 0 && c->d_hist_cos && c->nb <= 32)
   {  // (the CTA-per-instance kernel starts its tables at arbitrary orders and needs the coordinates themselves)
-    const eb_status hs = ensure_hist_cos(c);
-    if (hs != EB_OK) return hs;
+    if (!c->per_inst)  // per-instance rows are kept valid as frames move and states are stored
+    {
+      const eb_status hs = ensure_hist_cos(c);
+      if (hs != EB_OK) return hs;
+    }
     p.hist_cos = c->d_hist_cos;
   }
   p.mem_idx = mem_idx_dev;
   p.mem_idx_out = c->d_mem_idx_out;
-  p.phik = c->d_phik;
+  p.phik = c->per_inst ? c->d_phik_b : c->d_phik;
+  p.frames = c->d_frames;
   p.lamk = c->d_lamk;
   p.u0 = u0_dev;
   p.metric = metric_dev;
@@ -1288,7 +1441,7 @@ eb_status eb_control_dev(eb_controller* c, double xmin, double xmax, double ymin
     p.need = c->peer->need;
   }
   const int rounds = (c->N + 31) / 32;
-  cudaError_t e = launch_solve(p, c->cfg.model, rounds, c->stream);
+  cudaError_t e = launch_solve(p, c->cfg.model, rounds, c->stream, c->per_inst);
   if (e != cudaSuccess) return fail(EB_ERR_CUDA, std::string("solve_kernel launch: ") + cudaGetErrorString(e));
   c->launches += 1;
   c->cur ^= 1;
@@ -1322,6 +1475,7 @@ eb_status eb_control_host(eb_controller* c, double xmin, double xmax, double ymi
 {
   EB_TRACE("eb_control_host");
   if (!c || !x || !u0) return fail(EB_ERR_INVALID_ARGUMENT, "eb_control_host: NULL argument");
+  if (c->per_inst) return refuse_per_inst("eb_control_host");
   EB_CUDA(cudaSetDevice(c->cfg.device));
   const bool need_idx = mem_idx && c->mem_count > (long long)c->cfg.batch_size;
   if (need_idx)
@@ -1693,6 +1847,7 @@ eb_status eb_control_dev_gather(eb_controller* c, eb_peer_group* g, double xmin,
 {
   EB_TRACE("eb_control_dev_gather");
   if (!c || !g) return fail(EB_ERR_INVALID_ARGUMENT, "eb_control_dev_gather: NULL argument");
+  if (c->per_inst) return fail(EB_ERR_UNSUPPORTED, "eb_control_dev_gather: not available with per-instance targets");
   if (!g->connected) return fail(EB_ERR_INVALID_ARGUMENT, "eb_control_dev_gather: peer group is not connected");
   if (g->elems != 3LL * c->B) return fail(EB_ERR_INVALID_ARGUMENT, "eb_control_dev_gather: peer group sized for another batch");
   const int parity = (int)(g->step % eb::kPeerBuffers);
@@ -1763,6 +1918,7 @@ eb_status eb_control_dev_gather_wait(eb_controller* c, eb_peer_group* g, double 
 {
   EB_TRACE("eb_control_dev_gather_wait");
   if (!c || !g) return fail(EB_ERR_INVALID_ARGUMENT, "eb_control_dev_gather_wait: NULL argument");
+  if (c->per_inst) return fail(EB_ERR_UNSUPPORTED, "eb_control_dev_gather_wait: not available with per-instance targets");
   if (!g->connected) return fail(EB_ERR_INVALID_ARGUMENT, "eb_control_dev_gather_wait: peer group is not connected");
   if (g->elems != 3LL * c->B) return fail(EB_ERR_INVALID_ARGUMENT, "eb_control_dev_gather_wait: peer group sized for another batch");
   if (c->B >= g->fuse_min_batch)
@@ -2712,12 +2868,142 @@ eb_status eb_map_target_execute_host(eb_map_target* m, const signed char* cells,
 eb_status eb_set_phik_dev(eb_controller* c, const double* phik_dev, double lx, double ly)
 {
   if (!c || !phik_dev) return fail(EB_ERR_INVALID_ARGUMENT, "eb_set_phik_dev: NULL argument");
+  if (c->per_inst) return refuse_per_inst("eb_set_phik_dev");
   if (!(lx > 0.0) || !(ly > 0.0)) return fail(EB_ERR_INVALID_ARGUMENT, "eb_set_phik_dev: lx, ly must be positive");
   EB_CUDA(cudaSetDevice(c->cfg.device));
   EB_CUDA(cudaMemcpyAsync(c->d_phik, phik_dev, sizeof(double) * c->K, cudaMemcpyDeviceToDevice, c->stream));
   c->lx = lx;
   c->ly = ly;
   return EB_OK;
+}
+
+// ---------------------------------------------------------------------------
+// per-instance targets: one target, phi_k row and Fourier frame per instance (target_batch.cuh)
+// ---------------------------------------------------------------------------
+eb_status eb_set_target_gaussians_batch(eb_controller* c, int max_n, const int* counts, const double* mu,
+                                        const double* sigma)
+{
+  EB_TRACE("eb_set_target_gaussians_batch");
+  if (!c || !counts || max_n < 0 || max_n > eb::kTbMaxGauss || (max_n > 0 && (!mu || !sigma)))
+    return fail(EB_ERR_INVALID_ARGUMENT, "eb_set_target_gaussians_batch: bad argument (NULL, or max_n outside 0.." +
+                                             std::to_string(eb::kTbMaxGauss) + ")");
+  for (int i = 0; i < c->B; i++)
+    if (counts[i] < 0 || counts[i] > max_n)
+      return fail(EB_ERR_INVALID_ARGUMENT, "eb_set_target_gaussians_batch: counts[" + std::to_string(i) +
+                                               "] outside 0..max_n");
+  EB_CUDA(cudaSetDevice(c->cfg.device));
+  eb_status st = ensure_per_inst(c);
+  if (st != EB_OK) return st;
+  if (max_n > c->gmax)
+  {
+    cudaFree(c->d_gmu);
+    cudaFree(c->d_gsig);
+    c->d_gmu = c->d_gsig = nullptr;
+    c->gmax = 0;
+    const size_t gb = sizeof(double) * 2 * (size_t)max_n * c->B;
+    EB_CUDA(cudaMalloc(&c->d_gmu, gb));
+    EB_CUDA(cudaMalloc(&c->d_gsig, gb));
+  }
+  c->gmax = std::max(c->gmax, max_n);
+  // the caller's [B][max_n][2] rows into the [B][gmax][2] buffers
+  const size_t row = sizeof(double) * 2 * (size_t)max_n, pitch = sizeof(double) * 2 * (size_t)c->gmax;
+  if (max_n > 0)
+  {
+    EB_CUDA(cudaMemcpy2DAsync(c->d_gmu, pitch, mu, row, row, c->B, cudaMemcpyHostToDevice, c->stream));
+    EB_CUDA(cudaMemcpy2DAsync(c->d_gsig, pitch, sigma, row, row, c->B, cudaMemcpyHostToDevice, c->stream));
+  }
+  EB_CUDA(cudaMemcpyAsync(c->d_gcount, counts, sizeof(int) * (size_t)c->B, cudaMemcpyHostToDevice, c->stream));
+  EB_CUDA(cudaStreamSynchronize(c->stream));  // the caller's buffers may go once this returns
+  return EB_OK;
+}
+
+eb_status eb_config_target_batch_dev(eb_controller* c, const double* bounds_dev, int* rebuilt_dev)
+{
+  EB_TRACE("eb_config_target_batch_dev");
+  if (!c || !bounds_dev) return fail(EB_ERR_INVALID_ARGUMENT, "eb_config_target_batch_dev: NULL argument");
+  EB_CUDA(cudaSetDevice(c->cfg.device));
+  eb_status st = ensure_per_inst(c);
+  if (st != EB_OK) return st;
+  return target_batch(c, bounds_dev, nullptr, rebuilt_dev);
+}
+
+eb_status eb_set_phik_batch_dev(eb_controller* c, const double* phik_dev, const double* extent_dev)
+{
+  EB_TRACE("eb_set_phik_batch_dev");
+  if (!c || !phik_dev || !extent_dev) return fail(EB_ERR_INVALID_ARGUMENT, "eb_set_phik_batch_dev: NULL argument");
+  EB_CUDA(cudaSetDevice(c->cfg.device));
+  eb_status st = ensure_per_inst(c);
+  if (st != EB_OK) return st;
+  EB_CUDA(cudaMemcpyAsync(c->d_phik_b, phik_dev, sizeof(double) * (size_t)c->K * c->B, cudaMemcpyDeviceToDevice,
+                          c->stream));
+  return target_batch(c, nullptr, extent_dev, nullptr);
+}
+
+eb_status eb_get_phik_batch(const eb_controller* c, double* phik, double* extent)
+{
+  if (!c) return fail(EB_ERR_INVALID_ARGUMENT, "controller is NULL");
+  if (!c->per_inst) return fail(EB_ERR_INVALID_ARGUMENT, "eb_get_phik_batch: the controller holds a shared target (eb_get_phik)");
+  EB_CUDA(cudaSetDevice(c->cfg.device));
+  if (phik)
+    EB_CUDA(cudaMemcpyAsync(phik, c->d_phik_b, sizeof(double) * (size_t)c->K * c->B, cudaMemcpyDeviceToHost, c->stream));
+  if (extent)
+    EB_CUDA(cudaMemcpy2DAsync(extent, sizeof(double) * 2, c->d_frames + eb::kFrLx, sizeof(double) * eb::kFrDoubles,
+                              sizeof(double) * 2, c->B, cudaMemcpyDeviceToHost, c->stream));
+  EB_CUDA(cudaStreamSynchronize(c->stream));
+  return EB_OK;
+}
+
+eb_status eb_control_batch_dev(eb_controller* c, const double* bounds_dev, const double* x_dev, const int* mem_idx_dev,
+                               double* u0_dev, double* metric_dev)
+{
+  EB_TRACE("eb_control_batch_dev");
+  if (!c || !x_dev || !u0_dev) return fail(EB_ERR_INVALID_ARGUMENT, "eb_control_batch_dev: NULL argument");
+  if (!bounds_dev && !c->frames_set)
+    return fail(EB_ERR_INVALID_ARGUMENT, "eb_control_batch_dev: bounds NULL before any frame was configured");
+  EB_CUDA(cudaSetDevice(c->cfg.device));
+  eb_status st = ensure_per_inst(c);
+  if (st != EB_OK) return st;
+  if (bounds_dev && (st = target_batch(c, bounds_dev, nullptr, nullptr)) != EB_OK) return st;  // :230
+  return solve_step(c, x_dev, mem_idx_dev, u0_dev, metric_dev);
+}
+
+eb_status eb_control_batch_host(eb_controller* c, const double* bounds, const double* x, const int* mem_idx, double* u0,
+                                double* metric)
+{
+  EB_TRACE("eb_control_batch_host");
+  if (!c || !x || !u0) return fail(EB_ERR_INVALID_ARGUMENT, "eb_control_batch_host: NULL argument");
+  if (!bounds && !c->frames_set)
+    return fail(EB_ERR_INVALID_ARGUMENT, "eb_control_batch_host: bounds NULL before any frame was configured");
+  EB_CUDA(cudaSetDevice(c->cfg.device));
+  eb_status st = ensure_per_inst(c);
+  if (st != EB_OK) return st;
+  if (bounds)
+    EB_CUDA(cudaMemcpyAsync(c->d_bounds, bounds, sizeof(double) * 4 * (size_t)c->B, cudaMemcpyHostToDevice, c->stream));
+  const double* bd = bounds ? c->d_bounds : nullptr;
+  const bool need_idx = mem_idx && c->mem_count > (long long)c->cfg.batch_size;
+  if (need_idx)
+    EB_CUDA(cudaMemcpyAsync(c->d_mem_idx_in, mem_idx, sizeof(int) * (size_t)c->cfg.batch_size * c->B,
+                            cudaMemcpyHostToDevice, c->stream));
+  // as eb_control_host: page-locked caller buffers of a small batch are read / written in place
+  double *xm = nullptr, *um = nullptr, *mm = nullptr;
+  if (c->B <= zero_copy_max_batch())
+  {
+    xm = c->mapped(x);
+    um = xm ? c->mapped(u0) : nullptr;
+    mm = (um && metric) ? c->mapped(metric) : nullptr;
+  }
+  if (xm && um && (!metric || mm))
+  {
+    st = eb_control_batch_dev(c, bd, xm, need_idx ? c->d_mem_idx_in : nullptr, um, mm);
+    if (st != EB_OK) return st;
+    return check_fault(c);  // synchronises
+  }
+  EB_CUDA(cudaMemcpyAsync(c->d_pose, x, sizeof(double) * 3 * c->B, cudaMemcpyHostToDevice, c->stream));
+  st = eb_control_batch_dev(c, bd, c->d_pose, need_idx ? c->d_mem_idx_in : nullptr, c->d_u0, metric ? c->d_metric : nullptr);
+  if (st != EB_OK) return st;
+  EB_CUDA(cudaMemcpyAsync(u0, c->d_u0, sizeof(double) * 3 * c->B, cudaMemcpyDeviceToHost, c->stream));
+  if (metric) EB_CUDA(cudaMemcpyAsync(metric, c->d_metric, sizeof(double) * c->B, cudaMemcpyDeviceToHost, c->stream));
+  return check_fault(c);  // synchronises
 }
 
 // ---------------------------------------------------------------------------

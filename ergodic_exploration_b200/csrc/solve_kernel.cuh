@@ -138,7 +138,59 @@ struct SolveParams
   // num_basis > 32 (solve_kernel_big.cuh): one row of nb * nb doubles per resident CTA, and how many rows there are
   double* big_scratch;
   int big_rows;
+  // per-instance targets (PER_INST kernels): Fourier frame of every instance [B][kFrDoubles]; phik is then [B][nb*nb]
+  const double* frames;
 };
+
+// Layout of a per-instance frame record.  The derived values are computed by the same expressions as the shared
+// frame's (eb_control_dev), so an instance whose frame equals the shared one sees the same bits.
+enum FrameField
+{
+  kFrXmin,
+  kFrYmin,
+  kFrLx,
+  kFrLy,
+  kFrInvLx,
+  kFrInvLy,
+  kFrAx,
+  kFrBy,
+  kFrDoubles
+};
+
+// One value of the Fourier frame of `inst`: read at its use site (L1 serves the 64-byte record), never hoisted by hand
+// across the kernel, so the per-instance kernels keep the shared ones' register budget.
+template <bool PER_INST, int F>
+__device__ __forceinline__ double frame(const SolveParams& p, const int inst)
+{
+  if constexpr (PER_INST)
+    return __ldg(p.frames + (size_t)inst * kFrDoubles + F);
+  else if constexpr (F == kFrXmin)
+    return p.xmin;
+  else if constexpr (F == kFrYmin)
+    return p.ymin;
+  else if constexpr (F == kFrLx)
+    return p.lx;
+  else if constexpr (F == kFrLy)
+    return p.ly;
+  else if constexpr (F == kFrInvLx)
+    return p.inv_lx;
+  else if constexpr (F == kFrInvLy)
+    return p.inv_ly;
+  else if constexpr (F == kFrAx)
+    return p.ax;
+  else
+    return p.by;
+}
+
+// phi_k[k] of `inst`: the shared row, or the instance's own row of the [B][K] table
+template <bool PER_INST>
+__device__ __forceinline__ double phik_at(const SolveParams& p, const int inst, const int K, const int k)
+{
+  if constexpr (PER_INST)
+    return __ldg(p.phik + (size_t)inst * K + k);
+  else
+    return __ldg(p.phik + k);
+}
 
 // The first twist of one instance: lanes 0..2 store one contiguous 24-byte segment (u0 may live in mapped host
 // memory); with a peer group (N > 1 GPUs) the same row goes into every rank's gathered buffer.
@@ -426,7 +478,7 @@ inline size_t solve_smem_bytes(int tab_doubles, int fields, int rounds, int warp
   return sizeof(double) * warps * (size_t)(tab_doubles + fields * 32 * rounds);
 }
 
-template <int MODEL, int NB, int WARPS = kSolveWarps>
+template <int MODEL, int NB, int WARPS = kSolveWarps, bool PER_INST = false>
 __global__ void __launch_bounds__(WARPS * 32, WARPS == kSolveWarps ? SolveCfg<NB>::kMinBlocks : 1) solve_kernel(const SolveParams p)
 {
   using Cfg = SolveCfg<NB>;
@@ -508,9 +560,9 @@ __global__ void __launch_bounds__(WARPS * 32, WARPS == kSolveWarps ? SolveCfg<NB
       else
       {
         const double* h = p.hist + ((size_t)idx * p.B + inst) * 3;
-        const double xf = h[0] - p.xmin, yf = h[1] - p.ymin;
-        c1x = fast_cospi(xf * p.inv_lx);
-        c1y = fast_cospi(yf * p.inv_ly);
+        const double xf = h[0] - frame<PER_INST, kFrXmin>(p, inst), yf = h[1] - frame<PER_INST, kFrYmin>(p, inst);
+        c1x = fast_cospi(xf * frame<PER_INST, kFrInvLx>(p, inst));
+        c1y = fast_cospi(yf * frame<PER_INST, kFrInvLy>(p, inst));
       }
     }
     const int nvalid = min(32, p.M - base);
@@ -558,7 +610,7 @@ __global__ void __launch_bounds__(WARPS * 32, WARPS == kSolveWarps ? SolveCfg<NB
     if (MODEL == kModelSimpleCart && !(fabs(u1 - 0.0) < 1.0e-12)) atomicOr(p.fault, 1);  // cart.hpp:167-170
     double xo, yo, tho, ce, se;
     rollout_round<MODEL>(p.dt, valid, lane, u0, u1, u2, cy, xo, yo, tho, ce, se);
-    const double xf = xo - p.xmin, yf = yo - p.ymin;
+    const double xf = xo - frame<PER_INST, kFrXmin>(p, inst), yf = yo - frame<PER_INST, kFrYmin>(p, inst);
     rec[0 * npad + i] = ce;
     rec[1 * npad + i] = se;
     rec[2 * npad + i] = xf;
@@ -566,14 +618,14 @@ __global__ void __launch_bounds__(WARPS * 32, WARPS == kSolveWarps ? SolveCfg<NB
     double ca, cb;
     if (Cfg::kRecompute)
     {
-      ca = fast_cospi(xf * p.inv_lx);
-      cb = fast_cospi(yf * p.inv_ly);
+      ca = fast_cospi(xf * frame<PER_INST, kFrInvLx>(p, inst));
+      cb = fast_cospi(yf * frame<PER_INST, kFrInvLy>(p, inst));
     }
     else
     {
       double sa, sb;
-      fast_sincospi(xf * p.inv_lx, &sa, &ca);
-      fast_sincospi(yf * p.inv_ly, &sb, &cb);
+      fast_sincospi(xf * frame<PER_INST, kFrInvLx>(p, inst), &sa, &ca);
+      fast_sincospi(yf * frame<PER_INST, kFrInvLy>(p, inst), &sb, &cb);
       rec[4 * npad + i] = ca;
       rec[5 * npad + i] = sa;
       rec[6 * npad + i] = cb;
@@ -606,7 +658,7 @@ __global__ void __launch_bounds__(WARPS * 32, WARPS == kSolveWarps ? SolveCfg<NB
             // explicitly rounded (no FMA contraction): c_k as stored == c_k as used, whichever
             // way the compiler specialises the p.ck branch
             const double c = __dmul_rn(inv_t, acc[ti][tj][e]);
-            const double d = __dsub_rn(c, __ldg(p.phik + k));
+            const double d = __dsub_rn(c, phik_at<PER_INST>(p, inst, K, k));
             s = __ldg(p.lamk + k) * d;
             metric += s * d;
             if (p.ck) p.ck[(size_t)inst * K + k] = c;
@@ -645,8 +697,8 @@ __global__ void __launch_bounds__(WARPS * 32, WARPS == kSolveWarps ? SolveCfg<NB
       {
         const int ky = 8 * mi + g, kx = 4 * ks + q;
         const double sv = (ky < NB && kx < NB) ? Ssm[ky * Cfg::kSPitch + kx] : 0.0;
-        SA[mi][ks] = sv * ((double)kx * p.ax);
-        SB[mi][ks] = sv * ((double)ky * p.by);
+        SA[mi][ks] = sv * ((double)kx * frame<PER_INST, kFrAx>(p, inst));
+        SB[mi][ks] = sv * ((double)ky * frame<PER_INST, kFrBy>(p, inst));
       }
     __syncwarp();  // S has been read: the table region is free for the gradient tables
   }
@@ -669,8 +721,8 @@ __global__ void __launch_bounds__(WARPS * 32, WARPS == kSolveWarps ? SolveCfg<NB
     double ca, sa, cb, sb;
     if (Cfg::kRecompute)
     {
-      fast_sincospi(xf * p.inv_lx, &sa, &ca);
-      fast_sincospi(yf * p.inv_ly, &sb, &cb);
+      fast_sincospi(xf * frame<PER_INST, kFrInvLx>(p, inst), &sa, &ca);
+      fast_sincospi(yf * frame<PER_INST, kFrInvLy>(p, inst), &sb, &cb);
     }
     else
     {
@@ -807,7 +859,7 @@ __global__ void __launch_bounds__(WARPS * 32, WARPS == kSolveWarps ? SolveCfg<NB
         for (int j = 0; j < KB; j++)
         {
           cx[j] = xck;
-          asx[j] = ((double)(kb + j) * p.ax) * xsk;
+          asx[j] = ((double)(kb + j) * frame<PER_INST, kFrAx>(p, inst)) * xsk;
           const double cn = xt2 * xck - xcm, sn = xt2 * xsk - xsm;
           xcm = xck;
           xck = cn;
@@ -830,7 +882,7 @@ __global__ void __launch_bounds__(WARPS * 32, WARPS == kSolveWarps ? SolveCfg<NB
             ry1 = fma(s2.y, cx[j + 1], ry1);
           }
           ex = fma(ck, rx0 + rx1, ex);
-          ey = fma(((double)ky * p.by) * sk, ry0 + ry1, ey);
+          ey = fma(((double)ky * frame<PER_INST, kFrBy>(p, inst)) * sk, ry0 + ry1, ey);
           const double cn = yt2 * ck - cm, sn = yt2 * sk - sm;
           cm = ck;
           ck = cn;
@@ -862,8 +914,8 @@ __global__ void __launch_bounds__(WARPS * 32, WARPS == kSolveWarps ? SolveCfg<NB
 #endif
     // gradBarrier :454-474
     double bx = 0.0, byv = 0.0;
-    bx += 2.0 * (double)(xf > p.lx - p.beps) * (xf - (p.lx - p.beps));
-    byv += 2.0 * (double)(yf > p.ly - p.beps) * (yf - (p.ly - p.beps));
+    bx += 2.0 * (double)(xf > frame<PER_INST, kFrLx>(p, inst) - p.beps) * (xf - (frame<PER_INST, kFrLx>(p, inst) - p.beps));
+    byv += 2.0 * (double)(yf > frame<PER_INST, kFrLy>(p, inst) - p.beps) * (yf - (frame<PER_INST, kFrLy>(p, inst) - p.beps));
     bx += 2.0 * (double)(xf < p.beps) * (xf - p.beps);
     byv += 2.0 * (double)(yf < p.beps) * (yf - p.beps);
     bx *= p.bw;
@@ -957,10 +1009,11 @@ __global__ void __launch_bounds__(256) hist_cos_kernel(const double* __restrict_
   out[2 * e + 0] = fast_cospi(xf * inv_lx);
   out[2 * e + 1] = fast_cospi(yf * inv_ly);
 }
-// addStateMemory with the cache up to date: the new row and its cosines in one launch (instead of a copy + a launch)
+// addStateMemory with the cache up to date: the new row and its cosines in one launch (instead of a copy + a launch).
+// frames: per-instance targets, each row's cosines in its instance's frame (the scalar frame is ignored)
 __global__ void __launch_bounds__(256) add_state_kernel(const double* __restrict__ x, double* __restrict__ hist_row,
                                                         double* __restrict__ cos_row, int B, double xmin, double ymin,
-                                                        double inv_lx, double inv_ly)
+                                                        double inv_lx, double inv_ly, const double* __restrict__ frames)
 {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= B) return;
@@ -968,6 +1021,14 @@ __global__ void __launch_bounds__(256) add_state_kernel(const double* __restrict
   hist_row[3 * i + 0] = a;
   hist_row[3 * i + 1] = b;
   hist_row[3 * i + 2] = c;
+  if (frames)
+  {
+    const double* f = frames + (size_t)i * kFrDoubles;
+    xmin = f[kFrXmin];
+    ymin = f[kFrYmin];
+    inv_lx = f[kFrInvLx];
+    inv_ly = f[kFrInvLy];
+  }
   const double xf = a - xmin, yf = b - ymin;
   cos_row[2 * i + 0] = fast_cospi(xf * inv_lx);
   cos_row[2 * i + 1] = fast_cospi(yf * inv_ly);

@@ -61,7 +61,7 @@ __device__ __forceinline__ void big_chain_step(BigChain& c)
   c.sk = sn;
 }
 
-template <int MODEL>
+template <int MODEL, bool PER_INST = false>
 __global__ void __launch_bounds__(kBigThreads) solve_kernel_big(const SolveParams p, double* __restrict__ scratch)
 {
   extern __shared__ __align__(16) double smem_big[];
@@ -115,8 +115,8 @@ __global__ void __launch_bounds__(kBigThreads) solve_kernel_big(const SolveParam
         rollout_round<MODEL>(p.dt, valid, lane, u0, u1, u2, cy, xo, yo, tho, ce, se);
         rec[0 * npad + i] = ce;
         rec[1 * npad + i] = se;
-        rec[2 * npad + i] = xo - p.xmin;
-        rec[3 * npad + i] = yo - p.ymin;
+        rec[2 * npad + i] = xo - frame<PER_INST, kFrXmin>(p, inst);
+        rec[3 * npad + i] = yo - frame<PER_INST, kFrYmin>(p, inst);
       }
     }
     __syncthreads();
@@ -168,12 +168,12 @@ __global__ void __launch_bounds__(kBigThreads) solve_kernel_big(const SolveParam
               if (p.idx_mode != 0 && p.mem_idx_out && warp == 0 && pass == 0)
                 p.mem_idx_out[(size_t)inst * p.batch_size + s] = (int)idx;
               const double* h = p.hist + ((size_t)idx * p.B + inst) * 3;
-              coord = h[axis] - (axis ? p.ymin : p.xmin);
+              coord = h[axis] - (axis ? frame<PER_INST, kFrYmin>(p, inst) : frame<PER_INST, kFrXmin>(p, inst));
             }
             else
               coord = rec[(2 + axis) * npad + (s - p.M)];
           }
-          const double u = coord * (axis ? p.inv_ly : p.inv_lx);
+          const double u = coord * (axis ? frame<PER_INST, kFrInvLy>(p, inst) : frame<PER_INST, kFrInvLx>(p, inst));
           const int k0 = seg * kq, k1 = min(tabrows, k0 + kq);
           double* const col = (axis ? t_y : t_x) + lane;
           BigChain ch = big_chain_start(u, k0);
@@ -215,7 +215,7 @@ __global__ void __launch_bounds__(kBigThreads) solve_kernel_big(const SolveParam
             {
               const int k = ky * nb + kx;
               const double c = __dmul_rn(inv_t, acc[j][e]);
-              const double d = __dsub_rn(c, __ldg(p.phik + k));
+              const double d = __dsub_rn(c, phik_at<PER_INST>(p, inst, K, k));
               const double sv = __ldg(p.lamk + k) * d;
               metric += sv * d;
               if (p.ck) p.ck[(size_t)inst * K + k] = c;
@@ -249,8 +249,8 @@ __global__ void __launch_bounds__(kBigThreads) solve_kernel_big(const SolveParam
         const int axis = warp & 1, seg = warp >> 1;
         const int i = r * 32 + lane;
         const double coord = rec[(2 + axis) * npad + i];
-        const double u = coord * (axis ? p.inv_ly : p.inv_lx);
-        const double f = axis ? p.by : p.ax;
+        const double u = coord * (axis ? frame<PER_INST, kFrInvLy>(p, inst) : frame<PER_INST, kFrInvLx>(p, inst));
+        const double f = axis ? frame<PER_INST, kFrBy>(p, inst) : frame<PER_INST, kFrAx>(p, inst);
         const int k0 = seg * kq, k1 = min(tabrows, k0 + kq);
         double* const tc = (axis ? t_cy : t_cx) + lane;
         double* const ts = (axis ? t_bsy : t_asx) + lane;
@@ -357,8 +357,8 @@ __global__ void __launch_bounds__(kBigThreads) solve_kernel_big(const SolveParam
         }
         // gradBarrier :454-474
         double bx = 0.0, byv = 0.0;
-        bx += 2.0 * (double)(xf > p.lx - p.beps) * (xf - (p.lx - p.beps));
-        byv += 2.0 * (double)(yf > p.ly - p.beps) * (yf - (p.ly - p.beps));
+        bx += 2.0 * (double)(xf > frame<PER_INST, kFrLx>(p, inst) - p.beps) * (xf - (frame<PER_INST, kFrLx>(p, inst) - p.beps));
+        byv += 2.0 * (double)(yf > frame<PER_INST, kFrLy>(p, inst) - p.beps) * (yf - (frame<PER_INST, kFrLy>(p, inst) - p.beps));
         bx += 2.0 * (double)(xf < p.beps) * (xf - p.beps);
         byv += 2.0 * (double)(yf < p.beps) * (yf - p.beps);
         bx *= p.bw;

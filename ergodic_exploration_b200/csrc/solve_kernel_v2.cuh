@@ -132,7 +132,7 @@ inline size_t solve2_smem_bytes(int N, int warps)
   return sizeof(double) * warps * (size_t)(Solve2Cfg<NB>::kTabDoubles + Solve2Cfg<NB>::kFields * solve2_npad(N));
 }
 
-template <int MODEL, int NB, int WARPS = kSolveWarps>
+template <int MODEL, int NB, int WARPS = kSolveWarps, bool PER_INST = false>
 __global__ void __launch_bounds__(WARPS * 32, WARPS == kSolveWarps ? Solve2Cfg<NB>::kMinBlocks : 1) solve_kernel2(const SolveParams p)
 {
   using Cfg = Solve2Cfg<NB>;
@@ -165,8 +165,8 @@ __global__ void __launch_bounds__(WARPS * 32, WARPS == kSolveWarps ? Solve2Cfg<N
 
   // builder role of this lane: one axis of one state of a half-round
   const int axis = lane >> 4, slot = lane & 15;
-  const double inv_l = axis ? p.inv_ly : p.inv_lx;
-  const double origin = axis ? p.ymin : p.xmin;
+  const double inv_l = axis ? frame<PER_INST, kFrInvLy>(p, inst) : frame<PER_INST, kFrInvLx>(p, inst);
+  const double origin = axis ? frame<PER_INST, kFrYmin>(p, inst) : frame<PER_INST, kFrXmin>(p, inst);
 
   // ---- sampled past states (buffer.cpp:64-111), Fourier frame (:243-244) ----
   if (p.M > 0)
@@ -238,8 +238,8 @@ __global__ void __launch_bounds__(WARPS * 32, WARPS == kSolveWarps ? Solve2Cfg<N
     {
       rec[0 * npad + i] = ce;
       rec[1 * npad + i] = se;
-      rec[2 * npad + i] = xo - p.xmin;
-      rec[3 * npad + i] = yo - p.ymin;
+      rec[2 * npad + i] = xo - frame<PER_INST, kFrXmin>(p, inst);
+      rec[3 * npad + i] = yo - frame<PER_INST, kFrYmin>(p, inst);
     }
     __syncwarp();
     const int nvalid = min(32, p.N - r * 32);
@@ -298,7 +298,7 @@ __global__ void __launch_bounds__(WARPS * 32, WARPS == kSolveWarps ? Solve2Cfg<N
           {
             const int k = ky * nb + kx;
             const double c = __dmul_rn(inv_t, acc[ti][tj][e]);
-            const double d = __dsub_rn(c, __ldg(p.phik + k));
+            const double d = __dsub_rn(c, phik_at<PER_INST>(p, inst, K, k));
             s = __ldg(p.lamk + k) * d;
             metric += s * d;
             if (p.ck) p.ck[(size_t)inst * K + k] = c;
@@ -325,7 +325,7 @@ __global__ void __launch_bounds__(WARPS * 32, WARPS == kSolveWarps ? Solve2Cfg<N
       SF[mi][ks] = (ky < NB && kx < NB) ? Ssm[ky * Cfg::kSPitch + kx] : 0.0;
     }
   __syncwarp();  // S has been read: the table region is free for the y tables
-  const double a4 = 4.0 * p.ax;  // a_kx advances by 4 a per k-step (kx = 4 ks + q)
+  const double a4 = 4.0 * frame<PER_INST, kFrAx>(p, inst);  // a_kx advances by 4 a per k-step (kx = 4 ks + q)
 
   // ---- per round, last round first: metric gradient in 8-step tiles (:419-436), then the backward co-state
   //      pass and the control update of the same 32 steps (:277, :439-451) ----------------------------------
@@ -388,7 +388,7 @@ __global__ void __launch_bounds__(WARPS * 32, WARPS == kSolveWarps ? Solve2Cfg<N
       double R1[TILES][2], R2[TILES][2];
 #pragma unroll
       for (int mi = 0; mi < TILES; mi++) R1[mi][0] = R1[mi][1] = R2[mi][0] = R2[mi][1] = 0.0;
-      double akx = (double)q * p.ax;
+      double akx = (double)q * frame<PER_INST, kFrAx>(p, inst);
 #pragma unroll
       for (int ks = 0; ks < GKS; ks++)
       {
@@ -420,7 +420,7 @@ __global__ void __launch_bounds__(WARPS * 32, WARPS == kSolveWarps ? Solve2Cfg<N
         {
           const double2 cy2 = *reinterpret_cast<const double2*>(tyc + ky * 8 + 2 * q);
           const double2 sy2 = *reinterpret_cast<const double2*>(tys + ky * 8 + 2 * q);
-          const double bky = (double)ky * p.by;
+          const double bky = (double)ky * frame<PER_INST, kFrBy>(p, inst);
           v0 = fma(cy2.x, R1[mi][0], v0);
           v1 = fma(cy2.y, R1[mi][1], v1);
           w0 = fma(sy2.x, bky * R2[mi][0], w0);
@@ -465,8 +465,8 @@ __global__ void __launch_bounds__(WARPS * 32, WARPS == kSolveWarps ? Solve2Cfg<N
     }
     // gradBarrier :454-474
     double bx = 0.0, byv = 0.0;
-    bx += 2.0 * (double)(xf > p.lx - p.beps) * (xf - (p.lx - p.beps));
-    byv += 2.0 * (double)(yf > p.ly - p.beps) * (yf - (p.ly - p.beps));
+    bx += 2.0 * (double)(xf > frame<PER_INST, kFrLx>(p, inst) - p.beps) * (xf - (frame<PER_INST, kFrLx>(p, inst) - p.beps));
+    byv += 2.0 * (double)(yf > frame<PER_INST, kFrLy>(p, inst) - p.beps) * (yf - (frame<PER_INST, kFrLy>(p, inst) - p.beps));
     bx += 2.0 * (double)(xf < p.beps) * (xf - p.beps);
     byv += 2.0 * (double)(yf < p.beps) * (yf - p.beps);
     bx *= p.bw;

@@ -370,6 +370,36 @@ long long eb_map_target_launch_count(const eb_map_target *m);
 /* phik_ <- a device buffer of K doubles (stream-ordered copy), basis extent (lx, ly) */
 eb_status eb_set_phik_dev(eb_controller *c, const double *phik_dev, double lx, double ly);
 
+/* ---- per-instance targets ----------------------------------------------------------------------------------------
+ * Every instance owns its target, phi_k and map frame, as B reference ErgodicControl objects each driven with its own
+ * GridMap would.  The first of these calls switches the controller to per-instance mode; from then on the shared target
+ * calls (eb_set_target_gaussians, eb_config_target, eb_set_phik, eb_set_phik_dev, eb_get_phik, eb_control_host / _dev)
+ * return EB_ERR_INVALID_ARGUMENT and eb_control_dev_gather[_wait] EB_ERR_UNSUPPORTED.  Layouts are column-major
+ * (Armadillo): instance i owns column i.
+ * eb_set_target_gaussians_batch: Target::setTarget per instance; counts[i] <= max_n <= 256 Gaussians of instance i in
+ *   columns of mu / sigma (2 x max_n x B).  Does not rebuild phi_k by itself.
+ * eb_config_target_batch_dev: configTarget (ergodic_control.hpp:363-416) of every instance in one launch, bounds_dev
+ *   4 x B {xmin xmax ymin ymax}.  The origin is always recorded; phi_k is rebuilt where the extent moved by >= 1e-12
+ *   (rebuilt_dev[i] = 1).  A moved extent without Gaussians or a non-positive one is reported by the next synchronising
+ *   call (eb_check_status, eb_control_batch_host) as EB_ERR_INVALID_ARGUMENT.
+ * eb_set_phik_batch_dev: phi_k rows (K x B, device) and extents (2 x B {lx, ly}, device); origins are kept.  The
+ *   map-derived flow: eb_map_target_execute_dev(mt, cells, phik_dev + i * K, NULL) per instance into its column, then
+ *   one eb_set_phik_batch_dev.
+ * eb_control_batch_dev / _host: eb_control_dev / _host with per-instance bounds (4 x B, device / host).  bounds NULL:
+ *   the frames of the last configure are used and no frame launch is made (the per-tick fast path). */
+eb_status eb_set_target_gaussians_batch(eb_controller *c, int max_n, const int *counts /* B */,
+                                        const double *mu /* 2 x max_n x B */, const double *sigma /* 2 x max_n x B */);
+eb_status eb_set_phik_batch_dev(eb_controller *c, const double *phik_dev /* K x B */,
+                                const double *extent_dev /* 2 x B: lx, ly */);
+eb_status eb_get_phik_batch(const eb_controller *c, double *phik /* K x B, may be NULL */,
+                            double *extent /* 2 x B, may be NULL */);
+eb_status eb_config_target_batch_dev(eb_controller *c, const double *bounds_dev /* 4 x B: xmin xmax ymin ymax */,
+                                     int *rebuilt_dev /* B, may be NULL */);
+eb_status eb_control_batch_dev(eb_controller *c, const double *bounds_dev, const double *x_dev, const int *mem_idx_dev,
+                               double *u0_dev, double *metric_dev);
+eb_status eb_control_batch_host(eb_controller *c, const double *bounds, const double *x, const int *mem_idx,
+                                double *u0, double *metric);
+
 /* ---- kinematic models and the forward integrator (SURVEY.md section 8 rows a8 / a9) ----
  * model: 0 SimpleCart, 1 Omni (models/cart.hpp:152-206, models/omni.hpp:164-215), 2 Cart (cart.hpp:60-145;
  * params = { wheel_radius, wheel_base }; 2 wheel velocities), 3 Mecanum (omni.hpp:59-157; params = { wheel_radius,

@@ -33,6 +33,7 @@
 #include <string>
 #include <type_traits>
 #include <utility>
+#include <algorithm>
 #include <vector>
 
 #include <armadillo>
@@ -695,6 +696,44 @@ public:
     std::vector<double> mu, sg;
     target.pack(mu, sg);
     b200::check(eb_set_target_gaussians(h_.get(), int(target.gaussians().size()), mu.data(), sg.data()));
+  }
+  /** @brief one target per instance (targets.size() == B); switches the controller to per-instance targets */
+  void setTargets(const std::vector<Target>& targets)
+  {
+    if (targets.size() != batch_) throw std::logic_error("BatchedErgodicControl::setTargets: need B targets");
+    int max_n = 1;
+    for (const Target& t : targets) max_n = std::max(max_n, int(t.gaussians().size()));
+    std::vector<int> counts(batch_);
+    std::vector<double> mu(2 * size_t(max_n) * batch_, 0.0), sg(2 * size_t(max_n) * batch_, 1.0);
+    for (unsigned int i = 0; i < batch_; i++)
+    {
+      std::vector<double> m, s;
+      targets[i].pack(m, s);
+      counts[i] = int(targets[i].gaussians().size());
+      std::copy(m.begin(), m.end(), mu.begin() + 2 * size_t(max_n) * i);
+      std::copy(s.begin(), s.end(), sg.begin() + 2 * size_t(max_n) * i);
+    }
+    b200::check(eb_set_target_gaussians_batch(h_.get(), max_n, counts.data(), mu.data(), sg.data()));
+  }
+  /** @brief per-instance maps: instance i is driven in grids[i]'s frame (after setTargets) */
+  template <class GridT>
+  mat control(const std::vector<GridT>& grids, const mat& x, vec* metric = nullptr)
+  {
+    if (x.n_rows != 3 || x.n_cols != batch_) throw std::logic_error("BatchedErgodicControl::control: x must be 3 x B");
+    if (grids.size() != batch_) throw std::logic_error("BatchedErgodicControl::control: need B grids");
+    std::vector<double> bounds(4 * size_t(batch_));
+    for (unsigned int i = 0; i < batch_; i++)
+    {
+      bounds[4 * i + 0] = grids[i].xmin();
+      bounds[4 * i + 1] = grids[i].xmax();
+      bounds[4 * i + 2] = grids[i].ymin();
+      bounds[4 * i + 3] = grids[i].ymax();
+    }
+    mat u0(3, batch_);
+    if (metric) metric->set_size(batch_);
+    b200::check(eb_control_batch_host(h_.get(), bounds.data(), x.memptr(), nullptr, u0.memptr(),
+                                      metric ? metric->memptr() : nullptr));
+    return u0;
   }
   /** @brief 3 x (steps * B): instance i occupies columns [i*steps, (i+1)*steps) */
   mat optTraj() const

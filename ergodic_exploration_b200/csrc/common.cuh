@@ -111,7 +111,8 @@ __device__ __forceinline__ void sincos_kernel(double r, int n, double* s, double
 // VALUE: with pointer outputs the callers' sin / cos variables become
 // address-taken stack objects, and the fused kernel built with nvcc 12.9 then
 // produced wrong fast-path values (reproduced and bisected with
-// tools/diag_dump.py: -DEB_NO_SLOWPATH or this by-value form are both correct).
+// tools/diag_dump.py: dropping the slow path, or returning by value as here,
+// both give correct values).
 __device__ __noinline__ double2 slow_sincos2(double x)
 {
   double s, c;
@@ -128,7 +129,6 @@ __device__ __noinline__ double2 slow_sincospi2(double x)
 __device__ __forceinline__ void fast_sincos(double x, double* s, double* c)
 {
   double sv, cv;
-#ifndef EB_NO_SLOWPATH
   if (fabs(x) > 1073741824.0)
   {
     const double2 v = slow_sincos2(x);
@@ -136,7 +136,6 @@ __device__ __forceinline__ void fast_sincos(double x, double* s, double* c)
     cv = v.y;
   }
   else
-#endif
   {
     const double q = rint(x * kTrigR[0]);
     double r = fma(-q, kTrigR[1], x);
@@ -151,7 +150,6 @@ __device__ __forceinline__ void fast_sincos(double x, double* s, double* c)
 __device__ __forceinline__ void fast_sincospi(double t, double* s, double* c)
 {
   double sv, cv;
-#ifndef EB_NO_SLOWPATH
   if (fabs(t) > 1073741824.0)
   {
     const double2 v = slow_sincospi2(t);
@@ -159,7 +157,6 @@ __device__ __forceinline__ void fast_sincospi(double t, double* s, double* c)
     cv = v.y;
   }
   else
-#endif
   {
     const double q = rint(t + t);
     const double f = fma(-0.5, q, t);  // exact, |f| <= 1/4

@@ -616,32 +616,9 @@ inline bool replay_cos_cache()
   return v;
 }
 
-// EB_SOLVE_PDL=0 turns programmatic dependent launch of the per-step kernels off
-inline bool solve_pdl()
-{
-  static const bool v = [] {
-    const char* e = std::getenv("EB_SOLVE_PDL");
-    return !e || std::atoi(e) != 0;
-  }();
-  return v;
-}
-
 namespace
 {
-// num_basis 13..24 run solve_kernel2 (solve_kernel_v2.cuh); EB_SOLVE_V1=1 keeps the round-1 kernel for A/B timing
-inline bool use_v2(int nb)
-{
-  static const bool v1 = [] {
-    const char* e = std::getenv("EB_SOLVE_V1");
-    return e && std::atoi(e) != 0;
-  }();
-  static const bool small = [] {  // experiment: the v2 kernel for num_basis 9..12 as well
-    const char* e = std::getenv("EB_SOLVE_V2_SMALL");
-    return e && std::atoi(e) != 0;
-  }();
-  return !v1 && nb > (small ? 8 : 12) && nb <= 24;
-}
-
+// V2: solve_kernel2 (solve_kernel_v2.cuh), else solve_kernel (solve_kernel.cuh)
 template <int MODEL, int NB, bool V2, bool PER_INST = false>
 struct SolveLaunch
 {
@@ -681,8 +658,7 @@ struct SolveLaunch
     const int grid = (p.B + WARPS - 1) / WARPS;
     // Programmatic dependent launch: consecutive control() steps on one stream are kernel -> kernel dependencies; the
     // next step's CTAs may be placed while this step's last ones drain (every global access of the kernel sits behind
-    // its griddepcontrol.wait, so the data dependency is the stream's).  EB_SOLVE_PDL=0 turns it off.
-    static const bool pdl = solve_pdl();
+    // its griddepcontrol.wait, so the data dependency is the stream's).
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)grid);
     cfg.blockDim = dim3((unsigned)(WARPS * 32));
@@ -692,12 +668,11 @@ struct SolveLaunch
     at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     at[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = at;
-    cfg.numAttrs = pdl ? 1 : 0;
+    cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kernel, p);
   }
-  static cudaError_t launch(const eb::SolveParams& p, int rounds, cudaStream_t s)
+  static cudaError_t launch(const eb::SolveParams& p, cudaStream_t s)
   {
-    (void)rounds;
     // a batch that fits one wave of wide CTAs (one per SM) starts all of an SM's instances together
     static const int sms = [] {
       int dev = 0, n = 148;
@@ -761,56 +736,45 @@ int solve_big_resident(int nb, int N)
   return sms * std::max(1, per_sm);
 }
 
-template <int MODEL, bool PER_INST>
-cudaError_t launch_solve_m(const eb::SolveParams& p, int rounds, cudaStream_t s)
+// The solve kernel that serves num_basis `nb` <= 32: f is called with a (stateless) value of its SolveLaunch type.
+//   nb <= 8 | <= 10 | <= 12  -> solve_kernel<8 | 10 | 12>
+//   13..16 | 17..20 | 21..24 -> solve_kernel2<16 | 20 | 24>
+//   25..32                   -> solve_kernel<32>
+// nb > 32 runs solve_kernel_big (launch_solve_big).
+template <int MODEL, bool PER_INST, class F>
+auto with_solve_launch(int nb, F&& f)
 {
-  const int nb = p.nb;
-  if (nb > 32) return launch_solve_big<MODEL, PER_INST>(p, s);
-  if (nb <= 8) return SolveLaunch<MODEL, 8, false, PER_INST>::launch(p, rounds, s);
-  if (nb <= 12 && use_v2(nb))
-    return nb <= 10 ? SolveLaunch<MODEL, 10, true, PER_INST>::launch(p, rounds, s) : SolveLaunch<MODEL, 12, true, PER_INST>::launch(p, rounds, s);
-  if (nb <= 10) return SolveLaunch<MODEL, 10, false, PER_INST>::launch(p, rounds, s);
-  if (nb <= 12) return SolveLaunch<MODEL, 12, false, PER_INST>::launch(p, rounds, s);
-  if (use_v2(nb))
-  {
-    if (nb <= 16) return SolveLaunch<MODEL, 16, true, PER_INST>::launch(p, rounds, s);
-    if (nb <= 20) return SolveLaunch<MODEL, 20, true, PER_INST>::launch(p, rounds, s);
-    return SolveLaunch<MODEL, 24, true, PER_INST>::launch(p, rounds, s);
-  }
-  if (nb <= 16) return SolveLaunch<MODEL, 16, false, PER_INST>::launch(p, rounds, s);
-  if (nb <= 20) return SolveLaunch<MODEL, 20, false, PER_INST>::launch(p, rounds, s);
-  if (nb <= 24) return SolveLaunch<MODEL, 24, false, PER_INST>::launch(p, rounds, s);
-  return SolveLaunch<MODEL, 32, false, PER_INST>::launch(p, rounds, s);
+  if (nb <= 8) return f(SolveLaunch<MODEL, 8, false, PER_INST>{});
+  if (nb <= 10) return f(SolveLaunch<MODEL, 10, false, PER_INST>{});
+  if (nb <= 12) return f(SolveLaunch<MODEL, 12, false, PER_INST>{});
+  if (nb <= 16) return f(SolveLaunch<MODEL, 16, true, PER_INST>{});
+  if (nb <= 20) return f(SolveLaunch<MODEL, 20, true, PER_INST>{});
+  if (nb <= 24) return f(SolveLaunch<MODEL, 24, true, PER_INST>{});
+  return f(SolveLaunch<MODEL, 32, false, PER_INST>{});
 }
 
-// dynamic shared memory of the solve kernel instantiation that serves `nb` (same dispatch as launch_solve_m)
+template <int MODEL, bool PER_INST>
+cudaError_t launch_solve_m(const eb::SolveParams& p, cudaStream_t s)
+{
+  if (p.nb > 32) return launch_solve_big<MODEL, PER_INST>(p, s);
+  return with_solve_launch<MODEL, PER_INST>(p.nb, [&](auto L) { return decltype(L)::launch(p, s); });
+}
+
+// dynamic shared memory of the solve kernel that serves `nb` (the model does not change it)
 size_t solve_smem_for(int nb, int N)
 {
   if (nb > 32) return eb::solve_big_smem_bytes(nb, N);
-  if (nb <= 8) return SolveLaunch<0, 8, false>::smem(N);
-  if (nb <= 12 && use_v2(nb)) return nb <= 10 ? SolveLaunch<0, 10, true>::smem(N) : SolveLaunch<0, 12, true>::smem(N);
-  if (nb <= 10) return SolveLaunch<0, 10, false>::smem(N);
-  if (nb <= 12) return SolveLaunch<0, 12, false>::smem(N);
-  if (use_v2(nb))
-  {
-    if (nb <= 16) return SolveLaunch<0, 16, true>::smem(N);
-    if (nb <= 20) return SolveLaunch<0, 20, true>::smem(N);
-    return SolveLaunch<0, 24, true>::smem(N);
-  }
-  if (nb <= 16) return SolveLaunch<0, 16, false>::smem(N);
-  if (nb <= 20) return SolveLaunch<0, 20, false>::smem(N);
-  if (nb <= 24) return SolveLaunch<0, 24, false>::smem(N);
-  return SolveLaunch<0, 32, false>::smem(N);
+  return with_solve_launch<0, false>(nb, [&](auto L) { return decltype(L)::smem(N); });
 }
 
 // per_inst: the kernels read each instance's frame and phi_k row (p.frames, p.phik [B][K])
-cudaError_t launch_solve(const eb::SolveParams& p, int model, int rounds, cudaStream_t s, bool per_inst)
+cudaError_t launch_solve(const eb::SolveParams& p, int model, cudaStream_t s, bool per_inst)
 {
   if (per_inst)
-    return model == EB_MODEL_OMNI ? launch_solve_m<eb::kModelOmni, true>(p, rounds, s) :
-                                    launch_solve_m<eb::kModelSimpleCart, true>(p, rounds, s);
-  return model == EB_MODEL_OMNI ? launch_solve_m<eb::kModelOmni, false>(p, rounds, s) :
-                                  launch_solve_m<eb::kModelSimpleCart, false>(p, rounds, s);
+    return model == EB_MODEL_OMNI ? launch_solve_m<eb::kModelOmni, true>(p, s) :
+                                    launch_solve_m<eb::kModelSimpleCart, true>(p, s);
+  return model == EB_MODEL_OMNI ? launch_solve_m<eb::kModelOmni, false>(p, s) :
+                                  launch_solve_m<eb::kModelSimpleCart, false>(p, s);
 }
 
 eb_status ensure_hist(eb_controller* c, long long need)
@@ -1440,8 +1404,7 @@ static eb_status solve_step(eb_controller* c, const double* x_dev, const int* me
     p.my_flags = c->peer->my_flags;
     p.need = c->peer->need;
   }
-  const int rounds = (c->N + 31) / 32;
-  cudaError_t e = launch_solve(p, c->cfg.model, rounds, c->stream, c->per_inst);
+  cudaError_t e = launch_solve(p, c->cfg.model, c->stream, c->per_inst);
   if (e != cudaSuccess) return fail(EB_ERR_CUDA, std::string("solve_kernel launch: ") + cudaGetErrorString(e));
   c->launches += 1;
   c->cur ^= 1;
@@ -1960,7 +1923,7 @@ eb_status eb_control_dev_gather_wait(eb_controller* c, eb_peer_group* g, double 
     at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     at[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = at;
-    cfg.numAttrs = solve_pdl() ? 1 : 0;
+    cfg.numAttrs = 1;
     EB_CUDA(cudaLaunchKernelEx(&cfg, eb::peer_publish_wait_kernel, pp));
   }
   c->launches += 1;
@@ -2796,15 +2759,6 @@ eb_status eb_map_target_extent(const eb_map_target* m, double* lx, double* ly)
   return EB_OK;
 }
 
-static bool map_fused_enabled()
-{
-  static const bool v = [] {
-    const char* e = std::getenv("EB_MAP_FUSED");
-    return !e || std::atoi(e) != 0;
-  }();
-  return v;
-}
-
 // the density of the last execute's cells, materialised (allocated on first use)
 static eb_status map_density(eb_map_target* m)
 {
@@ -2830,10 +2784,11 @@ eb_status eb_map_target_execute_dev(eb_map_target* m, const signed char* cells_d
   m->last_cells = cells_dev;
   m->density_valid = false;
   // ONE kernel when the folded TMA tile kernel applies: the bytes are staged by TMA and the entropy table is looked up in
-  // shared memory -- the 8 B / cell density is never written (EB_MAP_FUSED=0: always the two-kernel route)
+  // shared memory -- the 8 B / cell density is never written.  Every other input takes the two-kernel route: the
+  // density, then the plan's phi_k.
   eb_phik_plan* const pl = m->plan;
   const bool big = (long long)pl->nx * pl->ny >= (1 << 18);  // as phik_execute: small grids take the simple kernels
-  if (map_fused_enabled() && pl->fold && pl->d_cxtf && (pl->algo == 4 || (pl->algo == 0 && big)) && !pl->peer &&
+  if (pl->fold && pl->d_cxtf && (pl->algo == 4 || (pl->algo == 0 && big)) && !pl->peer &&
       eb::phik_tma_u8_supported(pl->nx, pl->ny) && eb::phik_tma_encoder() && (reinterpret_cast<uintptr_t>(cells_dev) & 15) == 0)
   {
     const eb::PhikTmaOut out{ pl->d_done, pl->nb, phik_dev, phi_sum_dev, nullptr, nullptr };

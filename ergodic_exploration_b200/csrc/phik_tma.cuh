@@ -48,10 +48,7 @@ struct PtGeom
   static constexpr int kPhiBytes = U8 ? 2 * kPtU8BoxBytes : kBoxes * kPtBoxBytes;  // 4 KB | 32 KB
   static constexpr int kCxBytes = kCols * kPdPitch * 8;    // 9 / 18 KB
   static constexpr int kStageBytes = kPhiBytes + ((kCxBytes + 1023) / 1024) * 1024;
-#ifndef EB_PT_STAGES_FOLD
-#define EB_PT_STAGES_FOLD 4
-#endif
-  static constexpr int kStages = U8 ? 6 : (FOLD ? EB_PT_STAGES_FOLD : 3);
+  static constexpr int kStages = U8 ? 6 : (FOLD ? 4 : 3);
   static constexpr int kKSteps = kCols / 16;               // k-steps per warp and stage (a quarter of the columns, 4 per step)
   static constexpr int kLutBytes = U8 ? 256 * 8 : 0;
   static constexpr int kSmemBytes =
@@ -406,12 +403,8 @@ __global__ void __launch_bounds__(kPtThreads, 1)
   __shared__ unsigned int s_last;
   __shared__ double s_total;
   const int nparts = (int)gridDim.x;
-#ifdef EB_PT_FLATSUM
-  const int ngroups = 1, g_lo = 0, g_n = nparts, grp = 0;
-#else
   const int ngroups = (nparts + kPtGroup - 1) / kPtGroup;
   const int grp = (int)blockIdx.x / kPtGroup, g_lo = grp * kPtGroup, g_n = min(kPtGroup, nparts - g_lo);
-#endif
   __threadfence();
   pt_consumer_barrier();
   if (threadIdx.x == 0) s_last = atomicAdd(p.done + 1 + grp, 1u) == (unsigned)(g_n - 1) ? 1u : 0u;
@@ -530,10 +523,7 @@ inline bool phik_tma_make_map(const double* phi, int nx, int ny, CUtensorMap* ma
   const cuuint32_t box[2] = { (cuuint32_t)kPtBox, (cuuint32_t)kPtRows };
   const cuuint32_t estr[2] = { 1, 1 };
   return enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 2, const_cast<double*>(phi), dims, strides, box, estr,
-#ifndef EB_PT_L2PROMO
-#define EB_PT_L2PROMO CU_TENSOR_MAP_L2_PROMOTION_L2_256B
-#endif
-             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, EB_PT_L2PROMO,
+             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 

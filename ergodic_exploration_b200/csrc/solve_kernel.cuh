@@ -22,15 +22,15 @@
 //    warp contracts them with FP64 tensor-core tiles (mma.sync m8n8k4 ->
 //    DMMA.8x8x4), accumulators in registers.
 //  * the metric gradient is a pair of bilinear forms per step,
-//    sx^T (a.S) cy and cx^T (S.b) sy.  nb = 16 / 20 / 24: S sits in registers as
-//    DMMA A fragments and 8-step tiles of cos / sin tables are contracted on the
-//    tensor cores ("DMMA gradient" below); otherwise each lane evaluates them for
-//    its own time step with S broadcast from shared memory, cos/sin rows of a kx
-//    block held in registers.
+//    sx^T (a.S) cy and cx^T (S.b) sy: each lane evaluates them for its own time
+//    step with S broadcast from shared memory, cos/sin rows of a kx block held in
+//    registers.
 //  * N > 1 GPUs: the first twists are published to every rank over NVLink peer
 //    memory by this kernel itself (peer_gather.cuh).
-// Shared memory per warp: SolveCfg::kTabDoubles (the c_k or the gradient tables,
-// S aliases them) + (4 or 8)*32*rounds doubles of per-step records.
+// This kernel serves num_basis <= 12 and 25..32; 13..24 run solve_kernel2
+// (solve_kernel_v2.cuh), which also puts the gradient on the tensor cores.
+// Shared memory per warp: SolveCfg::kTabDoubles (the two c_k tables, S aliases
+// them) + (4 or 8)*32*rounds doubles of per-step records.
 #pragma once
 
 #include "common.cuh"
@@ -39,23 +39,10 @@ namespace eb
 {
 constexpr int kModelSimpleCart = 0;
 constexpr int kModelOmni = 1;
-#ifndef EB_SOLVE_WARPS
-#define EB_SOLVE_WARPS 4
-#endif
-constexpr int kSolveWarps = EB_SOLVE_WARPS;  // warps (instances in flight) per CTA
+constexpr int kSolveWarps = 4;   // warps (instances in flight) per CTA
 constexpr int kMaxPeers = 8;     // ranks of one NVSwitch box
 constexpr int kPeerBuffers = 4;  // gathered buffers rotating by step (fused gather)
 constexpr int kTabSlots = 16;    // time slots per coefficient chunk (half a round)
-constexpr int kGradPitch = 12;   // gradient x tables: 8 slots + 4 pad, 12 % 16 -> conflict-free fragment loads
-#ifndef EB_BANKFIX
-#define EB_BANKFIX 1
-#endif
-// y tables: pitch 8 puts consecutive rows 16 banks apart -> conflict-free LDS.128 of (t, t+1) pairs
-constexpr int kGradPitchY = EB_BANKFIX ? 8 : 12;
-// table stride: +8 doubles so the cos | sin tables written by one half-warp start 16 banks apart
-__host__ __device__ constexpr int grad_tab_stride(int nb) { return nb * kGradPitch + (EB_BANKFIX ? 8 : 0); }
-// S (NB x NB) in shared memory: pitch = 4 or 12 (mod 16) -> conflict-free A-fragment loads
-__host__ __device__ constexpr int s_pitch(int nb) { return (EB_BANKFIX && nb % 8 == 0) ? nb + 4 : nb; }
 constexpr int kTabStride = 20;   // 16 slots + 4 pad: 20 % 16 == 4 -> conflict-free fragment loads
 
 #ifdef EB_PHASE_TIMING
@@ -77,9 +64,9 @@ __device__ double g_dbg[4096 * 16];  // debug build only: per-step intermediates
 
 // Ablation timing (tools/ablate.sh; debug builds only, results are numerically WRONG): -DEB_ABL=<bits> removes a
 // class of work from the fused kernel so that its marginal cost can be read off the kernel time.
-//  1: c_k DMMAs -> integer xor of the operands   2: gradient DMMAs -> xor   4: c_k table recurrences + stores
-//  8: sin/cos polynomials -> 2 flops            16: gradient table recurrences + stores   64: warp scans -> identity
-//  128: v1 kernel returns at once (launch + drain cost of the grid)
+//  1: c_k DMMAs -> integer xor of the operands   2: gradient DMMAs (solve_kernel2) -> xor   4: c_k table recurrences
+//  + stores   8: sin/cos polynomials -> 2 flops   64: warp scans -> identity
+//  128: solve_kernel returns at once (launch + drain cost of the grid)
 #ifndef EB_ABL
 #define EB_ABL 0
 #endif
@@ -430,46 +417,21 @@ __device__ __forceinline__ void coeff_chunk(double* __restrict__ tabx, const int
 //  * kBlock: the gradient's kx range is walked in blocks of kBlock orders so that
 //    only 2 kBlock doubles of cos / sin rows are live in registers.
 //  * kMinBlocks: resident CTAs per SM the register allocation is tuned for.
-#ifndef EB_DMMA_GRAD
-#define EB_DMMA_GRAD 1
-#endif
-#ifndef EB_DMMA_GRAD_SMALL
-#define EB_DMMA_GRAD_SMALL 0
-#endif
-#ifndef EB_KB_16
-#define EB_KB_16 8
-#endif
-#ifndef EB_KB_20
-#define EB_KB_20 20
-#endif
-#ifndef EB_MINB_10  // tuning overrides (tools/variants.sh)
-#define EB_MINB_10 7
-#endif
-#ifndef EB_MINB_16
-#define EB_MINB_16 6
-#endif
-#ifndef EB_MINB_20
-#define EB_MINB_20 4
-#endif
+// Instantiated for NB = 8, 10, 12 and 32 (num_basis 13..24 run solve_kernel2).
 template <int NB>
 struct SolveCfg
 {
   static constexpr bool kRecompute = NB >= 16;
   static constexpr int kFields = kRecompute ? 4 : 8;
-  // gradient on the FP64 tensor cores (see "DMMA gradient" in solve_kernel): pays when the
-  // 8-row / 4-order tile padding is small, i.e. not for nb <= 12; nb = 32 would need 128
-  // registers of S fragments
-  static constexpr bool kDmmaGrad = EB_DMMA_GRAD && (NB == 16 || NB == 20 || NB == 24 || (EB_DMMA_GRAD_SMALL && NB <= 12));
-  // per-warp table region: the two c_k tables (pitch 20, 16 slots) or the four gradient
-  // tables (pitch 12, 8 slots), whichever is larger; S (NB x NB) aliases it
-  static constexpr int kSPitch = kDmmaGrad ? s_pitch(NB) : NB;
-  static constexpr int kTabDoubles = kDmmaGrad ? (4 * grad_tab_stride(NB) > NB * kSPitch ? 4 * grad_tab_stride(NB) : NB * kSPitch) : 2 * NB * kTabStride;
-  static constexpr int kBlock = NB <= 12 ? NB : (NB == 20 ? EB_KB_20 : NB == 16 ? EB_KB_16 : 8);
-  static constexpr int kMinBlocks =
-      (NB <= 10 ? EB_MINB_10 : NB <= 12 ? 6 : NB <= 16 ? EB_MINB_16 : NB <= 24 ? EB_MINB_20 : 4) * 4 / kSolveWarps;
+  // per-warp table region: the two c_k tables (pitch 20, 16 slots); S (NB x NB, pitch NB) aliases it
+  static constexpr int kSPitch = NB;
+  static constexpr int kTabDoubles = 2 * NB * kTabStride;
+  static constexpr int kBlock = NB <= 12 ? NB : 8;
+  static constexpr int kMinBlocks = NB <= 10 ? 7 : NB <= 12 ? 6 : 4;
   // Single-wave batches (configs[1]: 4096 instances on 148 SMs) run ONE CTA per SM with this many warps: the SM's
   // instances then start together instead of behind 7 serial CTA launches (measured 34.9 -> 31.2 us at 4096 x nb 10)
-  static constexpr int kWideWarps = NB <= 10 ? 28 : NB <= 16 ? 24 : 16;
+  static constexpr int kWideWarps = NB <= 10 ? 28 : NB <= 12 ? 24 : 16;
+  static_assert(NB <= 12 || NB == 32, "num_basis 13..24 run solve_kernel2");
   static_assert(NB % kBlock == 0, "kx blocks must tile NB");
 };
 
@@ -493,7 +455,6 @@ __global__ void __launch_bounds__(WARPS * 32, WARPS == kSolveWarps ? SolveCfg<NB
   const int inst = blockIdx.x * WARPS + warp;
   __shared__ WideIo<WARPS> wio;
   grid_dependency_wait();  // programmatic dependent launch: nothing global is touched before the previous kernel is complete
-#ifndef EB_NO_EARLY_UT
   // the first round's controls do not depend on the pose: their HBM latency runs under the pose staging (which may be a
   // PCIe round trip on the zero-copy host path) instead of behind it
   double e_u0 = 0.0, e_u1 = 0.0, e_u2 = 0.0;
@@ -504,16 +465,11 @@ __global__ void __launch_bounds__(WARPS * 32, WARPS == kSolveWarps ? SolveCfg<NB
     e_u1 = e_in[1];
     e_u2 = e_in[2];
   }
-#endif
   if constexpr (WideIo<WARPS>::kOn) wide_io_load(wio, p);
   if (inst >= p.B) return;
 #if EB_ABL & 128
   if (lane < 3) p.u0[(size_t)inst * 3 + lane] = 0.0;  // ablation timing only: the launch itself
   return;
-#endif
-#ifdef EB_STAGGER_NS
-  // experiment: de-phase the warps of a single-wave launch (every warp runs the same phases in lockstep otherwise)
-  if (WARPS > kSolveWarps) __nanosleep((unsigned)(EB_STAGGER_NS) * (unsigned)(warp % EB_STAGGER_GROUPS));
 #endif
   EB_PHASE(0);
 
@@ -592,16 +548,13 @@ __global__ void __launch_bounds__(WARPS * 32, WARPS == kSolveWarps ? SolveCfg<NB
     const int i = r * 32 + lane;
     const bool valid = i < p.N;
     double u0 = 0.0, u1 = 0.0, u2 = 0.0;
-#ifndef EB_NO_EARLY_UT
     if (r == 0)
     {
       u0 = e_u0;
       u1 = e_u1;
       u2 = e_u2;
     }
-    else
-#endif
-    if (i + 1 < p.N)
+    else if (i + 1 < p.N)
     {  // shift left by one column, last column zero
       u0 = ut_in[(i + 1) * 3 + 0];
       u1 = ut_in[(i + 1) * 3 + 1];
@@ -677,32 +630,6 @@ __global__ void __launch_bounds__(WARPS * 32, WARPS == kSolveWarps ? SolveCfg<NB
   // ---- per round, last round first: gradient of the ergodic metric, one time
   //      step per lane (:419-436), then the backward co-state pass and the
   //      control update of the same 32 steps (:277, :439-451) -------------------
-  // DMMA gradient (Cfg::kDmmaGrad).  R1 = (S diag(a_kx)) SX and R2 = (diag(b_ky) S) CX for the
-  // 8 time steps of a tile, SX[kx][t] = sin(kx a x_t), CX[kx][t] = cos(kx a x_t), are
-  // products of an nb x nb matrix with an nb x 8 table: S sits in registers as A fragments
-  // (folded with a_kx / b_ky once per instance), the tables are built per tile by the whole
-  // warp -- lane (axis, cos | sin, slot) runs one even/odd Chebyshev-type recurrence -- and
-  // e_x(t) = -w sum_ky cos(ky b y_t) R1[ky][t], e_y(t) = -w sum_ky sin(ky b y_t) R2[ky][t] are a
-  // fragment-wise product with the y tables and a recursive-halving reduction over the 8
-  // row lanes.  Tiles are 8 steps wide, so N = 50 costs 7 tiles instead of two full rounds.
-  constexpr int GKS = (NB + 3) / 4;  // k-steps over kx
-  double SA[Cfg::kDmmaGrad ? TILES : 1][Cfg::kDmmaGrad ? GKS : 1], SB[Cfg::kDmmaGrad ? TILES : 1][Cfg::kDmmaGrad ? GKS : 1];
-  if constexpr (Cfg::kDmmaGrad)
-  {
-    const int g = lane >> 2, q = lane & 3;
-#pragma unroll
-    for (int mi = 0; mi < TILES; mi++)
-#pragma unroll
-      for (int ks = 0; ks < GKS; ks++)
-      {
-        const int ky = 8 * mi + g, kx = 4 * ks + q;
-        const double sv = (ky < NB && kx < NB) ? Ssm[ky * Cfg::kSPitch + kx] : 0.0;
-        SA[mi][ks] = sv * ((double)kx * frame<PER_INST, kFrAx>(p, inst));
-        SB[mi][ks] = sv * ((double)ky * frame<PER_INST, kFrBy>(p, inst));
-      }
-    __syncwarp();  // S has been read: the table region is free for the gradient tables
-  }
-
   double r0c = 0.0, r1c = 0.0, r2c = 0.0;  // rho(T) = 0 (:203)
   for (int r = rounds - 1; r >= 0; r--)
   {
@@ -710,14 +637,12 @@ __global__ void __launch_bounds__(WARPS * 32, WARPS == kSolveWarps ? SolveCfg<NB
     const bool valid = i < p.N;
     const double ce = rec[0 * npad + i], se = rec[1 * npad + i];
     const double xf = rec[2 * npad + i], yf = rec[3 * npad + i];
-#ifndef EB_NO_EARLY_BWD
     double u0 = 0.0, u1 = 0.0;  // issued ahead of the gradient: their L2 latency runs under it (C2: 22.55 -> 22.42 us)
     if (i + 1 < p.N)
     {
       u0 = ut_in[(i + 1) * 3 + 0];
       u1 = ut_in[(i + 1) * 3 + 1];
     }
-#endif
     double ca, sa, cb, sb;
     if (Cfg::kRecompute)
     {
@@ -732,163 +657,46 @@ __global__ void __launch_bounds__(WARPS * 32, WARPS == kSolveWarps ? SolveCfg<NB
       sb = rec[7 * npad + i];
     }
     double ex = 0.0, ey = 0.0;
-    if constexpr (Cfg::kDmmaGrad)
+    // (cos, sin)((k-1) a x), (cos, sin)(k a x) started at k = 0, carried across the kx blocks
+    double xcm = ca, xck = 1.0, xsm = -sa, xsk = 0.0;
+    const double xt2 = 2.0 * ca, yt2 = 2.0 * cb;
+#pragma unroll
+    for (int kb = 0; kb < NB; kb += KB)
     {
-      const int g = lane >> 2, q = lane & 3;
-      const int axis = lane >> 4, chain = (lane >> 3) & 1, slot = lane & 7;
-      double* const gt = tabx;  // [axis][chain][k][12]: cos(kx a x) | sin(kx a x) | cos(ky b y) | sin(ky b y)
-      constexpr int TS = grad_tab_stride(NB);
-      const int mypitch = axis ? kGradPitchY : kGradPitch;
-      double* const mytab = gt + (axis * 2 + chain) * TS + slot;
-      const double* const txc = gt;
-      const double* const txs = gt + TS;
-      const double* const tyc = gt + 2 * TS;
-      const double* const tys = gt + 3 * TS;
-      // e_x / e_y of the round's 32 steps are handed to the time-step lanes through the pad
-      // slots (8..11) of rows 0..7 of the first two tables
-      auto stage = [&](int which, int t) { return gt + which * TS + (t >> 2) * kGradPitch + 8 + (t & 3); };
-      const int left = p.N - r * 32;  // valid steps in this round (warp-uniform)
-      const int ntiles = min(4, (left + 7) >> 3);
-      for (int nj = 0; nj < ntiles; nj++)
+      double cx[KB], asx[KB];  // cos(kx a x), a_kx sin(kx a x) for kx = kb .. kb + KB - 1
+#pragma unroll
+      for (int j = 0; j < KB; j++)
       {
-        const int src = 8 * nj + slot;
-        const double xc = __shfl_sync(kFull, ca, src), xs = __shfl_sync(kFull, sa, src);
-        const double yc = __shfl_sync(kFull, cb, src), ys = __shfl_sync(kFull, sb, src);
-        const bool ok = __shfl_sync(kFull, (int)valid, src) != 0;
-        const double c = axis ? yc : xc, sn = axis ? ys : xs;
-        // even / odd orders of cos(k t) (chain 0) or sin(k t) (chain 1): v_{k+2} = (4c^2 - 2) v_k - v_{k-2}
-        const double m = fma(4.0 * c, c, -2.0);
-        double em, ek, om, ok1;
-        if (chain == 0)
-        {
-          em = fma(2.0 * c, c, -1.0);  // cos(-2t)
-          ek = 1.0;
-          om = c;  // cos(-t)
-          ok1 = c;
-        }
-        else
-        {
-          em = -2.0 * sn * c;  // sin(-2t)
-          ek = 0.0;
-          om = -sn;  // sin(-t)
-          ok1 = sn;
-        }
-        if (!ok) em = ek = om = ok1 = 0.0;
-        __syncwarp();  // the previous tile's fragment / staging traffic is done
-#if EB_ABL & 16
-        mytab[0] = ek + ok1 + em * m;
-#else
-#pragma unroll
-        for (int k = 0; k < NB; k += 2)
-        {
-          mytab[k * mypitch] = ek;
-          mytab[(k + 1) * mypitch] = ok1;
-          const double en = fma(m, ek, -em), on = fma(m, ok1, -om);
-          em = ek;
-          ek = en;
-          om = ok1;
-          ok1 = on;
-        }
-#endif
-        __syncwarp();
-        double R1[TILES][2], R2[TILES][2];
-#pragma unroll
-        for (int mi = 0; mi < TILES; mi++) R1[mi][0] = R1[mi][1] = R2[mi][0] = R2[mi][1] = 0.0;
-#pragma unroll
-        for (int ks = 0; ks < GKS; ks++)
-        {
-          const int kx = 4 * ks + q;
-          const bool in = (GKS * 4 == NB) || (kx < NB);
-          const double bs = in ? txs[kx * kGradPitch + g] : 0.0;
-          const double bc = in ? txc[kx * kGradPitch + g] : 0.0;
-#pragma unroll
-          for (int mi = 0; mi < TILES; mi++)
-          {
-            dmma_gr(R1[mi][0], R1[mi][1], SA[mi][ks], bs);
-            dmma_gr(R2[mi][0], R2[mi][1], SB[mi][ks], bc);
-          }
-        }
-        // lane (g, q) holds R[ky = 8 mi + g][slot 2q, 2q + 1]: weight with the y tables
-        double v0 = 0.0, v1 = 0.0, w0 = 0.0, w1 = 0.0;  // e_x, e_y partial sums for slots 2q, 2q + 1
-#pragma unroll
-        for (int mi = 0; mi < TILES; mi++)
-        {
-          const int ky = 8 * mi + g;
-          if ((TILES * 8 == NB) || (ky < NB))
-          {
-            const double2 cy2 = *reinterpret_cast<const double2*>(tyc + ky * kGradPitchY + 2 * q);
-            const double2 sy2 = *reinterpret_cast<const double2*>(tys + ky * kGradPitchY + 2 * q);
-            v0 = fma(cy2.x, R1[mi][0], v0);
-            v1 = fma(cy2.y, R1[mi][1], v1);
-            w0 = fma(sy2.x, R2[mi][0], w0);
-            w1 = fma(sy2.y, R2[mi][1], w1);
-          }
-        }
-        // sum over the 8 row lanes g (lane = 4 g + q) by recursive halving:
-        //   xor 16: lanes g < 4 keep e_x, g >= 4 keep e_y;  xor 8: keep slot 2q (g & 2 == 0) or 2q + 1;  xor 4: full
-        {
-          const bool hi = (g & 4) != 0;
-          const double s0 = hi ? v0 : w0, s1 = hi ? v1 : w1;  // what the partner keeps
-          double k0 = hi ? w0 : v0, k1 = hi ? w1 : v1;
-          k0 += __shfl_xor_sync(kFull, s0, 16);
-          k1 += __shfl_xor_sync(kFull, s1, 16);
-          const bool odd = (g & 2) != 0;
-          double kk = odd ? k1 : k0;
-          kk += __shfl_xor_sync(kFull, odd ? k0 : k1, 8);
-          kk += __shfl_xor_sync(kFull, kk, 4);
-          if ((g & 1) == 0) *stage(hi ? 1 : 0, 8 * nj + 2 * q + (odd ? 1 : 0)) = kk;
-        }
+        cx[j] = xck;
+        asx[j] = ((double)(kb + j) * frame<PER_INST, kFrAx>(p, inst)) * xsk;
+        const double cn = xt2 * xck - xcm, sn = xt2 * xsk - xsm;
+        xcm = xck;
+        xck = cn;
+        xsm = xsk;
+        xsk = sn;
       }
-      __syncwarp();
-      if (lane < 8 * ntiles)
-      {
-        ex = *stage(0, lane);
-        ey = *stage(1, lane);
-      }
-    }
-    else
-    {
-      // (cos, sin)((k-1) a x), (cos, sin)(k a x) started at k = 0, carried across the kx blocks
-      double xcm = ca, xck = 1.0, xsm = -sa, xsk = 0.0;
-      const double xt2 = 2.0 * ca, yt2 = 2.0 * cb;
-#pragma unroll
-      for (int kb = 0; kb < NB; kb += KB)
-      {
-        double cx[KB], asx[KB];  // cos(kx a x), a_kx sin(kx a x) for kx = kb .. kb + KB - 1
-#pragma unroll
-        for (int j = 0; j < KB; j++)
-        {
-          cx[j] = xck;
-          asx[j] = ((double)(kb + j) * frame<PER_INST, kFrAx>(p, inst)) * xsk;
-          const double cn = xt2 * xck - xcm, sn = xt2 * xsk - xsm;
-          xcm = xck;
-          xck = cn;
-          xsm = xsk;
-          xsk = sn;
-        }
-        double cm = cb, ck = 1.0, sm = -sb, sk = 0.0;  // cos/sin(ky b y), advanced in the loop
+      double cm = cb, ck = 1.0, sm = -sb, sk = 0.0;  // cos/sin(ky b y), advanced in the loop
 #pragma unroll 2
-        for (int ky = 0; ky < NB; ky++)
-        {
-          double rx0 = 0.0, rx1 = 0.0, ry0 = 0.0, ry1 = 0.0;
-          const double* srow = Ssm + ky * Cfg::kSPitch + kb;
+      for (int ky = 0; ky < NB; ky++)
+      {
+        double rx0 = 0.0, rx1 = 0.0, ry0 = 0.0, ry1 = 0.0;
+        const double* srow = Ssm + ky * Cfg::kSPitch + kb;
 #pragma unroll
-          for (int j = 0; j < KB; j += 2)
-          {
-            const double2 s2 = *reinterpret_cast<const double2*>(srow + j);
-            rx0 = fma(s2.x, asx[j], rx0);
-            rx1 = fma(s2.y, asx[j + 1], rx1);
-            ry0 = fma(s2.x, cx[j], ry0);
-            ry1 = fma(s2.y, cx[j + 1], ry1);
-          }
-          ex = fma(ck, rx0 + rx1, ex);
-          ey = fma(((double)ky * frame<PER_INST, kFrBy>(p, inst)) * sk, ry0 + ry1, ey);
-          const double cn = yt2 * ck - cm, sn = yt2 * sk - sm;
-          cm = ck;
-          ck = cn;
-          sm = sk;
-          sk = sn;
+        for (int j = 0; j < KB; j += 2)
+        {
+          const double2 s2 = *reinterpret_cast<const double2*>(srow + j);
+          rx0 = fma(s2.x, asx[j], rx0);
+          rx1 = fma(s2.y, asx[j + 1], rx1);
+          ry0 = fma(s2.x, cx[j], ry0);
+          ry1 = fma(s2.y, cx[j + 1], ry1);
         }
+        ex = fma(ck, rx0 + rx1, ex);
+        ey = fma(((double)ky * frame<PER_INST, kFrBy>(p, inst)) * sk, ry0 + ry1, ey);
+        const double cn = yt2 * ck - cm, sn = yt2 * sk - sm;
+        cm = ck;
+        ck = cn;
+        sm = sk;
+        sk = sn;
       }
     }
     // dF/dx = -a sin(a x) cos(b y), dF/dy = -b cos(a x) sin(b y); times expl_weight (:433)
@@ -904,14 +712,6 @@ __global__ void __launch_bounds__(WARPS * 32, WARPS == kSolveWarps ? SolveCfg<NB
     }
 #endif
 
-#ifdef EB_NO_EARLY_BWD
-    double u0 = 0.0, u1 = 0.0;
-    if (i + 1 < p.N)
-    {
-      u0 = ut_in[(i + 1) * 3 + 0];
-      u1 = ut_in[(i + 1) * 3 + 1];
-    }
-#endif
     // gradBarrier :454-474
     double bx = 0.0, byv = 0.0;
     bx += 2.0 * (double)(xf > frame<PER_INST, kFrLx>(p, inst) - p.beps) * (xf - (frame<PER_INST, kFrLx>(p, inst) - p.beps));

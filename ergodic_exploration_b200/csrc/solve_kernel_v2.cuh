@@ -1,9 +1,9 @@
 // solve_kernel_v2.cuh -- the fused control() kernel for num_basis 13..24, re-laid to spare the SM's load/store
 // data pipe (sm_100a, FP64).  Same arithmetic contract and the same parameter block as solve_kernel.cuh (read its
-// header first: one warp per instance, lanes = time steps, warp-scan RK4, c_k and the metric gradient on the FP64
-// tensor cores); what changes is WHERE the DMMA operands come from.
+// header first: one warp per instance, lanes = time steps, warp-scan RK4, c_k on the FP64 tensor cores); here the
+// metric gradient runs on the tensor cores too, and the DMMA operands are laid out to spare shared memory.
 //
-// ncu on the round-1 kernel (profiles/solve_c5_r02_lsu.txt): the FP64 pipe (DFMA and DMMA share it on B200) was
+// ncu on the round-1 kernel (solve_kernel at nb 16..24, since retired; profiles/solve_c5_r02_lsu.txt): the FP64 pipe (DFMA and DMMA share it on B200) was
 // 60 % busy while `l1tex__data_pipe_lsu_wavefronts` -- shared-memory loads / stores, shuffles and global accesses,
 // ONE wavefront per cycle per SM for all four schedulers -- ran at 71 %, 84 % with the math removed: the kernel
 // was bound by operand traffic through shared memory, not by arithmetic.  So this version trades a few DFMAs for
@@ -28,13 +28,10 @@
 
 namespace eb
 {
-#ifndef EB_MINB2_16
-#define EB_MINB2_16 6
-#endif
-#ifndef EB_MINB2_20
-#define EB_MINB2_20 4
-#endif
+// S (NB x NB) in shared memory: pitch = 4 or 12 (mod 16) -> conflict-free A-fragment loads
+__host__ __device__ constexpr int s_pitch(int nb) { return nb % 8 == 0 ? nb + 4 : nb; }
 
+// Instantiated for NB = 16, 20 and 24.
 template <int NB>
 struct Solve2Cfg
 {
@@ -52,8 +49,8 @@ struct Solve2Cfg
   static constexpr int kStage = 64;                        // e_x | e_y of one round, handed to the time-step lanes
   static constexpr int kTabDoubles = kUnion + kStage;
   static constexpr int kFields = 8;                        // heading cos, sin; Fourier-frame x, y; cos, sin of a x; of b y
-  static constexpr int kMinBlocks = (NB <= 12 ? 7 : NB <= 16 ? EB_MINB2_16 : EB_MINB2_20) * 4 / kSolveWarps;
-  static constexpr int kWideWarps = NB <= 12 ? 28 : NB <= 16 ? 24 : 16;  // one CTA per SM for single-wave batches (see SolveCfg)
+  static constexpr int kMinBlocks = NB <= 16 ? 6 : 4;
+  static constexpr int kWideWarps = NB <= 16 ? 24 : 16;  // one CTA per SM for single-wave batches (see SolveCfg)
 };
 
 // per-step records are kept for the horizon rounded up to a half-round (16 steps)
@@ -138,7 +135,7 @@ __global__ void __launch_bounds__(WARPS * 32, WARPS == kSolveWarps ? Solve2Cfg<N
   using Cfg = Solve2Cfg<NB>;
   constexpr int TILES = Cfg::kTiles;
   constexpr int GKS = Cfg::kGks;
-  static_assert(NB % 2 == 0 && NB > 8 && NB <= 24, "solve_kernel2 serves num_basis 10..24 (even template sizes)");
+  static_assert(NB == 16 || NB == 20 || NB == 24, "solve_kernel2 serves num_basis 13..24 (template sizes 16, 20, 24)");
   extern __shared__ double smem[];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int rounds = (p.N + 31) >> 5;

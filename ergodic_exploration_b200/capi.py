@@ -171,6 +171,8 @@ SIGNATURES = {
     "eb_config_target_batch_dev": (C.c_int, [_vp, _vp, _vp]),
     "eb_control_batch_dev": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp]),
     "eb_control_batch_host": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp]),
+    "eb_set_map_targets_batch_dev": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "eb_set_map_targets_batch_host": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "eb_model_controls": (C.c_int, [C.c_int]),
     "eb_rk4_solve_host": (C.c_int, [C.c_int, C.c_int, _vp, C.c_double, C.c_double, _vp, _vp, C.c_int, C.c_int, _vp]),
     "eb_rk4_solve_dev": (C.c_int, [C.c_int, C.c_int, _vp, C.c_double, C.c_double, _vp, _vp, C.c_int, C.c_int, _vp, _vp, _vp]),

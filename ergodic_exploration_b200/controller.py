@@ -377,6 +377,61 @@ class ErgodicControl:
         assert extent.dtype == torch.float64 and extent.is_contiguous() and extent.numel() == 2 * self.batch
         check(self._lib.eb_set_phik_batch_dev(self._h, C.c_void_p(phik.data_ptr()), C.c_void_p(extent.data_ptr())))
 
+    def setMapTargets(self, cells, resolution, origin, update=None) -> None:
+        """Map-derived (entropy) target and map frame per instance, one kernel launch for the batch.
+
+        ``cells``: B int8 occupancy grids (ysize_i, xsize_i) in GridMap layout, all numpy (host path) or all CUDA
+        tensors (device path, torch's current stream); the entry of an instance that is not updated may be None.
+        ``resolution``: scalar or (B,); ``origin``: (B, 2) GridMap xmin / ymin; ``update``: (B,) bool or None (all).
+        Instance i gets the row MapTarget(xsize_i, ysize_i, resolution_i, nb).execute(cells_i) and the frame
+        origin_i, (xsize_i * res_i, ysize_i * res_i); control(None) or control(bounds of the maps) then uses them."""
+        B = self.batch
+        if len(cells) != B:
+            raise ValueError(f"setMapTargets needs {B} maps, got {len(cells)}")
+        res = np.broadcast_to(np.asarray(resolution, dtype=np.float64), (B,)).copy() if np.ndim(resolution) == 0 \
+            else _np_f64(resolution, (B,))
+        org = _np_f64(origin, (B, 2))
+        upd = None
+        if update is not None:
+            upd = np.ascontiguousarray(update)
+            if upd.shape != (B,):
+                raise ValueError(f"update must be ({B},), got {upd.shape}")
+            upd = upd.astype(np.int32)
+        present = [c for c in cells if c is not None]
+        dev = bool(present) and _is_cuda_tensor(present[0])
+        if any(_is_cuda_tensor(c) != dev for c in present):
+            raise ValueError("setMapTargets: cells must be all numpy arrays or all CUDA tensors")
+        xs = np.zeros(B, dtype=np.uint32)
+        ys = np.zeros(B, dtype=np.uint32)
+        ptrs = (C.c_void_p * B)()
+        keep = []
+        for i, c in enumerate(cells):
+            if c is None:
+                continue
+            if c.ndim != 2:
+                raise ValueError(f"setMapTargets: cells[{i}] must be 2-D (ysize, xsize), got {tuple(c.shape)}")
+            if dev:
+                if c.dtype != torch.int8 or not c.is_contiguous():
+                    raise ValueError(f"setMapTargets: cells[{i}] must be a contiguous int8 tensor")
+                ptrs[i] = c.data_ptr()
+            else:
+                c = np.ascontiguousarray(c)
+                if c.dtype != np.int8:
+                    raise ValueError(f"setMapTargets: cells[{i}] must be int8, got {c.dtype}")
+                keep.append(c)
+                ptrs[i] = c.ctypes.data
+            ys[i], xs[i] = c.shape
+        args = (C.addressof(ptrs), xs.ctypes.data, ys.ctypes.data, res.ctypes.data, org.ctypes.data,
+                upd.ctypes.data if upd is not None else None)
+        if dev:
+            self._sync_stream()
+            st = self._lib.eb_set_map_targets_batch_dev(self._h, *args)
+        else:
+            st = self._lib.eb_set_map_targets_batch_host(self._h, *args)
+        if st == capi.EB_ERR_INVALID_ARGUMENT:
+            raise ValueError(self._lib.eb_last_error().decode())
+        check(st)
+
     def get_phik_batch(self):
         """(phik (B, K), extent (B, 2)) of a per-instance controller"""
         ph = np.empty((self.batch, self.num_coeff))

@@ -23,6 +23,7 @@
 
 #include "collision_kernels.cuh"
 #include "map_target.cuh"
+#include "map_target_batch.cuh"
 #include "model_kernels.cuh"
 #include "peer_gather.cuh"
 #include "phik_dmma.cuh"
@@ -581,6 +582,17 @@ struct eb_controller
   int* d_gcount = nullptr;          // [B]
   int gmax = 0;
   double* d_bounds = nullptr;       // [B][4] staging of eb_control_batch_host
+  // map-derived targets per instance (eb_set_map_targets_batch_*, map_target_batch.cuh)
+  eb::MapBatchDesc* h_mb_desc = nullptr;  // [B] pinned: the maps of a call
+  eb::MapBatchDesc* d_mb_desc = nullptr;  // [B]
+  cudaEvent_t mb_staged = nullptr;        // recorded after the copies out of the pinned buffers
+  double* d_mb_slots = nullptr;           // [units][K] raw blocks
+  long long mb_slot_units = 0;
+  unsigned* d_mb_arrive = nullptr;        // [B] arrival counters (zero between launches)
+  signed char* h_mb_cells = nullptr;      // pinned staging of the _host call's maps
+  signed char* d_mb_cells = nullptr;
+  size_t mb_cells_bytes = 0;
+  int mb_grid = 0;                        // resident CTAs of map_target_batch_kernel on the device
 
   // device alias of a page-locked host buffer (nullptr for pageable memory);
   // looked up on every call -- a cached answer could outlive the allocation
@@ -1034,6 +1046,14 @@ void eb_destroy(eb_controller* c)
   cudaFree(c->d_gsig);
   cudaFree(c->d_gcount);
   cudaFree(c->d_bounds);
+  if (c->mb_staged) cudaEventSynchronize(c->mb_staged);
+  cudaFreeHost(c->h_mb_desc);
+  cudaFree(c->d_mb_desc);
+  if (c->mb_staged) cudaEventDestroy(c->mb_staged);
+  cudaFree(c->d_mb_slots);
+  cudaFree(c->d_mb_arrive);
+  cudaFreeHost(c->h_mb_cells);
+  cudaFree(c->d_mb_cells);
   eb_phik_plan_destroy(c->plan);
   delete c;
 }
@@ -2892,6 +2912,170 @@ eb_status eb_set_phik_batch_dev(eb_controller* c, const double* phik_dev, const 
   EB_CUDA(cudaMemcpyAsync(c->d_phik_b, phik_dev, sizeof(double) * (size_t)c->K * c->B, cudaMemcpyDeviceToDevice,
                           c->stream));
   return target_batch(c, nullptr, extent_dev, nullptr);
+}
+
+}  // extern "C"
+
+namespace
+{
+// the geometry of every flagged map; *n = flagged maps, *units = their work units
+eb_status map_targets_check(const eb_controller* c, const signed char* const* cells, const unsigned* xsize,
+                            const unsigned* ysize, const double* resolution, const int* update, const char* call, int* n,
+                            long long* units)
+{
+  *n = 0;
+  *units = 0;
+  for (int i = 0; i < c->B; i++)
+  {
+    if (update && !update[i]) continue;
+    if (xsize[i] < 1 || ysize[i] < 1 || !(resolution[i] > 0.0) || !std::isfinite(resolution[i]))
+      return fail(EB_ERR_INVALID_ARGUMENT, std::string(call) + ": map " + std::to_string(i) +
+                                               " needs xsize, ysize >= 1 and a finite resolution > 0");
+    if ((unsigned long long)xsize[i] * ysize[i] > 0x7fffffffull)
+      return fail(EB_ERR_INVALID_ARGUMENT, std::string(call) + ": map " + std::to_string(i) + " has more than 2^31 - 1 cells");
+    if (!cells[i]) return fail(EB_ERR_INVALID_ARGUMENT, std::string(call) + ": cells of map " + std::to_string(i) + " is NULL");
+    (*n)++;
+    *units += eb::mb_units((int)ysize[i]);
+  }
+  return EB_OK;
+}
+
+// map-derived targets of the flagged instances (map_target_batch.cuh); cells holds device pointers
+eb_status map_targets_batch(eb_controller* c, const signed char* const* cells, const unsigned* xsize,
+                            const unsigned* ysize, const double* resolution, const double* origin, const int* update,
+                            const char* call)
+{
+  const int B = c->B;
+  int n = 0;
+  long long units = 0;
+  eb_status st = map_targets_check(c, cells, xsize, ysize, resolution, update, call, &n, &units);
+  if (st != EB_OK) return st;
+  EB_CUDA(cudaSetDevice(c->cfg.device));
+  st = ensure_per_inst(c);
+  if (st != EB_OK) return st;
+  if (n == B) c->frames_set = true;
+  if (n == 0) return EB_OK;
+  if (!c->h_mb_desc)
+  {
+    EB_CUDA(cudaHostAlloc(&c->h_mb_desc, sizeof(eb::MapBatchDesc) * (size_t)B, cudaHostAllocDefault));
+    EB_CUDA(cudaMalloc(&c->d_mb_desc, sizeof(eb::MapBatchDesc) * (size_t)B));
+    EB_CUDA(cudaMalloc(&c->d_mb_arrive, sizeof(unsigned) * (size_t)B));
+    EB_CUDA(cudaMemset(c->d_mb_arrive, 0, sizeof(unsigned) * (size_t)B));
+    EB_CUDA(cudaEventCreateWithFlags(&c->mb_staged, cudaEventDisableTiming));
+    EB_CUDA(cudaFuncSetAttribute(eb::map_target_batch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 (int)eb::kMbSmemBytes));
+    int per_sm = 0, sms = 0;
+    EB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, eb::map_target_batch_kernel, eb::kMbThreads,
+                                                          eb::kMbSmemBytes));
+    EB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->cfg.device));
+    c->mb_grid = std::max(1, per_sm * sms);
+  }
+  if (units > c->mb_slot_units)
+  {
+    cudaFree(c->d_mb_slots);  // synchronises with earlier launches that use it
+    c->d_mb_slots = nullptr;
+    c->mb_slot_units = 0;
+    EB_CUDA(cudaMalloc(&c->d_mb_slots, sizeof(double) * (size_t)c->K * (size_t)units));
+    c->mb_slot_units = units;
+  }
+  EB_CUDA(cudaEventSynchronize(c->mb_staged));  // the previous call's copy out of the pinned descriptors is done
+  int k = 0, u0 = 0;
+  for (int i = 0; i < B; i++)
+  {
+    if (update && !update[i]) continue;
+    eb::MapBatchDesc& d = c->h_mb_desc[k++];
+    d.cells = cells[i];
+    d.nx = (int)xsize[i];
+    d.ny = (int)ysize[i];
+    d.res = resolution[i];
+    d.ox = origin[2 * i + 0];
+    d.oy = origin[2 * i + 1];
+    d.inst = i;
+    d.unit0 = u0;
+    u0 += eb::mb_units(d.ny);
+  }
+  EB_CUDA(cudaMemcpyAsync(c->d_mb_desc, c->h_mb_desc, sizeof(eb::MapBatchDesc) * (size_t)n, cudaMemcpyHostToDevice,
+                          c->stream));
+  EB_CUDA(cudaEventRecord(c->mb_staged, c->stream));
+  eb::MapBatchParams p{};
+  p.desc = c->d_mb_desc;
+  p.n = n;
+  p.units = (int)units;
+  p.nb = c->nb;
+  p.slots = c->d_mb_slots;
+  p.arrive = c->d_mb_arrive;
+  p.frames = c->d_frames;
+  p.phik = c->d_phik_b;
+  p.hist = c->d_hist;
+  p.hist_cos = c->d_hist_cos;
+  p.mem_count = c->d_hist_cos ? c->mem_count : 0;
+  p.B = B;
+  const int grid = (int)std::min<long long>(units, c->mb_grid);
+  eb::map_target_batch_kernel<<<grid, eb::kMbThreads, eb::kMbSmemBytes, c->stream>>>(p);
+  EB_CUDA(cudaGetLastError());
+  c->launches += 1;
+  return EB_OK;
+}
+}  // namespace
+
+extern "C" {
+
+eb_status eb_set_map_targets_batch_dev(eb_controller* c, const signed char* const* cells_dev, const unsigned* xsize,
+                                       const unsigned* ysize, const double* resolution, const double* origin,
+                                       const int* update)
+{
+  EB_TRACE("eb_set_map_targets_batch_dev");
+  if (!c || !cells_dev || !xsize || !ysize || !resolution || !origin)
+    return fail(EB_ERR_INVALID_ARGUMENT, "eb_set_map_targets_batch_dev: NULL argument");
+  return map_targets_batch(c, cells_dev, xsize, ysize, resolution, origin, update, "eb_set_map_targets_batch_dev");
+}
+
+eb_status eb_set_map_targets_batch_host(eb_controller* c, const signed char* const* cells, const unsigned* xsize,
+                                        const unsigned* ysize, const double* resolution, const double* origin,
+                                        const int* update)
+{
+  EB_TRACE("eb_set_map_targets_batch_host");
+  static const char* call = "eb_set_map_targets_batch_host";
+  if (!c || !cells || !xsize || !ysize || !resolution || !origin) return fail(EB_ERR_INVALID_ARGUMENT, std::string(call) + ": NULL argument");
+  int n = 0;
+  long long units = 0;
+  eb_status st = map_targets_check(c, cells, xsize, ysize, resolution, update, call, &n, &units);
+  if (st != EB_OK) return st;
+  // the flagged maps are packed into one pinned buffer (16-byte aligned offsets) and copied with one cudaMemcpyAsync
+  std::vector<size_t> off((size_t)c->B, 0);
+  size_t total = 0;
+  for (int i = 0; i < c->B; i++)
+  {
+    if (update && !update[i]) continue;
+    off[i] = total;
+    total += ((size_t)xsize[i] * ysize[i] + 15) & ~(size_t)15;
+  }
+  EB_CUDA(cudaSetDevice(c->cfg.device));
+  EB_CUDA(cudaStreamSynchronize(c->stream));  // no earlier copy still reads the staging buffers
+  if (total > c->mb_cells_bytes)
+  {
+    cudaFreeHost(c->h_mb_cells);
+    cudaFree(c->d_mb_cells);
+    c->h_mb_cells = nullptr;
+    c->d_mb_cells = nullptr;
+    c->mb_cells_bytes = 0;
+    EB_CUDA(cudaHostAlloc(&c->h_mb_cells, total, cudaHostAllocDefault));
+    EB_CUDA(cudaMalloc(&c->d_mb_cells, total));
+    c->mb_cells_bytes = total;
+  }
+  std::vector<const signed char*> dptr((size_t)c->B, nullptr);
+  for (int i = 0; i < c->B; i++)
+    if (!(update && !update[i]))
+    {
+      std::memcpy(c->h_mb_cells + off[i], cells[i], (size_t)xsize[i] * ysize[i]);
+      dptr[i] = c->d_mb_cells + off[i];
+    }
+  if (total > 0)
+    EB_CUDA(cudaMemcpyAsync(c->d_mb_cells, c->h_mb_cells, total, cudaMemcpyHostToDevice, c->stream));
+  st = map_targets_batch(c, dptr.data(), xsize, ysize, resolution, origin, update, call);
+  if (st != EB_OK) return st;
+  EB_CUDA(cudaStreamSynchronize(c->stream));
+  return EB_OK;
 }
 
 eb_status eb_get_phik_batch(const eb_controller* c, double* phik, double* extent)

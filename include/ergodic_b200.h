@@ -382,9 +382,8 @@ eb_status eb_set_phik_dev(eb_controller *c, const double *phik_dev, double lx, d
  *   4 x B {xmin xmax ymin ymax}.  The origin is always recorded; phi_k is rebuilt where the extent moved by >= 1e-12
  *   (rebuilt_dev[i] = 1).  A moved extent without Gaussians or a non-positive one is reported by the next synchronising
  *   call (eb_check_status, eb_control_batch_host) as EB_ERR_INVALID_ARGUMENT.
- * eb_set_phik_batch_dev: phi_k rows (K x B, device) and extents (2 x B {lx, ly}, device); origins are kept.  The
- *   map-derived flow: eb_map_target_execute_dev(mt, cells, phik_dev + i * K, NULL) per instance into its column, then
- *   one eb_set_phik_batch_dev.
+ * eb_set_phik_batch_dev: phi_k rows (K x B, device) and extents (2 x B {lx, ly}, device); origins are kept.  Map-derived
+ *   rows are simpler through eb_set_map_targets_batch_dev / _host below.
  * eb_control_batch_dev / _host: eb_control_dev / _host with per-instance bounds (4 x B, device / host).  bounds NULL:
  *   the frames of the last configure are used and no frame launch is made (the per-tick fast path). */
 eb_status eb_set_target_gaussians_batch(eb_controller *c, int max_n, const int *counts /* B */,
@@ -399,6 +398,32 @@ eb_status eb_control_batch_dev(eb_controller *c, const double *bounds_dev, const
                                double *u0_dev, double *metric_dev);
 eb_status eb_control_batch_host(eb_controller *c, const double *bounds, const double *x, const int *mem_idx,
                                 double *u0, double *metric);
+/* Map-derived (entropy) target per instance, ONE kernel launch for the whole batch.  For every instance i with
+ * update[i] != 0 (update NULL: all):
+ *   phi_k row i  <- the entropy target of map i, what eb_map_target_create(xsize[i], ysize[i], resolution[i], nb) +
+ *                   eb_map_target_execute compute (cell centres, Target::fill normalisation, spatialCoeff), to rounding;
+ *                   row i depends on map i alone (bit-identical whatever else is in the batch)
+ *   frame i      <- origin (origin[2i], origin[2i+1]) = the GridMap's xmin / ymin,
+ *                   extent (xsize[i] * resolution[i], ysize[i] * resolution[i])
+ *   the replay cosines of instance i are re-derived if its frame moved (as eb_config_target_batch_dev does).
+ * Rows, frames and replay cosines of the other instances are not touched.  Switches the controller to per-instance
+ * mode like every eb_*_batch target call.  xsize, ysize, resolution, origin (2 x B) and update are host arrays; cells
+ * holds B pointers (host array) to ysize[i] x xsize[i] int8 cells in GridMap layout (row-major, x fastest): device
+ * pointers for _dev (stream-ordered, returns at once; the cells must stay alive until the launch has run), host
+ * pointers for _host (packed into pinned memory, copied, run, synchronised).  The pointer of an instance that is not
+ * flagged is not read and may be NULL.  No flagged instance: nothing is launched.
+ * EB_ERR_INVALID_ARGUMENT, before anything is launched, for a flagged map with a zero size, a resolution <= 0 or
+ * non-finite, more than 2^31 - 1 cells, or a NULL cells pointer.
+ * Afterwards eb_control_batch_* runs with bounds NULL (once every instance has a frame), or with the maps' own bounds
+ * {xmin, xmin + xsize * res, ymin, ymin + ysize * res}: their extent is almost_equal to the frame's, so nothing is
+ * rebuilt (the rule the single-map flow relies on).  A later configure whose extent really moves rebuilds that instance
+ * from its Gaussians (eb_set_target_gaussians_batch), as for any per-instance target. */
+eb_status eb_set_map_targets_batch_dev(eb_controller *c, const signed char *const *cells_dev, const unsigned *xsize,
+                                       const unsigned *ysize, const double *resolution, const double *origin /* 2 x B */,
+                                       const int *update /* B or NULL */);
+eb_status eb_set_map_targets_batch_host(eb_controller *c, const signed char *const *cells, const unsigned *xsize,
+                                        const unsigned *ysize, const double *resolution, const double *origin,
+                                        const int *update);
 
 /* ---- kinematic models and the forward integrator (SURVEY.md section 8 rows a8 / a9) ----
  * model: 0 SimpleCart, 1 Omni (models/cart.hpp:152-206, models/omni.hpp:164-215), 2 Cart (cart.hpp:60-145;

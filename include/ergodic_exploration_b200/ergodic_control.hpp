@@ -715,7 +715,37 @@ public:
     }
     b200::check(eb_set_target_gaussians_batch(h_.get(), max_n, counts.data(), mu.data(), sg.data()));
   }
-  /** @brief per-instance maps: instance i is driven in grids[i]'s frame (after setTargets) */
+  /**
+   * @brief map-derived (entropy) target per instance from its occupancy grid, one kernel launch for the batch
+   * @param grids B grids with the GridMap getters gridData() / xsize() / ysize() / resolution() / xmin() / ymin()
+   * @param update instance i is updated when (*update)[i] (nullptr: all)
+   * @details instance i gets the phi_k of grids[i]'s entropy density and grids[i]'s frame; control(grids, x) then
+   * drives every robot in its own map.  Switches the controller to per-instance targets.
+   */
+  template <class GridT>
+  void setMapTargets(const std::vector<GridT>& grids, const std::vector<bool>* update = nullptr)
+  {
+    if (grids.size() != batch_) throw std::logic_error("BatchedErgodicControl::setMapTargets: need B grids");
+    if (update && update->size() != batch_)
+      throw std::logic_error("BatchedErgodicControl::setMapTargets: update needs B flags");
+    std::vector<const signed char*> cells(batch_, nullptr);
+    std::vector<unsigned> xs(batch_), ys(batch_);
+    std::vector<double> res(batch_), origin(2 * size_t(batch_));
+    std::vector<int> upd(batch_, 1);
+    for (unsigned int i = 0; i < batch_; i++)
+    {
+      if (update) upd[i] = (*update)[i] ? 1 : 0;
+      if (upd[i]) cells[i] = reinterpret_cast<const signed char*>(grids[i].gridData().data());
+      xs[i] = static_cast<unsigned>(grids[i].xsize());
+      ys[i] = static_cast<unsigned>(grids[i].ysize());
+      res[i] = grids[i].resolution();
+      origin[2 * i + 0] = grids[i].xmin();
+      origin[2 * i + 1] = grids[i].ymin();
+    }
+    b200::check(eb_set_map_targets_batch_host(h_.get(), cells.data(), xs.data(), ys.data(), res.data(), origin.data(),
+                                              upd.data()));
+  }
+  /** @brief per-instance maps: instance i is driven in grids[i]'s frame (after setTargets or setMapTargets) */
   template <class GridT>
   mat control(const std::vector<GridT>& grids, const mat& x, vec* metric = nullptr)
   {

@@ -188,6 +188,26 @@ SIGNATURES = {
     "eb_collision_check_dev": (C.c_int, [_vp, C.POINTER(EbCollision), _vp, C.c_int, _vp]),
     "eb_validate_control_host": (C.c_int, [_vp, C.POINTER(EbCollision), _vp, _vp, C.c_int, C.c_double, C.c_double, _vp]),
     "eb_validate_control_dev": (C.c_int, [_vp, C.POINTER(EbCollision), _vp, _vp, C.c_int, C.c_double, C.c_double, _vp]),
+    "eb_grid_batch_create": (C.c_int, [C.c_int, C.c_int, C.POINTER(_vp)]),
+    "eb_grid_batch_destroy": (None, [_vp]),
+    "eb_grid_batch_set_stream": (C.c_int, [_vp, _vp]),
+    "eb_grid_batch_launch_count": (C.c_longlong, [_vp]),
+    "eb_grid_batch_set_maps_dev": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "eb_grid_batch_set_maps_host": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "eb_collision_check_batch_host": (C.c_int, [_vp, C.POINTER(EbCollision), _vp, C.c_int, _vp]),
+    "eb_collision_check_batch_dev": (C.c_int, [_vp, C.POINTER(EbCollision), _vp, C.c_int, _vp]),
+    "eb_validate_control_batch_host": (C.c_int, [_vp, C.POINTER(EbCollision), _vp, _vp, C.c_int, C.c_double, C.c_double,
+                                                 _vp]),
+    "eb_validate_control_batch_dev": (C.c_int, [_vp, C.POINTER(EbCollision), _vp, _vp, C.c_int, C.c_double, C.c_double,
+                                                _vp]),
+    "eb_dwa_control_twist_batch_host": (C.c_int, [_vp, C.POINTER(EbCollision), C.POINTER(EbDwa), _vp, _vp, _vp, _vp, _vp,
+                                                  _vp]),
+    "eb_dwa_control_twist_batch_dev": (C.c_int, [_vp, C.POINTER(EbCollision), C.POINTER(EbDwa), _vp, _vp, _vp, _vp, _vp,
+                                                 _vp]),
+    "eb_dwa_control_traj_batch_host": (C.c_int, [_vp, C.POINTER(EbCollision), C.POINTER(EbDwa), _vp, _vp, _vp, C.c_int,
+                                                 C.c_int, C.c_double, _vp, _vp, _vp]),
+    "eb_dwa_control_traj_batch_dev": (C.c_int, [_vp, C.POINTER(EbCollision), C.POINTER(EbDwa), _vp, _vp, _vp, C.c_int,
+                                                C.c_int, C.c_double, _vp, _vp, _vp]),
 }
 
 _lib = None

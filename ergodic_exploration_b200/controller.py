@@ -188,6 +188,49 @@ def _np_f64(a, shape=None) -> np.ndarray:
     return a
 
 
+def map_batch_args(B: int, cells, resolution, origin, update, name: str):
+    """Checks and marshals the per-instance map arguments of eb_set_map_targets_batch_* / eb_grid_batch_set_maps_*.
+    Returns (device path?, the C arguments after the handle, the host arrays that must outlive the call)."""
+    if len(cells) != B:
+        raise ValueError(f"{name} needs {B} maps, got {len(cells)}")
+    res = np.broadcast_to(np.asarray(resolution, dtype=np.float64), (B,)).copy() if np.ndim(resolution) == 0 \
+        else _np_f64(resolution, (B,))
+    org = _np_f64(origin, (B, 2))
+    upd = None
+    if update is not None:
+        upd = np.ascontiguousarray(update)
+        if upd.shape != (B,):
+            raise ValueError(f"update must be ({B},), got {upd.shape}")
+        upd = upd.astype(np.int32)
+    present = [c for c in cells if c is not None]
+    dev = bool(present) and _is_cuda_tensor(present[0])
+    if any(_is_cuda_tensor(c) != dev for c in present):
+        raise ValueError(f"{name}: cells must be all numpy arrays or all CUDA tensors")
+    xs = np.zeros(B, dtype=np.uint32)
+    ys = np.zeros(B, dtype=np.uint32)
+    ptrs = (C.c_void_p * B)()
+    keep = [ptrs, xs, ys, res, org, upd]
+    for i, c in enumerate(cells):
+        if c is None:
+            continue
+        if c.ndim != 2:
+            raise ValueError(f"{name}: cells[{i}] must be 2-D (ysize, xsize), got {tuple(c.shape)}")
+        if dev:
+            if c.dtype != torch.int8 or not c.is_contiguous():
+                raise ValueError(f"{name}: cells[{i}] must be a contiguous int8 tensor")
+            ptrs[i] = c.data_ptr()
+        else:
+            c = np.ascontiguousarray(c)
+            if c.dtype != np.int8:
+                raise ValueError(f"{name}: cells[{i}] must be int8, got {c.dtype}")
+            keep.append(c)
+            ptrs[i] = c.ctypes.data
+        ys[i], xs[i] = c.shape
+    args = (C.addressof(ptrs), xs.ctypes.data, ys.ctypes.data, res.ctypes.data, org.ctypes.data,
+            upd.ctypes.data if upd is not None else None)
+    return dev, args, keep
+
+
 class ErgodicControl:
     """Batched drop-in for ErgodicControl<ModelT> (ergodic_control.hpp:72-185)."""
 
@@ -385,44 +428,7 @@ class ErgodicControl:
         ``resolution``: scalar or (B,); ``origin``: (B, 2) GridMap xmin / ymin; ``update``: (B,) bool or None (all).
         Instance i gets the row MapTarget(xsize_i, ysize_i, resolution_i, nb).execute(cells_i) and the frame
         origin_i, (xsize_i * res_i, ysize_i * res_i); control(None) or control(bounds of the maps) then uses them."""
-        B = self.batch
-        if len(cells) != B:
-            raise ValueError(f"setMapTargets needs {B} maps, got {len(cells)}")
-        res = np.broadcast_to(np.asarray(resolution, dtype=np.float64), (B,)).copy() if np.ndim(resolution) == 0 \
-            else _np_f64(resolution, (B,))
-        org = _np_f64(origin, (B, 2))
-        upd = None
-        if update is not None:
-            upd = np.ascontiguousarray(update)
-            if upd.shape != (B,):
-                raise ValueError(f"update must be ({B},), got {upd.shape}")
-            upd = upd.astype(np.int32)
-        present = [c for c in cells if c is not None]
-        dev = bool(present) and _is_cuda_tensor(present[0])
-        if any(_is_cuda_tensor(c) != dev for c in present):
-            raise ValueError("setMapTargets: cells must be all numpy arrays or all CUDA tensors")
-        xs = np.zeros(B, dtype=np.uint32)
-        ys = np.zeros(B, dtype=np.uint32)
-        ptrs = (C.c_void_p * B)()
-        keep = []
-        for i, c in enumerate(cells):
-            if c is None:
-                continue
-            if c.ndim != 2:
-                raise ValueError(f"setMapTargets: cells[{i}] must be 2-D (ysize, xsize), got {tuple(c.shape)}")
-            if dev:
-                if c.dtype != torch.int8 or not c.is_contiguous():
-                    raise ValueError(f"setMapTargets: cells[{i}] must be a contiguous int8 tensor")
-                ptrs[i] = c.data_ptr()
-            else:
-                c = np.ascontiguousarray(c)
-                if c.dtype != np.int8:
-                    raise ValueError(f"setMapTargets: cells[{i}] must be int8, got {c.dtype}")
-                keep.append(c)
-                ptrs[i] = c.ctypes.data
-            ys[i], xs[i] = c.shape
-        args = (C.addressof(ptrs), xs.ctypes.data, ys.ctypes.data, res.ctypes.data, org.ctypes.data,
-                upd.ctypes.data if upd is not None else None)
+        dev, args, keep = map_batch_args(self.batch, cells, resolution, origin, update, "setMapTargets")
         if dev:
             self._sync_stream()
             st = self._lib.eb_set_map_targets_batch_dev(self._h, *args)

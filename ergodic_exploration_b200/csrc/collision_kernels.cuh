@@ -22,6 +22,9 @@
 //    the map); the x86-64 behaviour -- wrap-around, i.e. the signed floor -- is
 //    what the CPU checker under tests restates and what is implemented here.
 // DynamicWindow::control (dynamic_window.cpp:93-287) runs on the same pieces (dwa_control_kernel).
+// Per-instance maps (eb_grid_batch): the PER_MAP instantiations of the three check kernels read, per thread (DWA: per
+// warp), the GridView record of their instance's map and derive its radii with collision_params' expressions; the
+// circle walk, the pose chain and the objective are the same code.  They always walk the circles (no dilated map).
 // The pose chain of validate_control / the window rollouts uses explicitly rounded multiplies / adds in
 // the reference's association order; sin / cos come from the CUDA library, so a
 // pose can differ from glibc's by an ulp or two (a cell index could differ only
@@ -64,6 +67,25 @@ struct CollisionParams
   const unsigned char* inflated;  // [ysize + 2 pad][xsize + 2 pad] or null
   int pad;
 };
+
+// the maps of an eb_grid_batch: pose / twist i of a PER_MAP call is checked against maps[i / per]
+struct MapSet
+{
+  const GridView* maps;  // [B] records; data points into the handle's arena
+  int per;
+  double boundary, padded, search;  // boundary_radius, boundary_radius + obstacle_threshold, search_radius
+};
+
+// p with map `inst` of m and the radii of collision_params (collision.cpp:130-133) for that map's resolution
+__device__ __forceinline__ CollisionParams on_map(const CollisionParams& p, const MapSet& m, int inst)
+{
+  CollisionParams q = p;
+  q.g = m.maps[inst];
+  q.r_bnd = (int)floor(__ddiv_rn(m.boundary, q.g.resolution));
+  q.r_col = (int)floor(__ddiv_rn(m.padded, q.g.resolution));
+  q.r_max = (int)floor(__ddiv_rn(m.search, q.g.resolution));
+  return q;
+}
 
 // numerics.hpp:77-89 with every operation explicitly rounded (no FMA contraction)
 __device__ __forceinline__ double normalize_angle_pi_rn(double rad)
@@ -183,6 +205,31 @@ __global__ void __launch_bounds__(256) inflate_scatter_kernel(const GridView g, 
   }
 }
 
+// The set call of an eb_grid_batch: one block per map that is written (a flagged instance's new cells) or moved (an
+// unflagged instance's cells, when the arena is laid out again); the block also stores the instance's new record.
+struct MapCopy
+{
+  const signed char* src;
+  GridView view;  // the new record; view.data is the destination
+  int inst;
+};
+
+__global__ void __launch_bounds__(256) map_copy_kernel(const MapCopy* __restrict__ copies, GridView* __restrict__ views)
+{
+  const MapCopy m = copies[blockIdx.x];
+  const size_t bytes = (size_t)m.view.xsize * m.view.ysize;
+  signed char* dst = const_cast<signed char*>(m.view.data);
+  size_t k = threadIdx.x;
+  if (((reinterpret_cast<uintptr_t>(m.src) | reinterpret_cast<uintptr_t>(dst)) & 15) == 0)
+  {
+    for (; k < bytes / 16; k += blockDim.x)
+      reinterpret_cast<uint4*>(dst)[k] = __ldg(reinterpret_cast<const uint4*>(m.src) + k);
+    k = bytes / 16 * 16 + threadIdx.x;
+  }
+  for (; k < bytes; k += blockDim.x) dst[k] = m.src[k];
+  if (threadIdx.x == 0) views[m.inst] = m.view;
+}
+
 // fraction of occupied cells, to pick between the two builders
 __global__ void __launch_bounds__(256) count_occupied_kernel(const GridView g, double thr, unsigned long long* count)
 {
@@ -194,11 +241,15 @@ __global__ void __launch_bounds__(256) count_occupied_kernel(const GridView g, d
   if ((threadIdx.x & 31) == 0 && local) atomicAdd(count, (unsigned long long)local);
 }
 
-__global__ void __launch_bounds__(128) collision_check_kernel(const CollisionParams p)
+template <bool PER_MAP>
+__global__ void __launch_bounds__(128) collision_check_kernel(const CollisionParams p, const MapSet m)
 {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= p.B) return;
-  p.out[i] = collision_check_pose(p, p.x0[(size_t)i * 3 + 0], p.x0[(size_t)i * 3 + 1]) ? 1 : 0;
+  if constexpr (PER_MAP)
+    p.out[i] = collision_check_pose(on_map(p, m, i / m.per), p.x0[(size_t)i * 3 + 0], p.x0[(size_t)i * 3 + 1]) ? 1 : 0;
+  else
+    p.out[i] = collision_check_pose(p, p.x0[(size_t)i * 3 + 0], p.x0[(size_t)i * 3 + 1]) ? 1 : 0;
 }
 
 // integrate_twist (numerics.hpp:273-298): body-frame displacement of one step of a constant
@@ -237,10 +288,8 @@ struct TwistStep
 
 // validate_control (numerics.hpp:312-330): constant twist integrated for `steps` steps,
 // the pose checked after every step; 1 = collision free
-__global__ void __launch_bounds__(128) validate_control_kernel(const CollisionParams p)
+__device__ __forceinline__ void validate_control_one(const CollisionParams& p, int i)
 {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= p.B) return;
   double x = p.x0[(size_t)i * 3 + 0], y = p.x0[(size_t)i * 3 + 1], th = p.x0[(size_t)i * 3 + 2];
   const TwistStep step(p.u[(size_t)i * 3 + 0], p.u[(size_t)i * 3 + 1], p.u[(size_t)i * 3 + 2], p.dt);
   int ok = 1;
@@ -254,6 +303,17 @@ __global__ void __launch_bounds__(128) validate_control_kernel(const CollisionPa
     }
   }
   p.out[i] = ok;
+}
+
+template <bool PER_MAP>
+__global__ void __launch_bounds__(128) validate_control_kernel(const CollisionParams p, const MapSet m)
+{
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= p.B) return;
+  if constexpr (PER_MAP)
+    validate_control_one(on_map(p, m, i / m.per), i);
+  else
+    validate_control_one(p, i);
 }
 
 // integrate_twist + normalize_angle_PI for a batch of poses (numerics.hpp:273-298, 77-89): the
@@ -298,15 +358,16 @@ struct DwaParams
 
 constexpr double kDblMax = 1.7976931348623157e308;
 
-__device__ __forceinline__ double dwa_objective(const DwaParams& p, const double* xt, double x, double y, double th,
-                                                double u0, double u1, double u2, const double* vref)
+// col: p.col, or p.col on the instance's own map (PER_MAP)
+__device__ __forceinline__ double dwa_objective(const DwaParams& p, const CollisionParams& col, const double* xt, double x,
+                                                double y, double th, double u0, double u1, double u2, const double* vref)
 {
   const TwistStep step(u0, u1, u2, p.col.dt);
   double t = 0.0, cost = 0.0;
   for (int k = 0; k < p.col.steps; k++)
   {
     step.advance(x, y, th);
-    if (collision_check_pose(p.col, x, y)) return kDblMax;
+    if (collision_check_pose(col, x, y)) return kDblMax;
     if (xt)
     {
       // index into the reference trajectory (:276)
@@ -322,11 +383,14 @@ __device__ __forceinline__ double dwa_objective(const DwaParams& p, const double
   return __dadd_rn(__dadd_rn(__dmul_rn(e0, e0), __dmul_rn(e1, e1)), __dmul_rn(e2, e2));
 }
 
-__global__ void __launch_bounds__(128) dwa_control_kernel(const DwaParams p)
+// PER_MAP: robot inst on map inst of m
+template <bool PER_MAP>
+__global__ void __launch_bounds__(128) dwa_control_kernel(const DwaParams p, const MapSet m)
 {
   const int lane = threadIdx.x & 31;
   const int inst = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   if (inst >= p.B) return;
+  const CollisionParams col = PER_MAP ? on_map(p.col, m, inst) : p.col;
   const double x = p.x0[(size_t)inst * 3 + 0], y = p.x0[(size_t)inst * 3 + 1], th = p.x0[(size_t)inst * 3 + 2];
   // DynamicWindow::window (:189-235)
   double lower[3], delta[3];
@@ -356,7 +420,7 @@ __global__ void __launch_bounds__(128) dwa_control_kernel(const DwaParams p)
   {
     double u0, u1, u2;
     twist(c, u0, u1, u2);
-    const double cost = dwa_objective(p, xt, x, y, th, u0, u1, u2, vref);
+    const double cost = dwa_objective(p, col, xt, x, y, th, u0, u1, u2, vref);
     if (cost < best)
     {
       best = cost;

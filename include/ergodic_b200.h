@@ -334,6 +334,60 @@ eb_status eb_dwa_control_traj_dev(eb_grid *g, const eb_collision *c, const eb_dw
                                   const double *vb_dev, const double *xt_ref_dev, int ncols, int per_instance,
                                   double dt_ref, int count, int *found_dev, double *u_opt_dev, double *min_cost_dev);
 
+/* ---- per-instance occupancy maps -------------------------------------------------------------------------------
+ * An eb_grid_batch holds B occupancy maps on one device and one stream, each with its own shape, resolution and origin,
+ * so B robots on B maps run their collision checks, validate_control and DynamicWindow as one launch per call.  For
+ * every instance i each output equals, bit for bit, what the eb_grid calls above return for eb_grid_create(map i) with
+ * eb_grid_set_dilation(1), whatever the other maps are: the radii r_bnd, r_col, r_max are derived per instance from the
+ * call's eb_collision and map i's resolution (collision.cpp:130-133), and the circles are always walked (there is no
+ * pre-dilated map per instance).
+ * eb_grid_batch_set_maps_dev / _host: the same arguments and rules as eb_set_map_targets_batch_dev / _host, so one set
+ *   of arrays per map update feeds both.  Instance i with update[i] != 0 (update NULL: all) gets a device copy of map i
+ *   (cells ysize[i] x xsize[i], GridMap layout), its resolution and its origin (origin[2i], origin[2i+1] = xmin, ymin).
+ *   The maps live in one device arena; unflagged instances keep their cells and geometry, also when a flagged map
+ *   outgrows its slot and every map moves to a new arena.  One kernel launch per call (none when nothing is flagged).
+ *   _dev is stream-ordered: the cells must stay alive until the copy kernel has run.  _host packs the flagged maps
+ *   into one pinned buffer, copies it with one cudaMemcpyAsync and synchronises.  EB_ERR_INVALID_ARGUMENT, before
+ *   anything is launched, for a flagged map with a zero size, a resolution <= 0 or non-finite, more than 2^31 - 1 cells,
+ *   or a NULL cells pointer.
+ * eb_collision_check_batch_* / eb_validate_control_batch_*: poses / x0 / u are 3 x (per * B), instance-major: pose p is
+ *   checked against map p / per (per >= 1); outputs per * B ints.
+ * eb_dwa_control_*_batch_*: robot i on map i (B robots); the other arguments as eb_dwa_control_twist_* / _traj_*
+ *   (xt_ref 3 x ncols shared, or 3 x ncols x B with per_instance = 1, e.g. the output of eb_opt_traj_dev).
+ * Every check is one kernel launch; _host adds the copies of inputs and outputs and a synchronise.  The checks return
+ * EB_ERR_INVALID_ARGUMENT before launching where the Collision constructor throws, for per < 1, per * B beyond INT_MAX,
+ * and while some instance has never been given a map. */
+typedef struct eb_grid_batch eb_grid_batch;
+eb_status eb_grid_batch_create(int device, int batch, eb_grid_batch **out);
+void eb_grid_batch_destroy(eb_grid_batch *g);
+eb_status eb_grid_batch_set_stream(eb_grid_batch *g, void *cuda_stream);
+long long eb_grid_batch_launch_count(const eb_grid_batch *g);
+eb_status eb_grid_batch_set_maps_dev(eb_grid_batch *g, const signed char *const *cells_dev, const unsigned *xsize,
+                                     const unsigned *ysize, const double *resolution, const double *origin /* 2 x B */,
+                                     const int *update /* B or NULL */);
+eb_status eb_grid_batch_set_maps_host(eb_grid_batch *g, const signed char *const *cells, const unsigned *xsize,
+                                      const unsigned *ysize, const double *resolution, const double *origin,
+                                      const int *update);
+eb_status eb_collision_check_batch_host(eb_grid_batch *g, const eb_collision *c, const double *poses, int per, int *hit);
+eb_status eb_collision_check_batch_dev(eb_grid_batch *g, const eb_collision *c, const double *poses_dev, int per,
+                                       int *hit_dev);
+eb_status eb_validate_control_batch_host(eb_grid_batch *g, const eb_collision *c, const double *x0, const double *u,
+                                         int per, double dt, double horizon, int *valid);
+eb_status eb_validate_control_batch_dev(eb_grid_batch *g, const eb_collision *c, const double *x0_dev,
+                                        const double *u_dev, int per, double dt, double horizon, int *valid_dev);
+eb_status eb_dwa_control_twist_batch_host(eb_grid_batch *g, const eb_collision *c, const eb_dwa *d, const double *x0,
+                                          const double *vb, const double *vref, int *found, double *u_opt,
+                                          double *min_cost);
+eb_status eb_dwa_control_twist_batch_dev(eb_grid_batch *g, const eb_collision *c, const eb_dwa *d, const double *x0_dev,
+                                         const double *vb_dev, const double *vref_dev, int *found_dev,
+                                         double *u_opt_dev, double *min_cost_dev);
+eb_status eb_dwa_control_traj_batch_host(eb_grid_batch *g, const eb_collision *c, const eb_dwa *d, const double *x0,
+                                         const double *vb, const double *xt_ref, int ncols, int per_instance,
+                                         double dt_ref, int *found, double *u_opt, double *min_cost);
+eb_status eb_dwa_control_traj_batch_dev(eb_grid_batch *g, const eb_collision *c, const eb_dwa *d, const double *x0_dev,
+                                        const double *vb_dev, const double *xt_ref_dev, int ncols, int per_instance,
+                                        double dt_ref, int *found_dev, double *u_opt_dev, double *min_cost_dev);
+
 /* ---- row-sharded phi_k on several GPUs (SURVEY.md section 8e) -----------------------
  * The all-reduce of the ranks' raw 32 x 32 blocks is fused into the tile kernel: the last CTA of every rank stores its
  * block into all ranks' receive buffers over NVLink peer memory (CUDA IPC mappings, exchanged once like eb_peer_group),

@@ -9,7 +9,8 @@
  *   Collision::collisionCheck(grid, pose)                     collision.cpp:126-143
  *   validate_control(collision, grid, x0, u, dt, horizon)     numerics.hpp:312-330
  *   DynamicWindow::control(grid, x0, vb, vref | xt_ref)       dynamic_window.cpp:93-187
- * for one pose / twist (the reference's signatures) or for a 3 x B batch sharing one map.
+ * for one pose / twist (the reference's signatures), for a 3 x B batch sharing one map (DeviceGrid), or for B
+ * instances on B maps (DeviceGridBatch: instance i is checked against map i, one kernel launch per call).
  * The grid type is anything with the reference GridMap's getters
  * (gridData(), xsize(), ysize(), resolution(), xmin(), ymin(); grid.hpp:201-255).
  * The reference's Collision keeps its radii private (collision.hpp:159-163), so the
@@ -22,6 +23,7 @@
 #include <memory>
 #include <cmath>
 #include <stdexcept>
+#include <string>
 #include <tuple>
 #include <vector>
 
@@ -69,6 +71,64 @@ private:
   std::shared_ptr<eb_grid> h_;
 };
 
+/**
+ * @brief B occupancy grids resident on the GPU, one per instance (eb_grid_batch): every map has its own shape,
+ * resolution and origin.  Built from and updated with the same GridMap-like objects as
+ * BatchedErgodicControl::setMapTargets, so one vector of grids per map update feeds both.
+ */
+class DeviceGridBatch
+{
+public:
+  template <class GridT>
+  explicit DeviceGridBatch(const std::vector<GridT>& grids) : batch_(static_cast<unsigned int>(grids.size()))
+  {
+    if (grids.empty()) throw std::logic_error("DeviceGridBatch: need at least one grid");
+    eb_grid_batch* g = nullptr;
+    check(eb_grid_batch_create(default_device(), int(batch_), &g));
+    h_.reset(g, eb_grid_batch_destroy);
+    update(grids);
+  }
+
+  /** @brief instance i gets grids[i]'s cells and geometry when (*update)[i] (nullptr: all); the others keep theirs */
+  template <class GridT>
+  void update(const std::vector<GridT>& grids, const std::vector<bool>* update = nullptr)
+  {
+    if (grids.size() != batch_) throw std::logic_error("DeviceGridBatch::update: need B grids");
+    if (update && update->size() != batch_) throw std::logic_error("DeviceGridBatch::update: update needs B flags");
+    std::vector<const signed char*> cells(batch_, nullptr);
+    std::vector<unsigned> xs(batch_), ys(batch_);
+    std::vector<double> res(batch_), origin(2 * size_t(batch_));
+    std::vector<int> upd(batch_, 1);
+    for (unsigned int i = 0; i < batch_; i++)
+    {
+      if (update) upd[i] = (*update)[i] ? 1 : 0;
+      if (upd[i]) cells[i] = reinterpret_cast<const signed char*>(grids[i].gridData().data());
+      xs[i] = static_cast<unsigned>(grids[i].xsize());
+      ys[i] = static_cast<unsigned>(grids[i].ysize());
+      res[i] = grids[i].resolution();
+      origin[2 * i + 0] = grids[i].xmin();
+      origin[2 * i + 1] = grids[i].ymin();
+    }
+    check(eb_grid_batch_set_maps_host(h_.get(), cells.data(), xs.data(), ys.data(), res.data(), origin.data(),
+                                      upd.data()));
+  }
+
+  eb_grid_batch* handle() const { return h_.get(); }
+  unsigned int batch() const { return batch_; }
+
+  /** @brief rows per instance of a 3 x (per * B) matrix */
+  int per(const arma::mat& m, const char* what) const
+  {
+    if (m.n_rows != 3 || m.n_cols == 0 || m.n_cols % batch_ != 0)
+      throw std::logic_error(std::string(what) + ": must be 3 x (per * B)");
+    return static_cast<int>(m.n_cols / batch_);
+  }
+
+private:
+  unsigned int batch_;
+  std::shared_ptr<eb_grid_batch> h_;
+};
+
 /** @brief Collision (collision.hpp:85-165) evaluated on the GPU, one pose or a batch */
 class Collision
 {
@@ -102,6 +162,15 @@ public:
     return hit;
   }
 
+  /** @brief per-instance maps: poses is 3 x (per * B), instance-major; pose p is checked against map p / per */
+  std::vector<int> collisionCheck(const DeviceGridBatch& grids, const arma::mat& poses) const
+  {
+    const int per = grids.per(poses, "collisionCheck: poses");
+    std::vector<int> hit(poses.n_cols);
+    check(eb_collision_check_batch_host(grids.handle(), &cfg_, poses.memptr(), per, hit.data()));
+    return hit;
+  }
+
   const eb_collision& config() const { return cfg_; }
 
 private:
@@ -129,6 +198,18 @@ inline std::vector<int> validate_control(const Collision& collision, const Devic
                                  static_cast<int>(x0.n_cols), dt, horizon, valid.data()));
   return valid;
 }
+/** @brief per-instance maps: x0 and u are 3 x (per * B), instance-major; row p is checked against map p / per */
+inline std::vector<int> validate_control(const Collision& collision, const DeviceGridBatch& grids, const arma::mat& x0,
+                                         const arma::mat& u, double dt, double horizon)
+{
+  const int per = grids.per(x0, "validate_control: x0");
+  if (u.n_rows != 3 || u.n_cols != x0.n_cols) throw std::logic_error("validate_control: x0 and u must be 3 x (per * B)");
+  std::vector<int> valid(x0.n_cols);
+  check(eb_validate_control_batch_host(grids.handle(), &collision.config(), x0.memptr(), u.memptr(), per, dt, horizon,
+                                       valid.data()));
+  return valid;
+}
+
 /** @brief DynamicWindow (dynamic_window.hpp:60-172) evaluated on the GPU, one robot or a batch */
 class DynamicWindow
 {
@@ -180,6 +261,38 @@ public:
     arma::mat u(3, x0.n_cols);
     check(eb_dwa_control_twist_host(grid.handle(), &collision_.config(), &cfg_, x0.memptr(), vb.memptr(),
                                     vref.memptr(), static_cast<int>(x0.n_cols), found.data(), u.memptr(), nullptr));
+    return std::make_tuple(found, u);
+  }
+
+  /** @brief per-instance maps: robot i (column i of the 3 x B x0, vb, vref) on map i */
+  std::tuple<std::vector<int>, arma::mat> controlBatch(const DeviceGridBatch& grids, const arma::mat& x0,
+                                                       const arma::mat& vb, const arma::mat& vref) const
+  {
+    const unsigned int B = grids.batch();
+    if (x0.n_rows != 3 || vb.n_rows != 3 || vref.n_rows != 3 || x0.n_cols != B || vb.n_cols != B || vref.n_cols != B)
+      throw std::logic_error("DynamicWindow::controlBatch: x0, vb, vref must be 3 x B");
+    std::vector<int> found(B);
+    arma::mat u(3, B);
+    check(eb_dwa_control_twist_batch_host(grids.handle(), &collision_.config(), &cfg_, x0.memptr(), vb.memptr(),
+                                          vref.memptr(), found.data(), u.memptr(), nullptr));
+    return std::make_tuple(found, u);
+  }
+
+  /**
+   * @brief per-instance maps and reference trajectories: robot i on map i follows columns [i * n, (i + 1) * n) of
+   * xt_ref (3 x (n * B), time step dt_ref), the layout BatchedErgodicControl::optTraj() returns
+   */
+  std::tuple<std::vector<int>, arma::mat> controlBatch(const DeviceGridBatch& grids, const arma::mat& x0,
+                                                       const arma::mat& vb, const arma::mat& xt_ref, double dt_ref) const
+  {
+    const unsigned int B = grids.batch();
+    if (x0.n_rows != 3 || vb.n_rows != 3 || x0.n_cols != B || vb.n_cols != B)
+      throw std::logic_error("DynamicWindow::controlBatch: x0, vb must be 3 x B");
+    const int ncols = grids.per(xt_ref, "DynamicWindow::controlBatch: xt_ref");
+    std::vector<int> found(B);
+    arma::mat u(3, B);
+    check(eb_dwa_control_traj_batch_host(grids.handle(), &collision_.config(), &cfg_, x0.memptr(), vb.memptr(),
+                                         xt_ref.memptr(), ncols, 1, dt_ref, found.data(), u.memptr(), nullptr));
     return std::make_tuple(found, u);
   }
 

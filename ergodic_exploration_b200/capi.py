@@ -208,6 +208,10 @@ SIGNATURES = {
                                                  C.c_int, C.c_double, _vp, _vp, _vp]),
     "eb_dwa_control_traj_batch_dev": (C.c_int, [_vp, C.POINTER(EbCollision), C.POINTER(EbDwa), _vp, _vp, _vp, C.c_int,
                                                 C.c_int, C.c_double, _vp, _vp, _vp]),
+    "eb_control_safe_batch_dev": (C.c_int, [_vp, _vp, C.POINTER(EbCollision), C.POINTER(EbDwa), C.c_double, C.c_double,
+                                            _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "eb_control_safe_batch_host": (C.c_int, [_vp, _vp, C.POINTER(EbCollision), C.POINTER(EbDwa), C.c_double, C.c_double,
+                                             _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
 }
 
 _lib = None

@@ -479,6 +479,62 @@ class ErgodicControl:
             check(st)
         return u0
 
+    def control_safe(self, grids, dwa, x, vb, val_dt: float, val_horizon: float, bounds=None, mem_idx=None,
+                     metric=None, collision=None):
+        """One safe control tick of B robots on B maps, the reference loop's arbitration between the ergodic twist
+        and the safety planner (exploration.hpp:238-247): control(bounds, x) of every instance, validate_control of
+        its twist on its own map (``grids``, a GridMapBatch) with val_dt and val_horizon, and only where that twist
+        collides DynamicWindow.control on that map with ``dwa``'s window, ``vb`` and the instance's optTraj() as the
+        reference trajectory.  ``collision`` (default ``dwa.collision``) is the Collision of the tick: both the
+        validation and the window's rollouts are checked with it, as in the reference node, which builds the window
+        from the controller's Collision.
+
+        Returns (u (B, 3), branch (B,) int32): branch 0 = the ergodic twist, 1 = the window's twist, 2 = the window
+        found nothing and u = 0.  Bit for bit what those calls return one after the other, with the window run only
+        for the robots that need it.  numpy inputs take the host path (copies, one synchronisation); CUDA tensors run
+        on torch's current stream without a host synchronisation (``metric`` (B,) float64 and ``mem_idx`` int32 then
+        tensors too).  ``bounds`` (B, 4) as in control(); None: the frames of the last configure."""
+        B = self.batch
+        if grids.batch != B:
+            raise ValueError(f"control_safe: the grid batch holds {grids.batch} maps for {B} instances")
+        dev = _is_cuda_tensor(x)
+        x, _, _ = grids._rows("x", x, dev, per_ok=False)
+        vb, _, _ = grids._rows("vb", vb, dev, per_ok=False)
+        col = dwa.collision if collision is None else collision
+        if dev:
+            b = self._bounds_dev(bounds) if bounds is not None else None
+            if metric is not None and not (_is_cuda_tensor(metric) and metric.dtype == torch.float64 and
+                                           metric.is_contiguous() and tuple(metric.shape) == (B,)):
+                raise ValueError(f"metric must be a contiguous ({B},) float64 CUDA tensor on the device path")
+            if mem_idx is not None and not (_is_cuda_tensor(mem_idx) and mem_idx.dtype == torch.int32 and
+                                            mem_idx.is_contiguous()):
+                raise ValueError("mem_idx must be a contiguous int32 CUDA tensor on the device path")
+            u = torch.empty((B, 3), dtype=torch.float64, device=x.device)
+            branch = torch.empty(B, dtype=torch.int32, device=x.device)
+            fn = self._lib.eb_control_safe_batch_dev
+        else:
+            b = None
+            if bounds is not None:
+                b = _np_f64(bounds.cpu().numpy() if _is_cuda_tensor(bounds) else bounds, (B, 4))
+            if metric is not None and not (isinstance(metric, np.ndarray) and metric.dtype == np.float64 and
+                                           metric.flags.c_contiguous and metric.shape == (B,)):
+                raise ValueError(f"metric must be a contiguous ({B},) float64 numpy array on the host path")
+            if mem_idx is not None:
+                mem_idx = np.ascontiguousarray(mem_idx, dtype=np.int32)
+            u, branch = np.empty((B, 3)), np.empty(B, dtype=np.int32)
+            fn = self._lib.eb_control_safe_batch_host
+        P = grids._ptr
+        self._sync_stream()
+        grids._stream()
+        st = fn(self._h, grids._h, C.byref(col.cfg), C.byref(dwa.cfg), float(val_dt), float(val_horizon),
+                P(b) if b is not None else None, P(x), P(mem_idx) if mem_idx is not None else None, P(vb), P(u),
+                P(branch), P(metric) if metric is not None else None)
+        if st != capi.EB_OK:
+            if st == capi.EB_ERR_INVALID_ARGUMENT:
+                raise ValueError(self._lib.eb_last_error().decode())
+            check(st)
+        return u, branch
+
     def check(self) -> None:
         """Synchronise and surface device-side faults of earlier device-path calls."""
         st = self._lib.eb_check_status(self._h)

@@ -288,7 +288,7 @@ struct TwistStep
 
 // validate_control (numerics.hpp:312-330): constant twist integrated for `steps` steps,
 // the pose checked after every step; 1 = collision free
-__device__ __forceinline__ void validate_control_one(const CollisionParams& p, int i)
+__device__ __forceinline__ int validate_control_ok(const CollisionParams& p, int i)
 {
   double x = p.x0[(size_t)i * 3 + 0], y = p.x0[(size_t)i * 3 + 1], th = p.x0[(size_t)i * 3 + 2];
   const TwistStep step(p.u[(size_t)i * 3 + 0], p.u[(size_t)i * 3 + 1], p.u[(size_t)i * 3 + 2], p.dt);
@@ -302,8 +302,10 @@ __device__ __forceinline__ void validate_control_one(const CollisionParams& p, i
       break;
     }
   }
-  p.out[i] = ok;
+  return ok;
 }
+
+__device__ __forceinline__ void validate_control_one(const CollisionParams& p, int i) { p.out[i] = validate_control_ok(p, i); }
 
 template <bool PER_MAP>
 __global__ void __launch_bounds__(128) validate_control_kernel(const CollisionParams p, const MapSet m)
@@ -383,6 +385,52 @@ __device__ __forceinline__ double dwa_objective(const DwaParams& p, const Collis
   return __dadd_rn(__dadd_rn(__dmul_rn(e0, e0), __dmul_rn(e1, e1)), __dmul_rn(e2, e2));
 }
 
+// DynamicWindow::window (:189-235) of robot inst: the first sample of each axis and the step between samples
+__device__ __forceinline__ void dwa_window(const DwaParams& p, int inst, double (&lower)[3], double (&delta)[3])
+{
+#pragma unroll
+  for (int a = 0; a < 3; a++)
+  {
+    const double v = p.vb[(size_t)inst * 3 + a], reach = __dmul_rn(p.acc_lim[a], p.acc_dt);
+    lower[a] = fmax(__dsub_rn(v, reach), p.vmin[a]);
+    const double upper = fmin(__dadd_rn(v, reach), p.vmax[a]);
+    delta[a] = p.n[a] > 1 ? __ddiv_rn(__dsub_rn(upper, lower[a]), (double)(p.n[a] - 1)) : 0.0;
+  }
+}
+
+// candidate c of the window in the reference's loop order (vx outer, vth inner), as its accumulated sums
+__device__ __forceinline__ void dwa_twist(const DwaParams& p, const double (&lower)[3], const double (&delta)[3],
+                                          unsigned int c, double& u0, double& u1, double& u2)
+{
+  const unsigned int k = c % p.n[2], j = (c / p.n[2]) % p.n[1], i = c / (p.n[2] * p.n[1]);
+  u0 = lower[0];
+  for (unsigned int s = 0; s < i; s++) u0 = __dadd_rn(u0, delta[0]);  // vx += dvx, i times
+  u1 = lower[1];
+  for (unsigned int s = 0; s < j; s++) u1 = __dadd_rn(u1, delta[1]);
+  u2 = lower[2];
+  for (unsigned int s = 0; s < k; s++) u2 = __dadd_rn(u2, delta[2]);
+}
+
+// warp arg-min of (cost, candidate) with ties to the lower candidate: the reference's first strict minimum in loop
+// order, whichever lanes evaluated which candidates
+__device__ __forceinline__ void dwa_argmin_warp(double& best, unsigned int& best_c)
+{
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1)
+  {
+    const double oc = __shfl_xor_sync(kFull, best, o);
+    const unsigned int oi = __shfl_xor_sync(kFull, best_c, o);
+    if (oc < best || (oc == best && oi < best_c))
+    {
+      best = oc;
+      best_c = oi;
+    }
+  }
+}
+
+// almost_equal(min_cost, max) (:132): 0 when no candidate beat the initial min_cost (the window found nothing)
+__device__ __forceinline__ int dwa_found(double best) { return (fabs(best - kDblMax) < 1.0e-12) ? 0 : 1; }
+
 // PER_MAP: robot inst on map inst of m
 template <bool PER_MAP>
 __global__ void __launch_bounds__(128) dwa_control_kernel(const DwaParams p, const MapSet m)
@@ -392,28 +440,14 @@ __global__ void __launch_bounds__(128) dwa_control_kernel(const DwaParams p, con
   if (inst >= p.B) return;
   const CollisionParams col = PER_MAP ? on_map(p.col, m, inst) : p.col;
   const double x = p.x0[(size_t)inst * 3 + 0], y = p.x0[(size_t)inst * 3 + 1], th = p.x0[(size_t)inst * 3 + 2];
-  // DynamicWindow::window (:189-235)
   double lower[3], delta[3];
-#pragma unroll
-  for (int a = 0; a < 3; a++)
-  {
-    const double v = p.vb[(size_t)inst * 3 + a], reach = __dmul_rn(p.acc_lim[a], p.acc_dt);
-    lower[a] = fmax(__dsub_rn(v, reach), p.vmin[a]);
-    const double upper = fmin(__dadd_rn(v, reach), p.vmax[a]);
-    delta[a] = p.n[a] > 1 ? __ddiv_rn(__dsub_rn(upper, lower[a]), (double)(p.n[a] - 1)) : 0.0;
-  }
+  dwa_window(p, inst, lower, delta);
   const double* xt = p.xt_ref ? p.xt_ref + (size_t)inst * (size_t)p.xt_stride : nullptr;
   const double* vref = p.vref ? p.vref + (size_t)inst * 3 : nullptr;
   const unsigned int total = p.n[0] * p.n[1] * p.n[2];
-  auto twist = [&](unsigned int c, double& u0, double& u1, double& u2) {
-    const unsigned int k = c % p.n[2], j = (c / p.n[2]) % p.n[1], i = c / (p.n[2] * p.n[1]);
-    u0 = lower[0];
-    for (unsigned int s = 0; s < i; s++) u0 = __dadd_rn(u0, delta[0]);  // vx += dvx, i times
-    u1 = lower[1];
-    for (unsigned int s = 0; s < j; s++) u1 = __dadd_rn(u1, delta[1]);
-    u2 = lower[2];
-    for (unsigned int s = 0; s < k; s++) u2 = __dadd_rn(u2, delta[2]);
-  };
+  // (the lambda and the inline arg-min below keep this kernel's instructions as they were before the helpers were
+  // factored out for dwa_fallback_kernel; direct calls change its register allocation)
+  auto twist = [&](unsigned int c, double& u0, double& u1, double& u2) { dwa_twist(p, lower, delta, c, u0, u1, u2); };
   double best = kDblMax;
   unsigned int best_c = 0xffffffffu;
   for (unsigned int c = lane; c < total; c += 32)
@@ -445,7 +479,7 @@ __global__ void __launch_bounds__(128) dwa_control_kernel(const DwaParams p, con
     p.u_opt[(size_t)inst * 3 + 0] = u0;
     p.u_opt[(size_t)inst * 3 + 1] = u1;
     p.u_opt[(size_t)inst * 3 + 2] = u2;
-    p.found[inst] = (fabs(best - kDblMax) < 1.0e-12) ? 0 : 1;  // almost_equal(min_cost, max) (:132)
+    p.found[inst] = dwa_found(best);
     if (p.min_cost) p.min_cost[inst] = best;
   }
 }

@@ -29,6 +29,7 @@
 #include "phik_dmma.cuh"
 #include "phik_kernels.cuh"
 #include "phik_tma.cuh"
+#include "safe_control.cuh"
 #include "solve_kernel.cuh"
 #include "solve_kernel_v2.cuh"
 #include "solve_kernel_big.cuh"
@@ -593,6 +594,11 @@ struct eb_controller
   signed char* d_mb_cells = nullptr;
   size_t mb_cells_bytes = 0;
   int mb_grid = 0;                        // resident CTAs of map_target_batch_kernel on the device
+  // safe control tick (eb_control_safe_batch_*, safe_control.cuh)
+  int* d_safe_list = nullptr;      // [1 + B]: the count of failing robots, then their indices
+  int* d_safe_branch = nullptr;    // [B] staging of the _host call
+  double* d_safe_vb = nullptr;     // [B][3] staging of the _host call
+  int safe_grid = 0;               // resident CTAs of dwa_fallback_kernel with this horizon
 
   // device alias of a page-locked host buffer (nullptr for pageable memory);
   // looked up on every call -- a cached answer could outlive the allocation
@@ -1054,6 +1060,9 @@ void eb_destroy(eb_controller* c)
   cudaFree(c->d_mb_arrive);
   cudaFreeHost(c->h_mb_cells);
   cudaFree(c->d_mb_cells);
+  cudaFree(c->d_safe_list);
+  cudaFree(c->d_safe_branch);
+  cudaFree(c->d_safe_vb);
   eb_phik_plan_destroy(c->plan);
   delete c;
 }
@@ -2567,6 +2576,10 @@ struct eb_grid_batch
   eb::MapCopy* h_copies = nullptr;
   eb::MapCopy* d_copies = nullptr;
   cudaEvent_t staged = nullptr;  // the last upload out of h_copies has been made
+  // eb_control_safe_batch_*: recorded on the grid batch's stream before a tick (maps_ready) and on the controller's
+  // stream after it (ticked); the next set call waits for the last tick before it writes or frees an arena
+  cudaEvent_t maps_ready = nullptr;
+  cudaEvent_t ticked = nullptr;
   signed char* h_cells = nullptr;
   signed char* d_cells = nullptr;
   size_t cells_bytes = 0;
@@ -2594,6 +2607,7 @@ eb_status grid_batch_set(eb_grid_batch* g, const signed char* const* cells, cons
   if (n == 0) return EB_OK;
   const int B = g->B;
   EB_CUDA(cudaSetDevice(g->device));
+  if (g->ticked) EB_CUDA(cudaStreamWaitEvent(g->stream, g->ticked, 0));  // a safe control tick may still read the maps
   if (!g->d_views)
   {
     EB_CUDA(cudaMalloc(&g->d_views, sizeof(eb::GridView) * (size_t)B));
@@ -2753,6 +2767,7 @@ void eb_grid_batch_destroy(eb_grid_batch* g)
   if (!g) return;
   cudaSetDevice(g->device);
   if (g->staged) cudaEventSynchronize(g->staged);
+  if (g->ticked) cudaEventSynchronize(g->ticked);
   cudaFree(g->d_views);
   cudaFree(g->d_arena);
   cudaFree(g->d_retired);
@@ -2767,6 +2782,8 @@ void eb_grid_batch_destroy(eb_grid_batch* g)
   cudaFree(g->d_ref);
   cudaFree(g->d_out);
   if (g->staged) cudaEventDestroy(g->staged);
+  if (g->maps_ready) cudaEventDestroy(g->maps_ready);
+  if (g->ticked) cudaEventDestroy(g->ticked);
   delete g;
 }
 
@@ -3623,6 +3640,151 @@ eb_status eb_control_batch_host(eb_controller* c, const double* bounds, const do
   if (st != EB_OK) return st;
   EB_CUDA(cudaMemcpyAsync(u0, c->d_u0, sizeof(double) * 3 * c->B, cudaMemcpyDeviceToHost, c->stream));
   if (metric) EB_CUDA(cudaMemcpyAsync(metric, c->d_metric, sizeof(double) * c->B, cudaMemcpyDeviceToHost, c->stream));
+  return check_fault(c);  // synchronises
+}
+
+}  // extern "C"
+
+// ---------------------------------------------------------------------------
+// safe control tick of B robots on B maps (safe_control.cuh)
+// ---------------------------------------------------------------------------
+namespace
+{
+// everything the tick refuses before it launches (or copies) anything, so an error leaves the controller as it was;
+// fills the fallback's window and collision parameters
+eb_status safe_batch_check(const eb_controller* c, eb_grid_batch* g, const eb_collision* col, const eb_dwa* d,
+                           double val_dt, const double* bounds, const char* call, eb::DwaParams* p, eb::MapSet* m)
+{
+  if (!c || !g || !col || !d) return fail(EB_ERR_INVALID_ARGUMENT, std::string(call) + ": NULL argument");
+  if (!c->per_inst)
+    return fail(EB_ERR_INVALID_ARGUMENT, std::string(call) + ": the controller holds a shared target; the safe tick "
+                                                             "needs per-instance targets (the eb_*_batch calls)");
+  if (!bounds && !c->frames_set)
+    return fail(EB_ERR_INVALID_ARGUMENT, std::string(call) + ": bounds NULL before any frame was configured");
+  if (g->B != c->B)
+    return fail(EB_ERR_INVALID_ARGUMENT, std::string(call) + ": the grid batch holds " + std::to_string(g->B) +
+                                             " maps for " + std::to_string(c->B) + " instances");
+  if (g->device != c->cfg.device)
+    return fail(EB_ERR_INVALID_ARGUMENT, std::string(call) + ": the grid batch and the controller are on different devices");
+  eb_status st = grid_batch_dwa(g, col, d, p, m);  // Collision constructor rules, every instance has a map, DWA dt
+  if (st != EB_OK) return st;
+  if (val_dt == 0.0) return fail(EB_ERR_INVALID_ARGUMENT, std::string(call) + ": val_dt is 0");
+  // the reference trajectory is each robot's optTraj(): N columns at the controller's time step
+  return dwa_traj_params(nullptr, c->N, 1, c->cfg.dt, p);
+}
+
+// the failing-robot list and the _host staging, allocated at the first tick; the fallback's resident grid
+eb_status ensure_safe(eb_controller* c)
+{
+  if (c->d_safe_list) return EB_OK;
+  const size_t B = (size_t)c->B;
+  EB_CUDA(cudaMalloc(&c->d_safe_branch, sizeof(int) * B));
+  EB_CUDA(cudaMalloc(&c->d_safe_vb, sizeof(double) * 3 * B));
+  auto kernel = c->cfg.model == EB_MODEL_OMNI ? eb::dwa_fallback_kernel<eb::kModelOmni> :
+                                                eb::dwa_fallback_kernel<eb::kModelSimpleCart>;
+  const size_t smem = sizeof(double) * 3 * (size_t)c->N;
+  EB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(double) * 3 * 4096)));
+  int per_sm = 0, sms = 0;
+  EB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, eb::kSafeThreads, smem));
+  EB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->cfg.device));
+  c->safe_grid = std::max(1, per_sm * sms);
+  EB_CUDA(cudaMalloc(&c->d_safe_list, sizeof(int) * (1 + B)));  // last: it marks the scratch as complete
+  return EB_OK;
+}
+}  // namespace
+
+extern "C" {
+
+eb_status eb_control_safe_batch_dev(eb_controller* c, eb_grid_batch* g, const eb_collision* col, const eb_dwa* dwa,
+                                    double val_dt, double val_horizon, const double* bounds_dev, const double* x_dev,
+                                    const int* mem_idx_dev, const double* vb_dev, double* u_dev, int* branch_dev,
+                                    double* metric_dev)
+{
+  EB_TRACE("eb_control_safe_batch_dev");
+  static const char* call = "eb_control_safe_batch_dev";
+  eb::DwaParams p{};
+  eb::MapSet m{};
+  eb_status st = safe_batch_check(c, g, col, dwa, val_dt, bounds_dev, call, &p, &m);
+  if (st != EB_OK) return st;
+  if (!x_dev || !vb_dev || !u_dev || !branch_dev) return fail(EB_ERR_INVALID_ARGUMENT, std::string(call) + ": NULL argument");
+  EB_CUDA(cudaSetDevice(c->cfg.device));
+  if ((st = ensure_safe(c)) != EB_OK) return st;
+  if (!g->maps_ready)
+  {
+    EB_CUDA(cudaEventCreateWithFlags(&g->maps_ready, cudaEventDisableTiming));
+    EB_CUDA(cudaEventCreateWithFlags(&g->ticked, cudaEventDisableTiming));
+  }
+  // after the set calls already enqueued on the grid batch's stream, without a host synchronisation
+  EB_CUDA(cudaEventRecord(g->maps_ready, g->stream));
+  EB_CUDA(cudaStreamWaitEvent(c->stream, g->maps_ready, 0));
+  EB_CUDA(cudaMemsetAsync(c->d_safe_list, 0, sizeof(int), c->stream));
+  // 1. the solve writes u0 straight into u: the validate kernel reads it there and the fallback overwrites the rows
+  //    of the robots whose twist collides
+  if ((st = eb_control_batch_dev(c, bounds_dev, x_dev, mem_idx_dev, u_dev, metric_dev)) != EB_OK) return st;
+  eb::SafeParams s{};
+  s.count = c->d_safe_list;
+  s.list = c->d_safe_list + 1;
+  s.ut = c->d_ut[c->cur];
+  s.dt = c->cfg.dt;
+  s.N = c->N;
+  s.u = u_dev;
+  s.branch = branch_dev;
+  s.fault = c->d_fault;
+  // 2. validate_control of every robot's twist on its map, failing robots listed
+  eb::CollisionParams v = p.col;
+  v.B = c->B;
+  v.x0 = x_dev;
+  v.u = u_dev;
+  v.dt = val_dt;
+  v.steps = (int)static_cast<unsigned int>(std::abs(val_horizon / val_dt));  // numerics.hpp:316
+  eb::validate_compact_kernel<<<(c->B + 127) / 128, 128, 0, c->stream>>>(v, m, s);
+  cudaError_t e = cudaGetLastError();
+  if (e == cudaSuccess)
+  {
+    // 3. the dynamic window of the listed robots against their optTraj()
+    c->launches += 1;
+    p.x0 = x_dev;
+    p.vb = vb_dev;
+    auto kernel = c->cfg.model == EB_MODEL_OMNI ? eb::dwa_fallback_kernel<eb::kModelOmni> :
+                                                  eb::dwa_fallback_kernel<eb::kModelSimpleCart>;
+    kernel<<<std::min(c->B, c->safe_grid), eb::kSafeThreads, sizeof(double) * 3 * (size_t)c->N, c->stream>>>(p, m, s);
+    e = cudaGetLastError();
+    if (e == cudaSuccess) c->launches += 1;
+  }
+  const cudaError_t r = cudaEventRecord(g->ticked, c->stream);  // the grid batch's next set call waits for this tick
+  if (e == cudaSuccess) e = r;
+  if (e != cudaSuccess) return fail(EB_ERR_CUDA, std::string(call) + ": " + cudaGetErrorString(e));
+  return EB_OK;
+}
+
+eb_status eb_control_safe_batch_host(eb_controller* c, eb_grid_batch* g, const eb_collision* col, const eb_dwa* dwa,
+                                     double val_dt, double val_horizon, const double* bounds, const double* x,
+                                     const int* mem_idx, const double* vb, double* u, int* branch, double* metric)
+{
+  EB_TRACE("eb_control_safe_batch_host");
+  static const char* call = "eb_control_safe_batch_host";
+  eb::DwaParams p{};
+  eb::MapSet m{};
+  eb_status st = safe_batch_check(c, g, col, dwa, val_dt, bounds, call, &p, &m);
+  if (st != EB_OK) return st;
+  if (!x || !vb || !u || !branch) return fail(EB_ERR_INVALID_ARGUMENT, std::string(call) + ": NULL argument");
+  EB_CUDA(cudaSetDevice(c->cfg.device));
+  if ((st = ensure_safe(c)) != EB_OK) return st;
+  const size_t B = (size_t)c->B;
+  if (bounds) EB_CUDA(cudaMemcpyAsync(c->d_bounds, bounds, sizeof(double) * 4 * B, cudaMemcpyHostToDevice, c->stream));
+  const bool need_idx = mem_idx && c->mem_count > (long long)c->cfg.batch_size;
+  if (need_idx)
+    EB_CUDA(cudaMemcpyAsync(c->d_mem_idx_in, mem_idx, sizeof(int) * (size_t)c->cfg.batch_size * B,
+                            cudaMemcpyHostToDevice, c->stream));
+  EB_CUDA(cudaMemcpyAsync(c->d_pose, x, sizeof(double) * 3 * B, cudaMemcpyHostToDevice, c->stream));
+  EB_CUDA(cudaMemcpyAsync(c->d_safe_vb, vb, sizeof(double) * 3 * B, cudaMemcpyHostToDevice, c->stream));
+  st = eb_control_safe_batch_dev(c, g, col, dwa, val_dt, val_horizon, bounds ? c->d_bounds : nullptr, c->d_pose,
+                                 need_idx ? c->d_mem_idx_in : nullptr, c->d_safe_vb, c->d_u0, c->d_safe_branch,
+                                 metric ? c->d_metric : nullptr);
+  if (st != EB_OK) return st;
+  EB_CUDA(cudaMemcpyAsync(u, c->d_u0, sizeof(double) * 3 * B, cudaMemcpyDeviceToHost, c->stream));
+  EB_CUDA(cudaMemcpyAsync(branch, c->d_safe_branch, sizeof(int) * B, cudaMemcpyDeviceToHost, c->stream));
+  if (metric) EB_CUDA(cudaMemcpyAsync(metric, c->d_metric, sizeof(double) * B, cudaMemcpyDeviceToHost, c->stream));
   return check_fault(c);  // synchronises
 }
 

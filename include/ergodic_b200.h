@@ -479,6 +479,41 @@ eb_status eb_set_map_targets_batch_host(eb_controller *c, const signed char *con
                                         const unsigned *ysize, const double *resolution, const double *origin,
                                         const int *update);
 
+/* ---- safe control tick of B robots on B maps -----------------------------------------------------------------------
+ * The reference loop's arbitration between the ergodic twist and the safety planner (exploration.hpp:238-247) for a
+ * per-instance controller and an eb_grid_batch of the same B on the same device, as one stream-ordered call with no
+ * host synchronisation.  For every robot i:
+ *   1. u0_i = what eb_control_batch_dev(c, bounds, x, mem_idx, u0, metric) returns; the controller's state (ut_, pose,
+ *      replay sampling) advances exactly as in that call, and metric (NULL: not written) is that call's;
+ *   2. ok_i = eb_validate_control_batch_dev of (x_i, u0_i) on map i with col, val_dt and val_horizon;
+ *   3. ok_i: u_i = u0_i, branch_i = 0.  Otherwise (found_i, ud_i) = eb_dwa_control_traj_batch_dev on map i with col, dwa,
+ *      vb_i and robot i's optTraj() (eb_opt_traj_dev, ncols = N, dt_ref = the controller's dt) as the reference;
+ *      found: u_i = ud_i, branch_i = 1; not found: u_i = 0, branch_i = 2.
+ * Every output equals that composition of calls bit for bit, and robot i's results depend on robot i alone.  The
+ * dynamic window runs only for the robots whose twist fails validation; the B x N x 3 optTraj is never written.
+ * Work runs on the controller's stream, after the work already enqueued on the grid batch's stream (an event: a
+ * eb_grid_batch_set_maps_dev followed by a tick needs no synchronisation), and the grid batch's next set call waits for
+ * the last tick before it writes or frees a map.  With bounds_dev NULL a tick is exactly three kernel launches, counted
+ * by eb_launch_count (solve, validate + compaction, dynamic window over the failing robots) plus a cudaMemsetAsync of a
+ * counter; given bounds add eb_control_batch_dev's frame launch.  Device-side faults of the solve surface as for
+ * eb_control_batch_dev (eb_check_status); _host copies x, vb, bounds and mem_idx in, runs, copies u, branch and metric
+ * out and synchronises.
+ * Refused before anything is launched or copied, so an error leaves the controller as it was: EB_ERR_INVALID_ARGUMENT
+ * for a NULL argument, a controller without per-instance targets (a shared target, or no eb_*_batch target call yet),
+ * bounds NULL before any frame was configured, a grid batch of another B or on another device, an instance without a
+ * map, an eb_collision the Collision constructor refuses, val_dt == 0 or dwa->dt == 0; EB_ERR_OUT_OF_RANGE when the
+ * window's rollout outlasts the N-column optTraj (as eb_dwa_control_traj_*).
+ * Not covered: the reference loop's policy of following the planner for a while once it took over, and replanning
+ * (ROS-loop policy; branch lets a caller build it), and multi-GPU (eb_control_dev_gather[_wait] stay EB_ERR_UNSUPPORTED
+ * for per-instance controllers). */
+eb_status eb_control_safe_batch_dev(eb_controller *c, eb_grid_batch *g, const eb_collision *col, const eb_dwa *dwa,
+                                    double val_dt, double val_horizon, const double *bounds_dev /* 4 x B or NULL */,
+                                    const double *x_dev /* 3 x B */, const int *mem_idx_dev, const double *vb_dev /* 3 x B */,
+                                    double *u_dev /* 3 x B */, int *branch_dev /* B */, double *metric_dev /* B or NULL */);
+eb_status eb_control_safe_batch_host(eb_controller *c, eb_grid_batch *g, const eb_collision *col, const eb_dwa *dwa,
+                                     double val_dt, double val_horizon, const double *bounds, const double *x,
+                                     const int *mem_idx, const double *vb, double *u, int *branch, double *metric);
+
 /* ---- kinematic models and the forward integrator (SURVEY.md section 8 rows a8 / a9) ----
  * model: 0 SimpleCart, 1 Omni (models/cart.hpp:152-206, models/omni.hpp:164-215), 2 Cart (cart.hpp:60-145;
  * params = { wheel_radius, wheel_base }; 2 wheel velocities), 3 Mecanum (omni.hpp:59-157; params = { wheel_radius,

@@ -10,7 +10,8 @@
  *   validate_control(collision, grid, x0, u, dt, horizon)     numerics.hpp:312-330
  *   DynamicWindow::control(grid, x0, vb, vref | xt_ref)       dynamic_window.cpp:93-187
  * for one pose / twist (the reference's signatures), for a 3 x B batch sharing one map (DeviceGrid), or for B
- * instances on B maps (DeviceGridBatch: instance i is checked against map i, one kernel launch per call).
+ * instances on B maps (DeviceGridBatch: instance i is checked against map i, one kernel launch per call); controlSafe
+ * runs the whole tick of B robots on B maps (control, validate_control, DynamicWindow where needed) as one call.
  * The grid type is anything with the reference GridMap's getters
  * (gridData(), xsize(), ysize(), resolution(), xmin(), ymin(); grid.hpp:201-255).
  * The reference's Collision keeps its radii private (collision.hpp:159-163), so the
@@ -299,11 +300,38 @@ public:
   double timeStep() const { return cfg_.dt; }
   double horizon() const { return cfg_.horizon; }
   unsigned int steps() const { return static_cast<unsigned int>(std::abs(cfg_.horizon / cfg_.dt)); }
+  const eb_dwa& config() const { return cfg_; }
 
 private:
   Collision collision_;
   eb_dwa cfg_;
 };
+
+/**
+ * @brief One safe control tick of B robots on B maps (eb_control_safe_batch_host), the reference loop's arbitration
+ * (exploration.hpp:238-247): u = ctl.control(grids, X); where validate_control(collision, grids, X, u, val_dt,
+ * val_horizon) fails, dwa.controlBatch(grids, X, VB, ctl.optTraj(), ctl's time step) takes over, and a robot whose
+ * window finds nothing gets the zero twist.  The window runs only for the robots that need it.  ctl must hold
+ * per-instance frames (setMapTargets or control(grids, x) before); they are used as they are.
+ * @return the 3 x B twists and the B branches (0 ergodic twist, 1 dynamic window, 2 nothing found)
+ */
+template <class ModelT>
+std::tuple<arma::mat, std::vector<int>> controlSafe(BatchedErgodicControl<ModelT>& ctl, const DeviceGridBatch& grids,
+                                                    const Collision& collision, const DynamicWindow& dwa,
+                                                    const arma::mat& X, const arma::mat& VB, double val_dt,
+                                                    double val_horizon)
+{
+  const unsigned int B = grids.batch();
+  if (ctl.batch() != B) throw std::logic_error("controlSafe: the controller and the grid batch need the same B");
+  if (X.n_rows != 3 || VB.n_rows != 3 || X.n_cols != B || VB.n_cols != B)
+    throw std::logic_error("controlSafe: X and VB must be 3 x B");
+  arma::mat u(3, B);
+  std::vector<int> branch(B);
+  check(eb_control_safe_batch_host(ctl.handle(), grids.handle(), &collision.config(), &dwa.config(), val_dt,
+                                   val_horizon, nullptr, X.memptr(), nullptr, VB.memptr(), u.memptr(), branch.data(),
+                                   nullptr));
+  return std::make_tuple(u, branch);
+}
 }  // namespace b200
 }  // namespace ergodic_exploration
 #endif

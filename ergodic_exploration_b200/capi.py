@@ -212,6 +212,12 @@ SIGNATURES = {
                                             _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "eb_control_safe_batch_host": (C.c_int, [_vp, _vp, C.POINTER(EbCollision), C.POINTER(EbDwa), C.c_double, C.c_double,
                                              _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "eb_control_batch_dev_gather": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp]),
+    "eb_control_batch_dev_gather_wait": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp]),
+    "eb_control_safe_batch_dev_gather": (C.c_int, [_vp, _vp, _vp, C.POINTER(EbCollision), C.POINTER(EbDwa), C.c_double,
+                                                   C.c_double, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "eb_control_safe_batch_dev_gather_wait": (C.c_int, [_vp, _vp, _vp, C.POINTER(EbCollision), C.POINTER(EbDwa),
+                                                        C.c_double, C.c_double, _vp, _vp, _vp, _vp, _vp, _vp]),
 }
 
 _lib = None

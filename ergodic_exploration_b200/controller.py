@@ -495,20 +495,11 @@ class ErgodicControl:
         on torch's current stream without a host synchronisation (``metric`` (B,) float64 and ``mem_idx`` int32 then
         tensors too).  ``bounds`` (B, 4) as in control(); None: the frames of the last configure."""
         B = self.batch
-        if grids.batch != B:
-            raise ValueError(f"control_safe: the grid batch holds {grids.batch} maps for {B} instances")
         dev = _is_cuda_tensor(x)
-        x, _, _ = grids._rows("x", x, dev, per_ok=False)
-        vb, _, _ = grids._rows("vb", vb, dev, per_ok=False)
+        x, vb = self._safe_rows(grids, x, vb, dev)
         col = dwa.collision if collision is None else collision
         if dev:
-            b = self._bounds_dev(bounds) if bounds is not None else None
-            if metric is not None and not (_is_cuda_tensor(metric) and metric.dtype == torch.float64 and
-                                           metric.is_contiguous() and tuple(metric.shape) == (B,)):
-                raise ValueError(f"metric must be a contiguous ({B},) float64 CUDA tensor on the device path")
-            if mem_idx is not None and not (_is_cuda_tensor(mem_idx) and mem_idx.dtype == torch.int32 and
-                                            mem_idx.is_contiguous()):
-                raise ValueError("mem_idx must be a contiguous int32 CUDA tensor on the device path")
+            b = self._dev_tick_args(bounds, mem_idx, metric)
             u = torch.empty((B, 3), dtype=torch.float64, device=x.device)
             branch = torch.empty(B, dtype=torch.int32, device=x.device)
             fn = self._lib.eb_control_safe_batch_dev
@@ -534,6 +525,26 @@ class ErgodicControl:
                 raise ValueError(self._lib.eb_last_error().decode())
             check(st)
         return u, branch
+
+    def _safe_rows(self, grids, x, vb, dev):
+        """x and vb of a safe tick as (B, 3) rows of the grid batch's robots, on the path of the call"""
+        if grids.batch != self.batch:
+            raise ValueError(f"control_safe: the grid batch holds {grids.batch} maps for {self.batch} instances")
+        x, _, _ = grids._rows("x", x, dev, per_ok=False)
+        vb, _, _ = grids._rows("vb", vb, dev, per_ok=False)
+        return x, vb
+
+    def _dev_tick_args(self, bounds, mem_idx, metric):
+        """the device path's bounds (B, 4) as a CUDA tensor or None, after checking metric and mem_idx"""
+        B = self.batch
+        b = self._bounds_dev(bounds) if bounds is not None else None
+        if metric is not None and not (_is_cuda_tensor(metric) and metric.dtype == torch.float64 and
+                                       metric.is_contiguous() and tuple(metric.shape) == (B,)):
+            raise ValueError(f"metric must be a contiguous ({B},) float64 CUDA tensor on the device path")
+        if mem_idx is not None and not (_is_cuda_tensor(mem_idx) and mem_idx.dtype == torch.int32 and
+                                        mem_idx.is_contiguous()):
+            raise ValueError("mem_idx must be a contiguous int32 CUDA tensor on the device path")
+        return b
 
     def check(self) -> None:
         """Synchronise and surface device-side faults of earlier device-path calls."""

@@ -1833,103 +1833,31 @@ unsigned long long eb_peer_group_steps(const eb_peer_group* g) { return g ? g->s
 // 1: a batch of this size publishes from inside the solve kernel, 0: from the group's side stream
 int eb_peer_group_fused(const eb_peer_group* g, int batch) { return (g && batch >= g->fuse_min_batch) ? 1 : 0; }
 
-// control() whose first twists land in every rank's gathered buffer (no collective call)
-eb_status eb_control_dev_gather(eb_controller* c, eb_peer_group* g, double xmin, double xmax, double ymin, double ymax,
-                                const double* x_dev, const int* mem_idx_dev, double* metric_dev)
+}  // extern "C"
+
+namespace
 {
-  EB_TRACE("eb_control_dev_gather");
-  if (!c || !g) return fail(EB_ERR_INVALID_ARGUMENT, "eb_control_dev_gather: NULL argument");
-  if (c->per_inst) return fail(EB_ERR_UNSUPPORTED, "eb_control_dev_gather: not available with per-instance targets");
-  if (!g->connected) return fail(EB_ERR_INVALID_ARGUMENT, "eb_control_dev_gather: peer group is not connected");
-  if (g->elems != 3LL * c->B) return fail(EB_ERR_INVALID_ARGUMENT, "eb_control_dev_gather: peer group sized for another batch");
-  const int parity = (int)(g->step % eb::kPeerBuffers);
-  // launching step n + 1 = g->step + 1 into the buffer of step n + 1 - kPeerBuffers: every rank must
-  // have finished step n + 2 - kPeerBuffers (its reads of the older step precede that launch)
-  const unsigned long long need =
-      g->step + 2 > (unsigned long long)eb::kPeerBuffers ? g->step + 2 - eb::kPeerBuffers : 0;
-  if (c->B < g->fuse_min_batch)
-  {
-    // single-wave batch: solve locally, publish from the group's own stream under the next step
-    EB_CUDA(cudaSetDevice(g->device));
-    if (g->step >= (unsigned long long)eb::kPeerBuffers) EB_CUDA(cudaStreamWaitEvent(c->stream, g->published[parity], 0));
-    const eb_status st =
-        eb_control_dev(c, xmin, xmax, ymin, ymax, x_dev, mem_idx_dev, g->local_u0[parity], metric_dev);
-    if (st != EB_OK) return st;
-    EB_CUDA(cudaEventRecord(g->solved[parity], c->stream));
-    EB_CUDA(cudaStreamWaitEvent(g->side, g->solved[parity], 0));
-    eb::PublishParams pp{};
-    pp.src = g->local_u0[parity];
-    pp.elems = g->elems;
-    pp.n_peer = g->world;
-    for (int r = 0; r < g->world; r++)
-    {
-      pp.dst[r] = g->peer_gathered[r][parity] + (size_t)g->rank * (size_t)g->elems;
-      pp.flag[r] = g->peer_flags[r] + g->rank;
-    }
-    pp.flag_value = g->step + 1;
-    pp.my_flags = g->flags;
-    pp.need = need;
-    pp.done_counter = g->side_counter;
-    // Few blocks on purpose: a single-wave solve kernel needs nearly every resident-CTA slot of the
-    // machine (1024 of 1036 at 4096 instances), and a publish block that is still running -- or
-    // waiting in the reuse guard for a slower rank -- when the next solve kernel starts must fit
-    // into the spare slots, or that kernel spills into a second wave.
-    const int blocks = (int)std::max<long long>(1, std::min<long long>(4, (g->elems / 2 + 4095) / 4096));
-    eb::peer_publish_kernel<<<blocks, 256, 0, g->side>>>(pp);
-    g->side_used = true;
-    EB_CUDA(cudaGetLastError());
-    EB_CUDA(cudaEventRecord(g->published[parity], g->side));
-    c->launches += 1;
-    g->step += 1;
-    return EB_OK;
-  }
-  PeerLaunch pl;
-  pl.n_peer = g->world;
-  for (int r = 0; r < g->world; r++)
-  {
-    pl.u0_peer[r] = g->peer_gathered[r][parity] + (size_t)g->rank * (size_t)g->elems;
-    pl.flag_peer[r] = g->peer_flags[r] + g->rank;
-  }
-  pl.flag_value = g->step + 1;
-  pl.done_counter = g->counter;
-  pl.my_flags = g->flags;
-  pl.need = need;
-  c->peer = &pl;
-  const eb_status st = eb_control_dev(c, xmin, xmax, ymin, ymax, x_dev, mem_idx_dev, c->d_u0, metric_dev);
-  c->peer = nullptr;
-  if (st == EB_OK) g->step += 1;
-  return st;
+// what every gathering call refuses about the group
+eb_status peer_group_check(const eb_controller* c, const eb_peer_group* g, const std::string& call)
+{
+  if (!g->connected) return fail(EB_ERR_INVALID_ARGUMENT, call + ": peer group is not connected");
+  if (g->elems != 3LL * c->B) return fail(EB_ERR_INVALID_ARGUMENT, call + ": peer group sized for another batch");
+  return EB_OK;
 }
 
-// control() + gather + wait in one call, everything on the controller's stream: when it returns (stream order), the
-// rows of EVERY rank for this step are in eb_peer_gathered_dev(g, step).  Single-wave batches publish and wait in one
-// kernel behind the solve kernel (peer_publish_wait_kernel); larger ones publish from inside the solve kernel and
-// enqueue the wait kernel.
-eb_status eb_control_dev_gather_wait(eb_controller* c, eb_peer_group* g, double xmin, double xmax, double ymin, double ymax,
-                                     const double* x_dev, const int* mem_idx_dev, double* metric_dev)
+// launching step n + 1 = g->step + 1 into the buffer of step n + 1 - kPeerBuffers: every rank must have finished step
+// n + 2 - kPeerBuffers (its reads of the older step precede that launch)
+unsigned long long peer_need(const eb_peer_group* g)
 {
-  EB_TRACE("eb_control_dev_gather_wait");
-  if (!c || !g) return fail(EB_ERR_INVALID_ARGUMENT, "eb_control_dev_gather_wait: NULL argument");
-  if (c->per_inst) return fail(EB_ERR_UNSUPPORTED, "eb_control_dev_gather_wait: not available with per-instance targets");
-  if (!g->connected) return fail(EB_ERR_INVALID_ARGUMENT, "eb_control_dev_gather_wait: peer group is not connected");
-  if (g->elems != 3LL * c->B) return fail(EB_ERR_INVALID_ARGUMENT, "eb_control_dev_gather_wait: peer group sized for another batch");
-  if (c->B >= g->fuse_min_batch)
-  {
-    eb_status st = eb_control_dev_gather(c, g, xmin, xmax, ymin, ymax, x_dev, mem_idx_dev, metric_dev);
-    if (st != EB_OK) return st;
-    return eb_peer_group_wait(g, c, g->step);
-  }
-  EB_CUDA(cudaSetDevice(g->device));
+  return g->step + 2 > (unsigned long long)eb::kPeerBuffers ? g->step + 2 - eb::kPeerBuffers : 0;
+}
+
+// the publication of this rank's block of the next step, whose twists are in src
+eb::PublishParams publish_params(const eb_peer_group* g, const double* src, unsigned int* counter)
+{
   const int parity = (int)(g->step % eb::kPeerBuffers);
-  const unsigned long long need =
-      g->step + 2 > (unsigned long long)eb::kPeerBuffers ? g->step + 2 - eb::kPeerBuffers : 0;
-  // a side-stream publication of an earlier step (mixed use of the two entry points) must have left this buffer
-  if (g->step >= (unsigned long long)eb::kPeerBuffers && g->side_used)
-    EB_CUDA(cudaStreamWaitEvent(c->stream, g->published[parity], 0));
-  const eb_status st = eb_control_dev(c, xmin, xmax, ymin, ymax, x_dev, mem_idx_dev, g->local_u0[parity], metric_dev);
-  if (st != EB_OK) return st;
   eb::PublishParams pp{};
-  pp.src = g->local_u0[parity];
+  pp.src = src;
   pp.elems = g->elems;
   pp.n_peer = g->world;
   for (int r = 0; r < g->world; r++)
@@ -1939,10 +1867,71 @@ eb_status eb_control_dev_gather_wait(eb_controller* c, eb_peer_group* g, double 
   }
   pp.flag_value = g->step + 1;
   pp.my_flags = g->flags;
-  pp.need = need;
-  pp.done_counter = g->counter;
-  const int blocks = (int)std::max<long long>(1, std::min<long long>(64, (g->elems / 2 + 255) / 256));
+  pp.need = peer_need(g);
+  pp.done_counter = counter;
+  return pp;
+}
+
+// One gathered control() step, after the caller's checks.  solve(u0) makes the step's solve launch, writing the first
+// twists to u0 (eb_control_dev or eb_control_batch_dev); while c->peer is set, the solve kernel also stores them into
+// every rank's buffer.  wait = false: eb_control_dev_gather's contract, true: eb_control_dev_gather_wait's.
+template <class Solve>
+eb_status gather_step(eb_controller* c, eb_peer_group* g, const bool wait, const Solve& solve)
+{
+  if (c->B >= g->fuse_min_batch)
   {
+    if (wait)
+    {
+      const eb_status st = gather_step(c, g, false, solve);
+      if (st != EB_OK) return st;
+      return eb_peer_group_wait(g, c, g->step);
+    }
+    const int parity = (int)(g->step % eb::kPeerBuffers);
+    PeerLaunch pl;
+    pl.n_peer = g->world;
+    for (int r = 0; r < g->world; r++)
+    {
+      pl.u0_peer[r] = g->peer_gathered[r][parity] + (size_t)g->rank * (size_t)g->elems;
+      pl.flag_peer[r] = g->peer_flags[r] + g->rank;
+    }
+    pl.flag_value = g->step + 1;
+    pl.done_counter = g->counter;
+    pl.my_flags = g->flags;
+    pl.need = peer_need(g);
+    c->peer = &pl;
+    const eb_status st = solve(c->d_u0);
+    c->peer = nullptr;
+    if (st == EB_OK) g->step += 1;
+    return st;
+  }
+  // single-wave batch: solve locally, then publish from the group's own stream under the next step (wait = false), or
+  // publish and wait in one kernel right behind the solve kernel (wait = true)
+  EB_CUDA(cudaSetDevice(g->device));
+  const int parity = (int)(g->step % eb::kPeerBuffers);
+  // a side-stream publication of an earlier step must have left this buffer
+  if (g->step >= (unsigned long long)eb::kPeerBuffers && (!wait || g->side_used))
+    EB_CUDA(cudaStreamWaitEvent(c->stream, g->published[parity], 0));
+  const eb_status st = solve(g->local_u0[parity]);
+  if (st != EB_OK) return st;
+  if (!wait)
+  {
+    EB_CUDA(cudaEventRecord(g->solved[parity], c->stream));
+    EB_CUDA(cudaStreamWaitEvent(g->side, g->solved[parity], 0));
+    const eb::PublishParams pp = publish_params(g, g->local_u0[parity], g->side_counter);
+    // Few blocks on purpose: a single-wave solve kernel needs nearly every resident-CTA slot of the
+    // machine (1024 of 1036 at 4096 instances), and a publish block that is still running -- or
+    // waiting in the reuse guard for a slower rank -- when the next solve kernel starts must fit
+    // into the spare slots, or that kernel spills into a second wave.
+    const int blocks = (int)std::max<long long>(1, std::min<long long>(4, (g->elems / 2 + 4095) / 4096));
+    eb::peer_publish_kernel<<<blocks, 256, 0, g->side>>>(pp);
+    g->side_used = true;
+    EB_CUDA(cudaGetLastError());
+    EB_CUDA(cudaEventRecord(g->published[parity], g->side));
+  }
+  else
+  {
+    const eb::PublishParams pp = publish_params(g, g->local_u0[parity], g->counter);
+    const int blocks = (int)std::max<long long>(1, std::min<long long>(64, (g->elems / 2 + 255) / 256));
     // programmatic dependent launch behind the solve kernel (and ahead of the next step's): see SolveLaunch::launch_w
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)blocks);
@@ -1958,6 +1947,75 @@ eb_status eb_control_dev_gather_wait(eb_controller* c, eb_peer_group* g, double 
   c->launches += 1;
   g->step += 1;
   return EB_OK;
+}
+
+// the checks of eb_control_batch_dev_gather[_wait]: eb_control_batch_dev's and the group's
+eb_status batch_gather_check(const eb_controller* c, const eb_peer_group* g, const double* bounds_dev,
+                             const double* x_dev, const char* call)
+{
+  if (!c || !g || !x_dev) return fail(EB_ERR_INVALID_ARGUMENT, std::string(call) + ": NULL argument");
+  if (!bounds_dev && !c->frames_set)
+    return fail(EB_ERR_INVALID_ARGUMENT, std::string(call) + ": bounds NULL before any frame was configured");
+  if (g->device != c->cfg.device)
+    return fail(EB_ERR_INVALID_ARGUMENT, std::string(call) + ": the peer group and the controller are on different devices");
+  return peer_group_check(c, g, call);
+}
+}  // namespace
+
+extern "C" {
+
+// control() whose first twists land in every rank's gathered buffer (no collective call)
+eb_status eb_control_dev_gather(eb_controller* c, eb_peer_group* g, double xmin, double xmax, double ymin, double ymax,
+                                const double* x_dev, const int* mem_idx_dev, double* metric_dev)
+{
+  EB_TRACE("eb_control_dev_gather");
+  if (!c || !g) return fail(EB_ERR_INVALID_ARGUMENT, "eb_control_dev_gather: NULL argument");
+  if (c->per_inst) return fail(EB_ERR_UNSUPPORTED, "eb_control_dev_gather: not available with per-instance targets");
+  const eb_status st = peer_group_check(c, g, "eb_control_dev_gather");
+  if (st != EB_OK) return st;
+  return gather_step(c, g, false, [&](double* u0) {
+    return eb_control_dev(c, xmin, xmax, ymin, ymax, x_dev, mem_idx_dev, u0, metric_dev);
+  });
+}
+
+// control() + gather + wait in one call, everything on the controller's stream: when it returns (stream order), the
+// rows of EVERY rank for this step are in eb_peer_gathered_dev(g, step).  Single-wave batches publish and wait in one
+// kernel behind the solve kernel (peer_publish_wait_kernel); larger ones publish from inside the solve kernel and
+// enqueue the wait kernel.
+eb_status eb_control_dev_gather_wait(eb_controller* c, eb_peer_group* g, double xmin, double xmax, double ymin, double ymax,
+                                     const double* x_dev, const int* mem_idx_dev, double* metric_dev)
+{
+  EB_TRACE("eb_control_dev_gather_wait");
+  if (!c || !g) return fail(EB_ERR_INVALID_ARGUMENT, "eb_control_dev_gather_wait: NULL argument");
+  if (c->per_inst) return fail(EB_ERR_UNSUPPORTED, "eb_control_dev_gather_wait: not available with per-instance targets");
+  const eb_status st = peer_group_check(c, g, "eb_control_dev_gather_wait");
+  if (st != EB_OK) return st;
+  return gather_step(c, g, true, [&](double* u0) {
+    return eb_control_dev(c, xmin, xmax, ymin, ymax, x_dev, mem_idx_dev, u0, metric_dev);
+  });
+}
+
+// eb_control_batch_dev whose first twists land in every rank's gathered buffer: the same machinery as the shared calls
+eb_status eb_control_batch_dev_gather(eb_controller* c, eb_peer_group* g, const double* bounds_dev, const double* x_dev,
+                                      const int* mem_idx_dev, double* metric_dev)
+{
+  EB_TRACE("eb_control_batch_dev_gather");
+  const eb_status st = batch_gather_check(c, g, bounds_dev, x_dev, "eb_control_batch_dev_gather");
+  if (st != EB_OK) return st;
+  return gather_step(c, g, false, [&](double* u0) {
+    return eb_control_batch_dev(c, bounds_dev, x_dev, mem_idx_dev, u0, metric_dev);
+  });
+}
+
+eb_status eb_control_batch_dev_gather_wait(eb_controller* c, eb_peer_group* g, const double* bounds_dev,
+                                           const double* x_dev, const int* mem_idx_dev, double* metric_dev)
+{
+  EB_TRACE("eb_control_batch_dev_gather_wait");
+  const eb_status st = batch_gather_check(c, g, bounds_dev, x_dev, "eb_control_batch_dev_gather_wait");
+  if (st != EB_OK) return st;
+  return gather_step(c, g, true, [&](double* u0) {
+    return eb_control_batch_dev(c, bounds_dev, x_dev, mem_idx_dev, u0, metric_dev);
+  });
 }
 
 // enqueues (on the controller's stream) a wait until every rank's rows of step `step` have arrived here
@@ -3680,16 +3738,130 @@ eb_status ensure_safe(eb_controller* c)
   const size_t B = (size_t)c->B;
   EB_CUDA(cudaMalloc(&c->d_safe_branch, sizeof(int) * B));
   EB_CUDA(cudaMalloc(&c->d_safe_vb, sizeof(double) * 3 * B));
-  auto kernel = c->cfg.model == EB_MODEL_OMNI ? eb::dwa_fallback_kernel<eb::kModelOmni> :
-                                                eb::dwa_fallback_kernel<eb::kModelSimpleCart>;
+  const bool omni = c->cfg.model == EB_MODEL_OMNI;
+  auto kernel = omni ? eb::dwa_fallback_kernel<eb::kModelOmni, false> : eb::dwa_fallback_kernel<eb::kModelSimpleCart, false>;
+  auto publishing = omni ? eb::dwa_fallback_kernel<eb::kModelOmni, true> : eb::dwa_fallback_kernel<eb::kModelSimpleCart, true>;
   const size_t smem = sizeof(double) * 3 * (size_t)c->N;
   EB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(double) * 3 * 4096)));
+  EB_CUDA(cudaFuncSetAttribute(publishing, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(double) * 3 * 4096)));
   int per_sm = 0, sms = 0;
   EB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, eb::kSafeThreads, smem));
   EB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->cfg.device));
   c->safe_grid = std::max(1, per_sm * sms);
   EB_CUDA(cudaMalloc(&c->d_safe_list, sizeof(int) * (1 + B)));  // last: it marks the scratch as complete
   return EB_OK;
+}
+}  // namespace
+
+extern "C" {
+
+}  // extern "C"
+
+namespace
+{
+// The tick's launches after its checks: the solve writes u0 into u, validate_compact_kernel lists the failing robots
+// and dwa_fallback_kernel overwrites their rows.  With pub (a peer group's step), both kernels also store the rows they
+// decide into every rank's gathered buffer and the fallback raises the arrival flags (safe_control.cuh).
+eb_status safe_tick(eb_controller* c, eb_grid_batch* g, eb::DwaParams& p, const eb::MapSet& m, double val_dt,
+                    double val_horizon, const double* bounds_dev, const double* x_dev, const int* mem_idx_dev,
+                    const double* vb_dev, double* u_dev, int* branch_dev, double* metric_dev,
+                    const eb::SafePublishParams* pub, const char* call)
+{
+  EB_CUDA(cudaSetDevice(c->cfg.device));
+  eb_status st = ensure_safe(c);
+  if (st != EB_OK) return st;
+  if (!g->maps_ready)
+  {
+    EB_CUDA(cudaEventCreateWithFlags(&g->maps_ready, cudaEventDisableTiming));
+    EB_CUDA(cudaEventCreateWithFlags(&g->ticked, cudaEventDisableTiming));
+  }
+  // after the set calls already enqueued on the grid batch's stream, without a host synchronisation
+  EB_CUDA(cudaEventRecord(g->maps_ready, g->stream));
+  EB_CUDA(cudaStreamWaitEvent(c->stream, g->maps_ready, 0));
+  EB_CUDA(cudaMemsetAsync(c->d_safe_list, 0, sizeof(int), c->stream));
+  // 1. the solve writes u0 straight into u: the validate kernel reads it there and the fallback overwrites the rows
+  //    of the robots whose twist collides
+  if ((st = eb_control_batch_dev(c, bounds_dev, x_dev, mem_idx_dev, u_dev, metric_dev)) != EB_OK) return st;
+  eb::SafePublishParams s{};
+  if (pub) s = *pub;
+  s.count = c->d_safe_list;
+  s.list = c->d_safe_list + 1;
+  s.ut = c->d_ut[c->cur];
+  s.dt = c->cfg.dt;
+  s.N = c->N;
+  s.u = u_dev;
+  s.branch = branch_dev;
+  s.fault = c->d_fault;
+  // 2. validate_control of every robot's twist on its map, failing robots listed
+  eb::CollisionParams v = p.col;
+  v.B = c->B;
+  v.x0 = x_dev;
+  v.u = u_dev;
+  v.dt = val_dt;
+  v.steps = (int)static_cast<unsigned int>(std::abs(val_horizon / val_dt));  // numerics.hpp:316
+  const int vblocks = (c->B + 127) / 128, fblocks = std::min(c->B, c->safe_grid);
+  if (pub)
+  {
+    s.arrivals = (unsigned int)(vblocks * (128 / 32) + fblocks);
+    eb::validate_compact_kernel<true><<<vblocks, 128, 0, c->stream>>>(v, m, s);
+  }
+  else
+    eb::validate_compact_kernel<false><<<vblocks, 128, 0, c->stream>>>(v, m, s);
+  cudaError_t e = cudaGetLastError();
+  if (e == cudaSuccess)
+  {
+    // 3. the dynamic window of the listed robots against their optTraj()
+    c->launches += 1;
+    p.x0 = x_dev;
+    p.vb = vb_dev;
+    const size_t smem = sizeof(double) * 3 * (size_t)c->N;
+    const bool omni = c->cfg.model == EB_MODEL_OMNI;
+    if (pub)
+      (omni ? eb::dwa_fallback_kernel<eb::kModelOmni, true> : eb::dwa_fallback_kernel<eb::kModelSimpleCart, true>)
+          <<<fblocks, eb::kSafeThreads, smem, c->stream>>>(p, m, s);
+    else
+      (omni ? eb::dwa_fallback_kernel<eb::kModelOmni, false> : eb::dwa_fallback_kernel<eb::kModelSimpleCart, false>)
+          <<<fblocks, eb::kSafeThreads, smem, c->stream>>>(p, m, s);
+    e = cudaGetLastError();
+    if (e == cudaSuccess) c->launches += 1;
+  }
+  const cudaError_t r = cudaEventRecord(g->ticked, c->stream);  // the grid batch's next set call waits for this tick
+  if (e == cudaSuccess) e = r;
+  if (e != cudaSuccess) return fail(EB_ERR_CUDA, std::string(call) + ": " + cudaGetErrorString(e));
+  return EB_OK;
+}
+
+// eb_control_safe_batch_dev_gather[_wait]: the tick whose final twists land in every rank's gathered buffer
+eb_status safe_gather(eb_controller* c, eb_peer_group* pg, eb_grid_batch* g, const eb_collision* col, const eb_dwa* dwa,
+                      double val_dt, double val_horizon, const double* bounds_dev, const double* x_dev,
+                      const int* mem_idx_dev, const double* vb_dev, int* branch_dev, double* metric_dev, bool wait,
+                      const char* call)
+{
+  eb::DwaParams p{};
+  eb::MapSet m{};
+  eb_status st = safe_batch_check(c, g, col, dwa, val_dt, bounds_dev, call, &p, &m);
+  if (st != EB_OK) return st;
+  if (!pg || !x_dev || !vb_dev || !branch_dev) return fail(EB_ERR_INVALID_ARGUMENT, std::string(call) + ": NULL argument");
+  if (pg->device != c->cfg.device)
+    return fail(EB_ERR_INVALID_ARGUMENT, std::string(call) + ": the peer group and the controller are on different devices");
+  if ((st = peer_group_check(c, pg, call)) != EB_OK) return st;
+  EB_CUDA(cudaSetDevice(c->cfg.device));
+  if (pg->side_used)
+  {
+    // side-stream publications of earlier steps (eb_control_*_gather on a single-wave batch): the one into this
+    // step's buffer must have left it, and the last one must have raised its flags before this step raises higher ones
+    const unsigned long long n = pg->step;
+    if (n >= (unsigned long long)eb::kPeerBuffers) EB_CUDA(cudaStreamWaitEvent(c->stream, pg->published[n % eb::kPeerBuffers], 0));
+    if (n >= 1) EB_CUDA(cudaStreamWaitEvent(c->stream, pg->published[(n - 1) % eb::kPeerBuffers], 0));
+  }
+  eb::SafePublishParams pub{};
+  pub.peer = publish_params(pg, nullptr, pg->counter);
+  pub.wait = wait ? 1 : 0;
+  // the solve writes its twists into the controller's scratch, not to the peers: they are final only after the window
+  st = safe_tick(c, g, p, m, val_dt, val_horizon, bounds_dev, x_dev, mem_idx_dev, vb_dev, c->d_u0, branch_dev,
+                 metric_dev, &pub, call);
+  if (st == EB_OK) pg->step += 1;
+  return st;
 }
 }  // namespace
 
@@ -3707,54 +3879,29 @@ eb_status eb_control_safe_batch_dev(eb_controller* c, eb_grid_batch* g, const eb
   eb_status st = safe_batch_check(c, g, col, dwa, val_dt, bounds_dev, call, &p, &m);
   if (st != EB_OK) return st;
   if (!x_dev || !vb_dev || !u_dev || !branch_dev) return fail(EB_ERR_INVALID_ARGUMENT, std::string(call) + ": NULL argument");
-  EB_CUDA(cudaSetDevice(c->cfg.device));
-  if ((st = ensure_safe(c)) != EB_OK) return st;
-  if (!g->maps_ready)
-  {
-    EB_CUDA(cudaEventCreateWithFlags(&g->maps_ready, cudaEventDisableTiming));
-    EB_CUDA(cudaEventCreateWithFlags(&g->ticked, cudaEventDisableTiming));
-  }
-  // after the set calls already enqueued on the grid batch's stream, without a host synchronisation
-  EB_CUDA(cudaEventRecord(g->maps_ready, g->stream));
-  EB_CUDA(cudaStreamWaitEvent(c->stream, g->maps_ready, 0));
-  EB_CUDA(cudaMemsetAsync(c->d_safe_list, 0, sizeof(int), c->stream));
-  // 1. the solve writes u0 straight into u: the validate kernel reads it there and the fallback overwrites the rows
-  //    of the robots whose twist collides
-  if ((st = eb_control_batch_dev(c, bounds_dev, x_dev, mem_idx_dev, u_dev, metric_dev)) != EB_OK) return st;
-  eb::SafeParams s{};
-  s.count = c->d_safe_list;
-  s.list = c->d_safe_list + 1;
-  s.ut = c->d_ut[c->cur];
-  s.dt = c->cfg.dt;
-  s.N = c->N;
-  s.u = u_dev;
-  s.branch = branch_dev;
-  s.fault = c->d_fault;
-  // 2. validate_control of every robot's twist on its map, failing robots listed
-  eb::CollisionParams v = p.col;
-  v.B = c->B;
-  v.x0 = x_dev;
-  v.u = u_dev;
-  v.dt = val_dt;
-  v.steps = (int)static_cast<unsigned int>(std::abs(val_horizon / val_dt));  // numerics.hpp:316
-  eb::validate_compact_kernel<<<(c->B + 127) / 128, 128, 0, c->stream>>>(v, m, s);
-  cudaError_t e = cudaGetLastError();
-  if (e == cudaSuccess)
-  {
-    // 3. the dynamic window of the listed robots against their optTraj()
-    c->launches += 1;
-    p.x0 = x_dev;
-    p.vb = vb_dev;
-    auto kernel = c->cfg.model == EB_MODEL_OMNI ? eb::dwa_fallback_kernel<eb::kModelOmni> :
-                                                  eb::dwa_fallback_kernel<eb::kModelSimpleCart>;
-    kernel<<<std::min(c->B, c->safe_grid), eb::kSafeThreads, sizeof(double) * 3 * (size_t)c->N, c->stream>>>(p, m, s);
-    e = cudaGetLastError();
-    if (e == cudaSuccess) c->launches += 1;
-  }
-  const cudaError_t r = cudaEventRecord(g->ticked, c->stream);  // the grid batch's next set call waits for this tick
-  if (e == cudaSuccess) e = r;
-  if (e != cudaSuccess) return fail(EB_ERR_CUDA, std::string(call) + ": " + cudaGetErrorString(e));
-  return EB_OK;
+  return safe_tick(c, g, p, m, val_dt, val_horizon, bounds_dev, x_dev, mem_idx_dev, vb_dev, u_dev, branch_dev,
+                   metric_dev, nullptr, call);
+}
+
+eb_status eb_control_safe_batch_dev_gather(eb_controller* c, eb_peer_group* pg, eb_grid_batch* g, const eb_collision* col,
+                                           const eb_dwa* dwa, double val_dt, double val_horizon, const double* bounds_dev,
+                                           const double* x_dev, const int* mem_idx_dev, const double* vb_dev,
+                                           int* branch_dev, double* metric_dev)
+{
+  EB_TRACE("eb_control_safe_batch_dev_gather");
+  return safe_gather(c, pg, g, col, dwa, val_dt, val_horizon, bounds_dev, x_dev, mem_idx_dev, vb_dev, branch_dev,
+                     metric_dev, false, "eb_control_safe_batch_dev_gather");
+}
+
+eb_status eb_control_safe_batch_dev_gather_wait(eb_controller* c, eb_peer_group* pg, eb_grid_batch* g,
+                                                const eb_collision* col, const eb_dwa* dwa, double val_dt,
+                                                double val_horizon, const double* bounds_dev, const double* x_dev,
+                                                const int* mem_idx_dev, const double* vb_dev, int* branch_dev,
+                                                double* metric_dev)
+{
+  EB_TRACE("eb_control_safe_batch_dev_gather_wait");
+  return safe_gather(c, pg, g, col, dwa, val_dt, val_horizon, bounds_dev, x_dev, mem_idx_dev, vb_dev, branch_dev,
+                     metric_dev, true, "eb_control_safe_batch_dev_gather_wait");
 }
 
 eb_status eb_control_safe_batch_host(eb_controller* c, eb_grid_batch* g, const eb_collision* col, const eb_dwa* dwa,

@@ -17,9 +17,19 @@
 //    helpers dwa_control_kernel uses.
 // CTA per robot rather than dwa_control_kernel's warp per robot: when few robots fail, the call's latency is one
 // robot's window, and one candidate per thread evaluates a 3 x 8 x 5 window in one round of rollouts instead of four.
+//
+// Multi-GPU (eb_control_safe_batch_dev_gather[_wait], PUBLISH = true): a robot's final twist is known only in one of the
+// two kernels, so each of them stores the rows it decides straight into every rank's gathered buffer over peer memory
+// (peer_gather.cuh's layout and reuse guard): the validation kernel the rows of the valid robots -- they travel while
+// the window runs -- and the fallback the rows of the listed ones.  The fallback's last CTA raises this rank's arrival
+// flag on every peer and, in the _wait form, waits for every rank's.  The PUBLISH = false instantiations are the
+// single-GPU tick.
 #pragma once
 
+#include <type_traits>
+
 #include "collision_kernels.cuh"
+#include "peer_gather.cuh"
 #include "solve_kernel.cuh"
 
 namespace eb
@@ -38,12 +48,59 @@ struct SafeParams
   int* fault;        // SimpleCart twist with a y-velocity (rollout_kernel)
 };
 
+// the safe tick whose twists also go to every rank of a peer group
+struct SafePublishParams : SafeParams
+{
+  PublishParams peer;     // dst / flag / flag_value / my_flags / need / done_counter of the step (src, elems unused)
+  unsigned int arrivals;  // what counts out on peer.done_counter: every validation warp, then every fallback CTA
+  int wait;               // 1: the fallback's last CTA also waits for every rank's flag (the _wait form)
+};
+
+template <bool PUBLISH>
+using SafeArgs = std::conditional_t<PUBLISH, SafePublishParams, SafeParams>;
+
+// peer_gather.cuh's reuse guard, by one warp before it stores into this step's buffer: every rank has finished the step
+// that last read it
+__device__ __forceinline__ void peer_reuse_guard(const PublishParams& pp, const int lane)
+{
+  if (lane < pp.n_peer)
+    while (*(const volatile unsigned long long*)(pp.my_flags + lane) < pp.need) __nanosleep(100);
+  __syncwarp();
+}
+
+// one robot's final twist into its row of every rank's gathered buffer
+__device__ __forceinline__ void peer_store_row(const PublishParams& pp, const size_t inst, const double u0, const double u1,
+                                               const double u2)
+{
+#pragma unroll
+  for (int q = 0; q < kPublishPeers; q++)
+    if (q < pp.n_peer)
+    {
+      pp.dst[q][inst * 3 + 0] = u0;
+      pp.dst[q][inst * 3 + 1] = u1;
+      pp.dst[q][inst * 3 + 2] = u2;
+    }
+}
+
 // p.x0 = the poses, p.u = the solve's twists: branch 0 for a valid twist, else the robot goes on the list
-__global__ void __launch_bounds__(128) validate_compact_kernel(const CollisionParams p, const MapSet m, const SafeParams s)
+template <bool PUBLISH>
+__global__ void __launch_bounds__(128) validate_compact_kernel(const CollisionParams p, const MapSet m, const SafeArgs<PUBLISH> s)
 {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   const bool fails = i < p.B && !validate_control_ok(on_map(p, m, i), i);
   if (i < p.B && !fails) s.branch[i] = 0;
+  if constexpr (PUBLISH)
+  {
+    // A valid robot's twist is final: its row goes to every rank now, while the window of the failing ones runs.
+    // Then every warp releases its rows at GPU scope into the arrival counter; the fallback's last CTA takes them up
+    // (see there), so no warp here pays for a system-scope fence.
+    const int lane = threadIdx.x & 31;
+    peer_reuse_guard(s.peer, lane);
+    if (i < p.B && !fails) peer_store_row(s.peer, i, p.u[(size_t)i * 3 + 0], p.u[(size_t)i * 3 + 1], p.u[(size_t)i * 3 + 2]);
+    __threadfence();
+    __syncwarp();
+    if (lane == 0) atomicAdd(s.peer.done_counter, 1u);
+  }
   const unsigned int mask = __ballot_sync(kFull, fails);
   if (mask == 0) return;
   const int lane = threadIdx.x & 31, leader = __ffs(mask) - 1;
@@ -54,8 +111,8 @@ __global__ void __launch_bounds__(128) validate_compact_kernel(const CollisionPa
 }
 
 // robot i of the list: p.x0 the poses, p.vb the body twists, p.ncols = N and p.tf = N * dt (the optTraj reference)
-template <int MODEL>
-__global__ void __launch_bounds__(kSafeThreads) dwa_fallback_kernel(const DwaParams p, const MapSet m, const SafeParams s)
+template <int MODEL, bool PUBLISH>
+__global__ void __launch_bounds__(kSafeThreads) dwa_fallback_kernel(const DwaParams p, const MapSet m, const SafeArgs<PUBLISH> s)
 {
   extern __shared__ double s_xt[];  // [N][3]: the robot's optTraj()
   __shared__ double w_best[kSafeThreads / 32];
@@ -126,6 +183,7 @@ __global__ void __launch_bounds__(kSafeThreads) dwa_fallback_kernel(const DwaPar
       best = lane < kSafeThreads / 32 ? w_best[lane] : kDblMax;
       best_c = lane < kSafeThreads / 32 ? w_c[lane] : 0xffffffffu;
       dwa_argmin_warp(best, best_c);
+      if constexpr (PUBLISH) peer_reuse_guard(s.peer, lane);
       if (lane == 0)
       {
         double u0 = 0.0, u1 = 0.0, u2 = 0.0;  // nothing found: the zero twist
@@ -135,9 +193,43 @@ __global__ void __launch_bounds__(kSafeThreads) dwa_fallback_kernel(const DwaPar
         s.u[(size_t)inst * 3 + 1] = u1;
         s.u[(size_t)inst * 3 + 2] = u2;
         s.branch[inst] = found ? 1 : 2;
+        if constexpr (PUBLISH) peer_store_row(s.peer, inst, u0, u1, u2);
       }
     }
     __syncthreads();  // s_xt and the warp minima are the next robot's
+  }
+  if constexpr (PUBLISH)
+  {
+    // Every CTA counts out, also one whose stride found no robot: the list's length is known only on the device.
+    // Memory ordering, as in publish_first_twist (solve_kernel.cuh): thread 0 stored this CTA's rows; its GPU-scope
+    // fence and counter increment release them, and every validation warp did the same for its rows before.  The
+    // increments are atomic RMWs on one counter of this device, so the last CTA's increment reads a value that
+    // follows all of them, synchronises with each of those releases at GPU scope, and its system-scope fence is
+    // cumulative over every row they released -- of both kernels.  The argument needs no ordering from the kernel
+    // boundary: the PTX memory model says nothing about stream order, and a peer reading the flag is not on this stream.
+    __shared__ unsigned int s_last;
+    if (threadIdx.x == 0)
+    {
+      __threadfence();
+      const unsigned int prev = atomicAdd(s.peer.done_counter, 1u);
+      s_last = prev == s.arrivals - 1u ? 1u : 0u;
+      if (s_last)
+      {
+        *s.peer.done_counter = 0u;  // ready for the next step on this stream
+        __threadfence_system();
+#pragma unroll
+        for (int q = 0; q < kPublishPeers; q++)
+          if (q < s.peer.n_peer) *(volatile unsigned long long*)s.peer.flag[q] = s.peer.flag_value;
+      }
+    }
+    __syncthreads();
+    if (s.wait && s_last)
+    {  // peer_publish_wait_kernel's wait: every rank's rows of this step are here for what follows on the stream
+      if (threadIdx.x < s.peer.n_peer)
+        while (*(const volatile unsigned long long*)(s.peer.my_flags + threadIdx.x) < s.peer.flag_value) __nanosleep(64);
+      __syncthreads();
+      __threadfence_system();  // acquire
+    }
   }
 }
 }  // namespace eb

@@ -12,7 +12,9 @@ The hot path shards by construction (SURVEY.md §8e):
   * PeerGather replaces that per-step all_gather by the fused gather of
     csrc/peer_gather.cuh: every rank maps the others' gathered buffers once
     (CUDA IPC, NVLink peer memory) and the solve kernel itself stores its rows
-    into all of them -- no collective call inside the step.
+    into all of them -- no collective call inside the step.  Its control_batch /
+    control_safe do the same for per-instance controllers and the safe tick of
+    B robots on B maps (the validation and fallback kernels store the rows).
 Nothing here computes; it only decides who owns what and moves results.
 """
 from __future__ import annotations
@@ -233,6 +235,70 @@ class PeerGather:
             raise ValueError(self._lib.eb_last_error().decode())
         check(st)
         return self.steps
+
+    def _ctl(self, ctl):
+        ctl = self.ctl if ctl is None else ctl
+        assert ctl.batch == self.ctl.batch and ctl.device == self.ctl.device
+        return ctl
+
+    def _raise(self, st):
+        if st == capi.EB_ERR_INVALID_ARGUMENT:
+            raise ValueError(self._lib.eb_last_error().decode())
+        check(st)
+
+    def _batch(self, fn, bounds, x, mem_idx, metric, ctl) -> int:
+        ctl = self._ctl(ctl)
+        if not (torch.is_tensor(x) and x.is_cuda and x.dtype == torch.float64 and x.is_contiguous()
+                and x.numel() == 3 * ctl.batch):
+            raise ValueError(f"x must be a contiguous ({ctl.batch}, 3) float64 CUDA tensor")
+        b = ctl._dev_tick_args(bounds, mem_idx, metric)
+        ctl._sync_stream()
+        P = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None
+        self._raise(fn(ctl._h, self._h, P(b), P(x), P(mem_idx), P(metric)))
+        return self.steps
+
+    def control_batch(self, bounds, x: torch.Tensor, mem_idx: Optional[torch.Tensor] = None,
+                      metric: Optional[torch.Tensor] = None, ctl=None) -> int:
+        """ErgodicControl.control(bounds, x) of a per-instance controller (``bounds`` (B, 4) or None: the frames of
+        the last configure) whose twists land in every rank's gathered buffer (eb_control_batch_dev_gather); returns
+        the step number, whose rows ``gathered(step)`` holds once ``wait(step)`` has passed.  CUDA tensors only."""
+        return self._batch(self._lib.eb_control_batch_dev_gather, bounds, x, mem_idx, metric, ctl)
+
+    def control_batch_wait(self, bounds, x: torch.Tensor, mem_idx: Optional[torch.Tensor] = None,
+                           metric: Optional[torch.Tensor] = None, ctl=None) -> int:
+        """control_batch + wait as one stream-ordered operation (eb_control_batch_dev_gather_wait)"""
+        return self._batch(self._lib.eb_control_batch_dev_gather_wait, bounds, x, mem_idx, metric, ctl)
+
+    def _safe(self, fn, grids, dwa, x, vb, val_dt, val_horizon, bounds, mem_idx, metric, collision, ctl):
+        ctl = self._ctl(ctl)
+        if not torch.is_tensor(x) or not x.is_cuda:
+            raise ValueError("PeerGather.control_safe takes CUDA tensors")
+        x, vb = ctl._safe_rows(grids, x, vb, True)
+        b = ctl._dev_tick_args(bounds, mem_idx, metric)
+        col = dwa.collision if collision is None else collision
+        branch = torch.empty(ctl.batch, dtype=torch.int32, device=x.device)
+        ctl._sync_stream()
+        grids._stream()
+        P = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None
+        self._raise(fn(ctl._h, self._h, grids._h, C.byref(col.cfg), C.byref(dwa.cfg), float(val_dt), float(val_horizon),
+                       P(b), P(x), P(mem_idx), P(vb), P(branch), P(metric)))
+        return self.steps, branch
+
+    def control_safe(self, grids, dwa, x: torch.Tensor, vb: torch.Tensor, val_dt: float, val_horizon: float,
+                     bounds=None, mem_idx: Optional[torch.Tensor] = None, metric: Optional[torch.Tensor] = None,
+                     collision=None, ctl=None):
+        """ErgodicControl.control_safe on the device path whose final twists u land in every rank's gathered buffer
+        (eb_control_safe_batch_dev_gather).  Returns (step, branch): ``gathered(step)`` holds every rank's u once
+        ``wait(step)`` has passed; branch (B,) int32 stays local."""
+        return self._safe(self._lib.eb_control_safe_batch_dev_gather, grids, dwa, x, vb, val_dt, val_horizon, bounds,
+                          mem_idx, metric, collision, ctl)
+
+    def control_safe_wait(self, grids, dwa, x: torch.Tensor, vb: torch.Tensor, val_dt: float, val_horizon: float,
+                          bounds=None, mem_idx: Optional[torch.Tensor] = None, metric: Optional[torch.Tensor] = None,
+                          collision=None, ctl=None):
+        """control_safe + wait as one stream-ordered operation (eb_control_safe_batch_dev_gather_wait)"""
+        return self._safe(self._lib.eb_control_safe_batch_dev_gather_wait, grids, dwa, x, vb, val_dt, val_horizon,
+                          bounds, mem_idx, metric, collision, ctl)
 
     def wait(self, step: Optional[int] = None) -> None:
         """enqueue (on the current stream) a wait until every rank's rows of ``step`` are here"""

@@ -428,7 +428,8 @@ eb_status eb_set_phik_dev(eb_controller *c, const double *phik_dev, double lx, d
  * Every instance owns its target, phi_k and map frame, as B reference ErgodicControl objects each driven with its own
  * GridMap would.  The first of these calls switches the controller to per-instance mode; from then on the shared target
  * calls (eb_set_target_gaussians, eb_config_target, eb_set_phik, eb_set_phik_dev, eb_get_phik, eb_control_host / _dev)
- * return EB_ERR_INVALID_ARGUMENT and eb_control_dev_gather[_wait] EB_ERR_UNSUPPORTED.  Layouts are column-major
+ * return EB_ERR_INVALID_ARGUMENT and eb_control_dev_gather[_wait] EB_ERR_UNSUPPORTED (eb_control_batch_dev_gather[_wait]
+ * below gather per-instance twists).  Layouts are column-major
  * (Armadillo): instance i owns column i.
  * eb_set_target_gaussians_batch: Target::setTarget per instance; counts[i] <= max_n <= 256 Gaussians of instance i in
  *   columns of mu / sigma (2 x max_n x B).  Does not rebuild phi_k by itself.
@@ -504,8 +505,7 @@ eb_status eb_set_map_targets_batch_host(eb_controller *c, const signed char *con
  * map, an eb_collision the Collision constructor refuses, val_dt == 0 or dwa->dt == 0; EB_ERR_OUT_OF_RANGE when the
  * window's rollout outlasts the N-column optTraj (as eb_dwa_control_traj_*).
  * Not covered: the reference loop's policy of following the planner for a while once it took over, and replanning
- * (ROS-loop policy; branch lets a caller build it), and multi-GPU (eb_control_dev_gather[_wait] stay EB_ERR_UNSUPPORTED
- * for per-instance controllers). */
+ * (ROS-loop policy; branch lets a caller build it). */
 eb_status eb_control_safe_batch_dev(eb_controller *c, eb_grid_batch *g, const eb_collision *col, const eb_dwa *dwa,
                                     double val_dt, double val_horizon, const double *bounds_dev /* 4 x B or NULL */,
                                     const double *x_dev /* 3 x B */, const int *mem_idx_dev, const double *vb_dev /* 3 x B */,
@@ -513,6 +513,42 @@ eb_status eb_control_safe_batch_dev(eb_controller *c, eb_grid_batch *g, const eb
 eb_status eb_control_safe_batch_host(eb_controller *c, eb_grid_batch *g, const eb_collision *col, const eb_dwa *dwa,
                                      double val_dt, double val_horizon, const double *bounds, const double *x,
                                      const int *mem_idx, const double *vb, double *u, int *branch, double *metric);
+
+/* ---- per-instance control and the safe tick on several GPUs ------------------------------------------------------
+ * The per-instance counterparts of eb_control_dev_gather[_wait]: each rank of an eb_peer_group (elems = 3 * B, created
+ * on the controller's device) runs its B robots, and the twists land in every rank's gathered buffer over peer memory,
+ * with no collective call.  Each call is one step of the group (eb_peer_group_steps advances by one; a group's steps may
+ * mix these calls and eb_peer_group_wait), and after it rows [rank * B, (rank + 1) * B) of eb_peer_gathered_dev(pg,
+ * step) on every rank hold, bit for bit, what this rank's
+ *   eb_control_batch_dev_gather[_wait]:      eb_control_batch_dev(c, bounds_dev, x_dev, mem_idx_dev, u0, metric_dev)
+ *   eb_control_safe_batch_dev_gather[_wait]: eb_control_safe_batch_dev(c, g, col, dwa, ..., u, branch_dev, metric_dev)
+ * returns as u0 / u.  The controller's state advances exactly as in that call; branch_dev (B) and metric_dev (B, may be
+ * NULL) are this rank's local outputs.  Plain forms: the rows are here after eb_peer_group_wait(pg, c, step).  _wait
+ * forms: when the enqueued work has run, every rank's rows of the step are here; everything runs on the controller's
+ * stream.  The buffers rotate and are reused as for eb_control_dev_gather.
+ * eb_control_batch_dev_gather[_wait] publish as eb_control_dev_gather[_wait] do for the same batch size: from inside the
+ * solve kernel (batch >= eb_gather_fuse_min_batch()), else through peer_publish_kernel on the group's stream (or
+ * peer_publish_wait_kernel behind the solve kernel for _wait).  eb_control_safe_batch_dev_gather[_wait] are the safe
+ * tick's three launches (plus its counter memset): the solve writes to controller scratch, the validation stores the
+ * rows of the valid robots to every rank, the dynamic window those of the failing ones, raises the arrival flags and,
+ * for _wait, waits for every rank's.  Given bounds add one frame launch, as in the single-GPU calls.
+ * Refused, with nothing launched and the step counter unchanged: whatever the single-GPU call refuses, a NULL or
+ * unconnected group or one sized for another batch (as eb_control_dev_gather), and a group on another device than the
+ * controller (EB_ERR_INVALID_ARGUMENT). */
+eb_status eb_control_batch_dev_gather(eb_controller *c, eb_peer_group *pg, const double *bounds_dev /* 4 x B or NULL */,
+                                      const double *x_dev, const int *mem_idx_dev, double *metric_dev);
+eb_status eb_control_batch_dev_gather_wait(eb_controller *c, eb_peer_group *pg, const double *bounds_dev,
+                                           const double *x_dev, const int *mem_idx_dev, double *metric_dev);
+eb_status eb_control_safe_batch_dev_gather(eb_controller *c, eb_peer_group *pg, eb_grid_batch *g, const eb_collision *col,
+                                           const eb_dwa *dwa, double val_dt, double val_horizon,
+                                           const double *bounds_dev /* 4 x B or NULL */, const double *x_dev,
+                                           const int *mem_idx_dev, const double *vb_dev, int *branch_dev,
+                                           double *metric_dev);
+eb_status eb_control_safe_batch_dev_gather_wait(eb_controller *c, eb_peer_group *pg, eb_grid_batch *g,
+                                                const eb_collision *col, const eb_dwa *dwa, double val_dt,
+                                                double val_horizon, const double *bounds_dev, const double *x_dev,
+                                                const int *mem_idx_dev, const double *vb_dev, int *branch_dev,
+                                                double *metric_dev);
 
 /* ---- kinematic models and the forward integrator (SURVEY.md section 8 rows a8 / a9) ----
  * model: 0 SimpleCart, 1 Omni (models/cart.hpp:152-206, models/omni.hpp:164-215), 2 Cart (cart.hpp:60-145;

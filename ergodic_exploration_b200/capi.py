@@ -173,6 +173,7 @@ SIGNATURES = {
     "eb_control_batch_host": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp]),
     "eb_set_map_targets_batch_dev": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "eb_set_map_targets_batch_host": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "eb_set_map_targets_from_grid_batch": (C.c_int, [_vp, _vp, _vp, _vp, _vp]),
     "eb_model_controls": (C.c_int, [C.c_int]),
     "eb_rk4_solve_host": (C.c_int, [C.c_int, C.c_int, _vp, C.c_double, C.c_double, _vp, _vp, C.c_int, C.c_int, _vp]),
     "eb_rk4_solve_dev": (C.c_int, [C.c_int, C.c_int, _vp, C.c_double, C.c_double, _vp, _vp, C.c_int, C.c_int, _vp, _vp, _vp]),
@@ -194,6 +195,9 @@ SIGNATURES = {
     "eb_grid_batch_launch_count": (C.c_longlong, [_vp]),
     "eb_grid_batch_set_maps_dev": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "eb_grid_batch_set_maps_host": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "eb_grid_batch_set_rows_dev": (C.c_int, [_vp, _vp, _vp, _vp, _vp]),
+    "eb_grid_batch_set_rows_host": (C.c_int, [_vp, _vp, _vp, _vp, _vp]),
+    "eb_grid_batch_get_map_host": (C.c_int, [_vp, C.c_int, _vp]),
     "eb_collision_check_batch_host": (C.c_int, [_vp, C.POINTER(EbCollision), _vp, C.c_int, _vp]),
     "eb_collision_check_batch_dev": (C.c_int, [_vp, C.POINTER(EbCollision), _vp, C.c_int, _vp]),
     "eb_validate_control_batch_host": (C.c_int, [_vp, C.POINTER(EbCollision), _vp, _vp, C.c_int, C.c_double, C.c_double,

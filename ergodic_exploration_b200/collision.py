@@ -16,7 +16,7 @@ import numpy as np
 
 from . import capi
 from .capi import EbCollision, EbDwa, check
-from .controller import map_batch_args
+from .controller import map_batch_args, row_args, update_arg
 
 try:
     import torch
@@ -237,6 +237,7 @@ class GridMapBatch:
         h = C.c_void_p()
         check(self._lib.eb_grid_batch_create(device, self.batch, C.byref(h)))
         self._h = h
+        self._shape = [None] * self.batch  # (ysize, xsize) of each map that has been set
 
     def set(self, cells, resolution, origin, update=None) -> None:
         """The maps of the flagged instances, with the arguments of ErgodicControl.setMapTargets: ``cells`` B int8
@@ -250,6 +251,59 @@ class GridMapBatch:
             raise ValueError(self._lib.eb_last_error().decode())
         check(st)
         del keep
+        for i, c in enumerate(cells):
+            if update is None or update[i]:
+                self._shape[i] = tuple(int(v) for v in c.shape)
+
+    def set_rows(self, rows, row_begin, update=None) -> None:
+        """Rows [row_begin[i], row_begin[i] + n_i) of map i of every flagged instance <- ``rows[i]``, an (n_i, xsize_i)
+        int8 array (all numpy: host path; all CUDA tensors: device path on torch's current stream, the tensors must
+        stay alive until the copy has run) or None (nothing written).  Shapes, resolutions and origins do not change;
+        the map must have been set.  One kernel launch.  Pass the same row_begin and each band's n_i as row_count to
+        ErgodicControl.setMapTargets(grids, row_begin, row_count) to recompute only the changed rows' targets."""
+        B = self.batch
+        if len(rows) != B:
+            raise ValueError(f"GridMapBatch.set_rows needs {B} bands, got {len(rows)}")
+        rb = row_args(B, row_begin, "row_begin")
+        upd = update_arg(B, update)
+        present = [r for r in rows if r is not None]
+        dev = bool(present) and _is_cuda(present[0])
+        if any(_is_cuda(r) != dev for r in present):
+            raise ValueError("GridMapBatch.set_rows: rows must be all numpy arrays or all CUDA tensors")
+        rc = np.zeros(B, dtype=np.uint32)
+        ptrs = (C.c_void_p * B)()
+        keep = []
+        for i, r in enumerate(rows):
+            if r is None or (upd is not None and not upd[i]):
+                continue
+            if self._shape[i] is None:
+                raise ValueError(f"GridMapBatch.set_rows: instance {i} has no map")
+            if r.ndim != 2 or r.shape[1] != self._shape[i][1]:
+                raise ValueError(f"GridMapBatch.set_rows: rows[{i}] must be (n, {self._shape[i][1]}), got {tuple(r.shape)}")
+            if dev:
+                if r.dtype != torch.int8 or not r.is_contiguous():
+                    raise ValueError(f"GridMapBatch.set_rows: rows[{i}] must be a contiguous int8 tensor")
+                ptrs[i] = r.data_ptr()
+            else:
+                r = np.ascontiguousarray(r)
+                if r.dtype != np.int8:
+                    raise ValueError(f"GridMapBatch.set_rows: rows[{i}] must be int8, got {r.dtype}")
+                keep.append(r)
+                ptrs[i] = r.ctypes.data
+            rc[i] = r.shape[0]
+        self._stream()
+        fn = self._lib.eb_grid_batch_set_rows_dev if dev else self._lib.eb_grid_batch_set_rows_host
+        self._raise(fn(self._h, C.addressof(ptrs), rb.ctypes.data, rc.ctypes.data,
+                       upd.ctypes.data if upd is not None else None))
+        del keep
+
+    def get_map(self, i: int) -> np.ndarray:
+        """map i as held on the device, a (ysize_i, xsize_i) int8 numpy array (synchronises)"""
+        if not 0 <= i < self.batch or self._shape[i] is None:
+            raise ValueError(f"GridMapBatch.get_map: instance {i} has no map")
+        out = np.empty(self._shape[i], dtype=np.int8)
+        self._raise(self._lib.eb_grid_batch_get_map_host(self._h, int(i), out.ctypes.data))
+        return out
 
     def launch_count(self) -> int:
         return int(self._lib.eb_grid_batch_launch_count(self._h))

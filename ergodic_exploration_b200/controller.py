@@ -231,6 +231,24 @@ def map_batch_args(B: int, cells, resolution, origin, update, name: str):
     return dev, args, keep
 
 
+def row_args(B: int, a, name: str) -> np.ndarray:
+    """row_begin / row_count of the row-band calls as a (B,) uint32 host array"""
+    a = np.asarray(a.cpu().numpy() if _is_cuda_tensor(a) else a)
+    if a.shape != (B,) or (a.size and (not np.issubdtype(a.dtype, np.integer) or a.min() < 0 or a.max() > 0xFFFFFFFF)):
+        raise ValueError(f"{name} must be ({B},) non-negative integers, got shape {a.shape}, dtype {a.dtype}")
+    return np.ascontiguousarray(a, dtype=np.uint32)
+
+
+def update_arg(B: int, update):
+    """update of the batched map calls as a (B,) int32 host array, or None (all)"""
+    if update is None:
+        return None
+    upd = np.ascontiguousarray(update)
+    if upd.shape != (B,):
+        raise ValueError(f"update must be ({B},), got {upd.shape}")
+    return upd.astype(np.int32)
+
+
 class ErgodicControl:
     """Batched drop-in for ErgodicControl<ModelT> (ergodic_control.hpp:72-185)."""
 
@@ -420,20 +438,57 @@ class ErgodicControl:
         assert extent.dtype == torch.float64 and extent.is_contiguous() and extent.numel() == 2 * self.batch
         check(self._lib.eb_set_phik_batch_dev(self._h, C.c_void_p(phik.data_ptr()), C.c_void_p(extent.data_ptr())))
 
-    def setMapTargets(self, cells, resolution, origin, update=None) -> None:
+    def setMapTargets(self, cells, resolution=None, origin=None, update=None, *, row_begin=None,
+                      row_count=None) -> None:
         """Map-derived (entropy) target and map frame per instance, one kernel launch for the batch.
+
+        ``cells`` may be a GridMapBatch of the same B on the same device: setMapTargets(grids, row_begin=None,
+        row_count=None, update=None) (positionally, the second and third arguments are then row_begin and row_count)
+        derives every flagged instance from map i of the batch, without uploading the cells again, bit for bit what
+        the call with map i's cells, resolution and origin gives.  row_begin / row_count (B,) declare the rows of map i
+        that changed (GridMapBatch.set_rows) since this controller last derived instance i from this batch; only the
+        64-row units that meet them are recomputed.  None: whole maps.  Runs on torch's current stream when CUDA is
+        available, after the work enqueued on the grid batch, without a host synchronisation.
 
         ``cells``: B int8 occupancy grids (ysize_i, xsize_i) in GridMap layout, all numpy (host path) or all CUDA
         tensors (device path, torch's current stream); the entry of an instance that is not updated may be None.
         ``resolution``: scalar or (B,); ``origin``: (B, 2) GridMap xmin / ymin; ``update``: (B,) bool or None (all).
         Instance i gets the row MapTarget(xsize_i, ysize_i, resolution_i, nb).execute(cells_i) and the frame
         origin_i, (xsize_i * res_i, ysize_i * res_i); control(None) or control(bounds of the maps) then uses them."""
+        from .collision import GridMapBatch
+
+        if isinstance(cells, GridMapBatch):
+            if resolution is not None or origin is not None:
+                if row_begin is not None or row_count is not None:
+                    raise TypeError("setMapTargets(grids, ...): row_begin / row_count given twice")
+                row_begin, row_count = resolution, origin
+            return self._map_targets_from_grids(cells, row_begin, row_count, update)
+        if resolution is None or origin is None:
+            raise TypeError("setMapTargets(cells, resolution, origin, update=None) needs resolution and origin")
         dev, args, keep = map_batch_args(self.batch, cells, resolution, origin, update, "setMapTargets")
         if dev:
             self._sync_stream()
             st = self._lib.eb_set_map_targets_batch_dev(self._h, *args)
         else:
             st = self._lib.eb_set_map_targets_batch_host(self._h, *args)
+        if st == capi.EB_ERR_INVALID_ARGUMENT:
+            raise ValueError(self._lib.eb_last_error().decode())
+        check(st)
+
+    def _map_targets_from_grids(self, grids, row_begin, row_count, update):
+        B = self.batch
+        if grids.batch != B:
+            raise ValueError(f"setMapTargets: the grid batch holds {grids.batch} maps for {B} instances")
+        if (row_begin is None) != (row_count is None):
+            raise ValueError("setMapTargets: row_begin and row_count must both be given or both be None")
+        rb = row_args(B, row_begin, "row_begin") if row_begin is not None else None
+        rc = row_args(B, row_count, "row_count") if row_count is not None else None
+        upd = update_arg(B, update)
+        self._sync_stream()
+        grids._stream()
+        st = self._lib.eb_set_map_targets_from_grid_batch(
+            self._h, grids._h, rb.ctypes.data if rb is not None else None, rc.ctypes.data if rc is not None else None,
+            upd.ctypes.data if upd is not None else None)
         if st == capi.EB_ERR_INVALID_ARGUMENT:
             raise ValueError(self._lib.eb_last_error().decode())
         check(st)

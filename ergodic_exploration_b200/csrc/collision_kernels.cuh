@@ -230,6 +230,28 @@ __global__ void __launch_bounds__(256) map_copy_kernel(const MapCopy* __restrict
   if (threadIdx.x == 0) views[m.inst] = m.view;
 }
 
+// eb_grid_batch_set_rows_*: one CTA per band of whole rows, a contiguous byte range of the map's slot; the map's
+// record does not change
+struct BandCopy
+{
+  const signed char* src;
+  signed char* dst;
+  size_t bytes;
+};
+
+__global__ void __launch_bounds__(256) band_copy_kernel(const BandCopy* __restrict__ bands)
+{
+  const BandCopy b = bands[blockIdx.x];
+  size_t k = threadIdx.x;
+  if (((reinterpret_cast<uintptr_t>(b.src) | reinterpret_cast<uintptr_t>(b.dst)) & 15) == 0)
+  {
+    for (; k < b.bytes / 16; k += blockDim.x)
+      reinterpret_cast<uint4*>(b.dst)[k] = __ldg(reinterpret_cast<const uint4*>(b.src) + k);
+    k = b.bytes / 16 * 16 + threadIdx.x;
+  }
+  for (; k < b.bytes; k += blockDim.x) b.dst[k] = b.src[k];
+}
+
 // fraction of occupied cells, to pick between the two builders
 __global__ void __launch_bounds__(256) count_occupied_kernel(const GridView g, double thr, unsigned long long* count)
 {

@@ -11,6 +11,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <atomic>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -594,6 +595,19 @@ struct eb_controller
   signed char* d_mb_cells = nullptr;
   size_t mb_cells_bytes = 0;
   int mb_grid = 0;                        // resident CTAs of map_target_batch_kernel on the device
+  // kept blocks of eb_set_map_targets_from_grid_batch: instance i's raw block of unit v of its map is slot
+  // kb_slot0[i] + v of d_kb (kb_cap[i] slots reserved); kb_key[i] says which map the blocks belong to
+  struct KeptKey
+  {
+    unsigned long long grid = 0, map = 0;  // grid batch serial (0: no kept blocks), map serial in it
+    unsigned nx = 0, ny = 0;
+    double res = 0.0;
+  };
+  double* d_kb = nullptr;
+  std::vector<int> kb_slot0, kb_cap;
+  std::vector<KeptKey> kb_key;
+  eb::MapKept* h_mb_kept = nullptr;  // [B] pinned: the recomputed units of a call
+  eb::MapKept* d_mb_kept = nullptr;
   // safe control tick (eb_control_safe_batch_*, safe_control.cuh)
   int* d_safe_list = nullptr;      // [1 + B]: the count of failing robots, then their indices
   int* d_safe_branch = nullptr;    // [B] staging of the _host call
@@ -1057,6 +1071,9 @@ void eb_destroy(eb_controller* c)
   cudaFree(c->d_mb_desc);
   if (c->mb_staged) cudaEventDestroy(c->mb_staged);
   cudaFree(c->d_mb_slots);
+  cudaFreeHost(c->h_mb_kept);
+  cudaFree(c->d_mb_kept);
+  cudaFree(c->d_kb);
   cudaFree(c->d_mb_arrive);
   cudaFreeHost(c->h_mb_cells);
   cudaFree(c->d_mb_cells);
@@ -2638,6 +2655,11 @@ struct eb_grid_batch
   // stream after it (ticked); the next set call waits for the last tick before it writes or frees an arena
   cudaEvent_t maps_ready = nullptr;
   cudaEvent_t ticked = nullptr;
+  // eb_set_map_targets_from_grid_batch: this handle (unique per process) and, per map, how often a set call replaced it
+  unsigned long long serial = 0;
+  std::vector<unsigned long long> map_serial;
+  eb::BandCopy* h_bands = nullptr;  // eb_grid_batch_set_rows_*: pinned band records, uploaded like h_copies
+  eb::BandCopy* d_bands = nullptr;
   signed char* h_cells = nullptr;
   signed char* d_cells = nullptr;
   size_t cells_bytes = 0;
@@ -2737,7 +2759,11 @@ eb_status grid_batch_set(eb_grid_batch* g, const signed char* const* cells, cons
     g->d_arena = arena;
     g->slot = slot;
   }
-  for (int i = 0; i < B; i++) g->unmapped -= (!g->views[i].data && views[i].data) ? 1 : 0;
+  for (int i = 0; i < B; i++)
+  {
+    g->unmapped -= (!g->views[i].data && views[i].data) ? 1 : 0;
+    g->map_serial[i] += (update && !update[i]) ? 0 : 1;  // kept target blocks of the old map are stale
+  }
   g->views = views;
   return EB_OK;
 }
@@ -2815,6 +2841,9 @@ eb_status eb_grid_batch_create(int device, int batch, eb_grid_batch** out)
   g->B = batch;
   g->views.assign((size_t)batch, eb::GridView{});
   g->slot.assign((size_t)batch, 0);
+  g->map_serial.assign((size_t)batch, 0);
+  static std::atomic<unsigned long long> next_serial{ 0 };
+  g->serial = ++next_serial;
   g->unmapped = batch;
   *out = g;
   return EB_OK;
@@ -2831,6 +2860,8 @@ void eb_grid_batch_destroy(eb_grid_batch* g)
   cudaFree(g->d_retired);
   cudaFreeHost(g->h_copies);
   cudaFree(g->d_copies);
+  cudaFreeHost(g->h_bands);
+  cudaFree(g->d_bands);
   cudaFreeHost(g->h_cells);
   cudaFree(g->d_cells);
   cudaFree(g->d_a);
@@ -2906,6 +2937,133 @@ eb_status eb_grid_batch_set_maps_host(eb_grid_batch* g, const signed char* const
   EB_CUDA(cudaMemcpyAsync(g->d_cells, g->h_cells, total, cudaMemcpyHostToDevice, g->stream));
   st = grid_batch_set(g, dptr.data(), xsize, ysize, resolution, origin, update, n);
   if (st != EB_OK) return st;
+  EB_CUDA(cudaStreamSynchronize(g->stream));
+  return EB_OK;
+}
+
+}  // extern "C"
+
+namespace
+{
+// the rules of eb_grid_batch_set_rows_*; *n = bands with rows to write
+eb_status grid_batch_check_rows(const eb_grid_batch* g, const signed char* const* rows, const unsigned* row_begin,
+                                const unsigned* row_count, const int* update, const char* call, int* n)
+{
+  *n = 0;
+  if (!g || !rows || !row_begin || !row_count) return fail(EB_ERR_INVALID_ARGUMENT, std::string(call) + ": NULL argument");
+  for (int i = 0; i < g->B; i++)
+  {
+    if (update && !update[i]) continue;
+    const eb::GridView& v = g->views[i];
+    if (!v.data) return fail(EB_ERR_INVALID_ARGUMENT, std::string(call) + ": instance " + std::to_string(i) + " has no map");
+    if ((unsigned long long)row_begin[i] + row_count[i] > v.ysize)
+      return fail(EB_ERR_INVALID_ARGUMENT, std::string(call) + ": rows [" + std::to_string(row_begin[i]) + ", +" +
+                                               std::to_string(row_count[i]) + ") of map " + std::to_string(i) +
+                                               " pass its " + std::to_string(v.ysize) + " rows");
+    if (row_count[i] == 0) continue;
+    if (!rows[i]) return fail(EB_ERR_INVALID_ARGUMENT, std::string(call) + ": rows of map " + std::to_string(i) + " is NULL");
+    (*n)++;
+  }
+  return EB_OK;
+}
+
+// writes the bands (device pointers) into the arena with one band_copy_kernel launch
+eb_status grid_batch_set_rows(eb_grid_batch* g, const signed char* const* rows, const unsigned* row_begin,
+                              const unsigned* row_count, const int* update, int n)
+{
+  if (n == 0) return EB_OK;
+  EB_CUDA(cudaSetDevice(g->device));
+  if (!g->h_bands)
+  {
+    EB_CUDA(cudaHostAlloc(&g->h_bands, sizeof(eb::BandCopy) * (size_t)g->B, cudaHostAllocDefault));
+    EB_CUDA(cudaMalloc(&g->d_bands, sizeof(eb::BandCopy) * (size_t)g->B));
+  }
+  EB_CUDA(cudaEventSynchronize(g->staged));  // the previous upload out of the pinned records is done
+  int k = 0;
+  for (int i = 0; i < g->B; i++)
+  {
+    if ((update && !update[i]) || row_count[i] == 0) continue;
+    const eb::GridView& v = g->views[i];
+    signed char* dst = const_cast<signed char*>(v.data) + (size_t)row_begin[i] * v.xsize;
+    g->h_bands[k++] = eb::BandCopy{ rows[i], dst, (size_t)row_count[i] * v.xsize };
+  }
+  // the records go up before the wait for the last tick, so the next call's wait on `staged` does not wait for it
+  EB_CUDA(cudaMemcpyAsync(g->d_bands, g->h_bands, sizeof(eb::BandCopy) * (size_t)k, cudaMemcpyHostToDevice, g->stream));
+  EB_CUDA(cudaEventRecord(g->staged, g->stream));
+  if (g->ticked) EB_CUDA(cudaStreamWaitEvent(g->stream, g->ticked, 0));  // a tick or target call may still read the maps
+  eb::band_copy_kernel<<<k, 256, 0, g->stream>>>(g->d_bands);
+  EB_CUDA(cudaGetLastError());
+  g->launches += 1;
+  return EB_OK;
+}
+}  // namespace
+
+extern "C" {
+
+eb_status eb_grid_batch_set_rows_dev(eb_grid_batch* g, const signed char* const* rows_dev, const unsigned* row_begin,
+                                     const unsigned* row_count, const int* update)
+{
+  EB_TRACE("eb_grid_batch_set_rows_dev");
+  int n = 0;
+  const eb_status st = grid_batch_check_rows(g, rows_dev, row_begin, row_count, update, "eb_grid_batch_set_rows_dev", &n);
+  if (st != EB_OK) return st;
+  return grid_batch_set_rows(g, rows_dev, row_begin, row_count, update, n);
+}
+
+eb_status eb_grid_batch_set_rows_host(eb_grid_batch* g, const signed char* const* rows, const unsigned* row_begin,
+                                      const unsigned* row_count, const int* update)
+{
+  EB_TRACE("eb_grid_batch_set_rows_host");
+  int n = 0;
+  eb_status st = grid_batch_check_rows(g, rows, row_begin, row_count, update, "eb_grid_batch_set_rows_host", &n);
+  if (st != EB_OK || n == 0) return st;
+  // the bands are packed into the set call's pinned buffer (16-byte aligned offsets) and copied with one
+  // cudaMemcpyAsync
+  std::vector<size_t> off((size_t)g->B, 0);
+  size_t total = 0;
+  for (int i = 0; i < g->B; i++)
+  {
+    if ((update && !update[i]) || row_count[i] == 0) continue;
+    off[i] = total;
+    total += ((size_t)row_count[i] * g->views[i].xsize + 15) & ~(size_t)15;
+  }
+  EB_CUDA(cudaSetDevice(g->device));
+  EB_CUDA(cudaStreamSynchronize(g->stream));  // no earlier copy still reads the staging buffers
+  if (total > g->cells_bytes)
+  {
+    cudaFreeHost(g->h_cells);
+    cudaFree(g->d_cells);
+    g->h_cells = nullptr;
+    g->d_cells = nullptr;
+    g->cells_bytes = 0;
+    EB_CUDA(cudaHostAlloc(&g->h_cells, total, cudaHostAllocDefault));
+    EB_CUDA(cudaMalloc(&g->d_cells, total));
+    g->cells_bytes = total;
+  }
+  std::vector<const signed char*> dptr((size_t)g->B, nullptr);
+  for (int i = 0; i < g->B; i++)
+    if (!(update && !update[i]) && row_count[i] > 0)
+    {
+      std::memcpy(g->h_cells + off[i], rows[i], (size_t)row_count[i] * g->views[i].xsize);
+      dptr[i] = g->d_cells + off[i];
+    }
+  EB_CUDA(cudaMemcpyAsync(g->d_cells, g->h_cells, total, cudaMemcpyHostToDevice, g->stream));
+  st = grid_batch_set_rows(g, dptr.data(), row_begin, row_count, update, n);
+  if (st != EB_OK) return st;
+  EB_CUDA(cudaStreamSynchronize(g->stream));
+  return EB_OK;
+}
+
+eb_status eb_grid_batch_get_map_host(const eb_grid_batch* g, int i, signed char* cells)
+{
+  if (!g || !cells) return fail(EB_ERR_INVALID_ARGUMENT, "eb_grid_batch_get_map_host: NULL argument");
+  if (i < 0 || i >= g->B)
+    return fail(EB_ERR_INVALID_ARGUMENT, "eb_grid_batch_get_map_host: instance " + std::to_string(i) + " is not in [0, " +
+                                             std::to_string(g->B) + ")");
+  const eb::GridView& v = g->views[(size_t)i];
+  if (!v.data) return fail(EB_ERR_INVALID_ARGUMENT, "eb_grid_batch_get_map_host: instance " + std::to_string(i) + " has no map");
+  EB_CUDA(cudaSetDevice(g->device));
+  EB_CUDA(cudaMemcpyAsync(cells, v.data, (size_t)v.xsize * v.ysize, cudaMemcpyDeviceToHost, g->stream));
   EB_CUDA(cudaStreamSynchronize(g->stream));
   return EB_OK;
 }
@@ -3496,6 +3654,26 @@ eb_status map_targets_check(const eb_controller* c, const signed char* const* ce
   return EB_OK;
 }
 
+// the descriptors, arrival counters and resident grid of map_target_batch_kernel, allocated at the first call
+eb_status ensure_map_batch(eb_controller* c)
+{
+  if (c->h_mb_desc) return EB_OK;
+  const int B = c->B;
+  EB_CUDA(cudaHostAlloc(&c->h_mb_desc, sizeof(eb::MapBatchDesc) * (size_t)B, cudaHostAllocDefault));
+  EB_CUDA(cudaMalloc(&c->d_mb_desc, sizeof(eb::MapBatchDesc) * (size_t)B));
+  EB_CUDA(cudaMalloc(&c->d_mb_arrive, sizeof(unsigned) * (size_t)B));
+  EB_CUDA(cudaMemset(c->d_mb_arrive, 0, sizeof(unsigned) * (size_t)B));
+  EB_CUDA(cudaEventCreateWithFlags(&c->mb_staged, cudaEventDisableTiming));
+  for (auto kernel : { eb::map_target_batch_kernel<false>, eb::map_target_batch_kernel<true> })
+    EB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)eb::kMbSmemBytes));
+  int per_sm = 0, sms = 0;
+  EB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, eb::map_target_batch_kernel<false>, eb::kMbThreads,
+                                                        eb::kMbSmemBytes));
+  EB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->cfg.device));
+  c->mb_grid = std::max(1, per_sm * sms);
+  return EB_OK;
+}
+
 // map-derived targets of the flagged instances (map_target_batch.cuh); cells holds device pointers
 eb_status map_targets_batch(eb_controller* c, const signed char* const* cells, const unsigned* xsize,
                             const unsigned* ysize, const double* resolution, const double* origin, const int* update,
@@ -3511,21 +3689,7 @@ eb_status map_targets_batch(eb_controller* c, const signed char* const* cells, c
   if (st != EB_OK) return st;
   if (n == B) c->frames_set = true;
   if (n == 0) return EB_OK;
-  if (!c->h_mb_desc)
-  {
-    EB_CUDA(cudaHostAlloc(&c->h_mb_desc, sizeof(eb::MapBatchDesc) * (size_t)B, cudaHostAllocDefault));
-    EB_CUDA(cudaMalloc(&c->d_mb_desc, sizeof(eb::MapBatchDesc) * (size_t)B));
-    EB_CUDA(cudaMalloc(&c->d_mb_arrive, sizeof(unsigned) * (size_t)B));
-    EB_CUDA(cudaMemset(c->d_mb_arrive, 0, sizeof(unsigned) * (size_t)B));
-    EB_CUDA(cudaEventCreateWithFlags(&c->mb_staged, cudaEventDisableTiming));
-    EB_CUDA(cudaFuncSetAttribute(eb::map_target_batch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 (int)eb::kMbSmemBytes));
-    int per_sm = 0, sms = 0;
-    EB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, eb::map_target_batch_kernel, eb::kMbThreads,
-                                                          eb::kMbSmemBytes));
-    EB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->cfg.device));
-    c->mb_grid = std::max(1, per_sm * sms);
-  }
+  if ((st = ensure_map_batch(c)) != EB_OK) return st;
   if (units > c->mb_slot_units)
   {
     cudaFree(c->d_mb_slots);  // synchronises with earlier launches that use it
@@ -3567,7 +3731,7 @@ eb_status map_targets_batch(eb_controller* c, const signed char* const* cells, c
   p.mem_count = c->d_hist_cos ? c->mem_count : 0;
   p.B = B;
   const int grid = (int)std::min<long long>(units, c->mb_grid);
-  eb::map_target_batch_kernel<<<grid, eb::kMbThreads, eb::kMbSmemBytes, c->stream>>>(p);
+  eb::map_target_batch_kernel<false><<<grid, eb::kMbThreads, eb::kMbSmemBytes, c->stream>>>(p);
   EB_CUDA(cudaGetLastError());
   c->launches += 1;
   return EB_OK;
@@ -3631,6 +3795,183 @@ eb_status eb_set_map_targets_batch_host(eb_controller* c, const signed char* con
   st = map_targets_batch(c, dptr.data(), xsize, ysize, resolution, origin, update, call);
   if (st != EB_OK) return st;
   EB_CUDA(cudaStreamSynchronize(c->stream));
+  return EB_OK;
+}
+
+}  // extern "C"
+
+namespace
+{
+// moves the kept blocks to a new region in which instance i has cap[i] slots; the blocks of the instances whose slot
+// keeps its size move with them (one copy per run of such instances), the others are recomputed whole by the caller
+eb_status kept_relayout(eb_controller* c, const std::vector<int>& cap)
+{
+  const int B = c->B;
+  const size_t K = (size_t)c->K;
+  std::vector<int> slot0((size_t)B, 0);
+  long long total = 0;
+  for (int i = 0; i < B; i++)
+  {
+    slot0[i] = (int)total;
+    total += cap[i];
+  }
+  if (total > 0x7fffffffLL) return fail(EB_ERR_INVALID_ARGUMENT, "eb_set_map_targets_from_grid_batch: more than 2^31 - 1 units");
+  double* kb = nullptr;
+  EB_CUDA(cudaMalloc(&kb, sizeof(double) * K * (size_t)total));
+  cudaError_t e = cudaSuccess;
+  bool copied = false;
+  for (int i = 0; i < B && e == cudaSuccess;)
+  {
+    if (cap[i] != c->kb_cap[i] || c->kb_cap[i] == 0)
+    {
+      i++;
+      continue;
+    }
+    int j = i, units = 0;
+    for (; j < B && cap[j] == c->kb_cap[j]; j++) units += cap[j];
+    e = cudaMemcpyAsync(kb + K * slot0[i], c->d_kb + K * c->kb_slot0[i], sizeof(double) * K * units,
+                        cudaMemcpyDeviceToDevice, c->stream);
+    copied = true;
+    i = j;
+  }
+  if (e == cudaSuccess && copied) e = cudaStreamSynchronize(c->stream);  // the old region is read no more
+  if (e != cudaSuccess)
+  {
+    cudaFree(kb);
+    return fail(EB_ERR_CUDA, std::string("eb_set_map_targets_from_grid_batch: ") + cudaGetErrorString(e));
+  }
+  cudaFree(c->d_kb);
+  c->d_kb = kb;
+  for (int i = 0; i < B; i++)
+    if (cap[i] != c->kb_cap[i]) c->kb_key[i] = eb_controller::KeptKey{};
+  c->kb_cap = cap;
+  c->kb_slot0 = slot0;
+  return EB_OK;
+}
+}  // namespace
+
+extern "C" {
+
+eb_status eb_set_map_targets_from_grid_batch(eb_controller* c, eb_grid_batch* g, const unsigned* row_begin,
+                                             const unsigned* row_count, const int* update)
+{
+  EB_TRACE("eb_set_map_targets_from_grid_batch");
+  static const char* call = "eb_set_map_targets_from_grid_batch";
+  if (!c || !g) return fail(EB_ERR_INVALID_ARGUMENT, std::string(call) + ": NULL argument");
+  if (!row_begin != !row_count)
+    return fail(EB_ERR_INVALID_ARGUMENT, std::string(call) + ": row_begin and row_count must both be given or both NULL");
+  if (g->B != c->B)
+    return fail(EB_ERR_INVALID_ARGUMENT, std::string(call) + ": the grid batch holds " + std::to_string(g->B) +
+                                             " maps for " + std::to_string(c->B) + " instances");
+  if (g->device != c->cfg.device)
+    return fail(EB_ERR_INVALID_ARGUMENT, std::string(call) + ": the grid batch and the controller are on different devices");
+  const int B = c->B;
+  if (c->kb_key.empty())
+  {
+    c->kb_key.assign((size_t)B, eb_controller::KeptKey{});
+    c->kb_cap.assign((size_t)B, 0);
+    c->kb_slot0.assign((size_t)B, 0);
+  }
+  // the run of units each flagged instance recomputes: the units that meet its declared rows, or all of them
+  std::vector<eb::MapKept> run((size_t)B, eb::MapKept{ 0, 0, 0 });
+  std::vector<int> cap = c->kb_cap;
+  int n = 0;
+  long long work = 0;
+  bool grown = false;
+  for (int i = 0; i < B; i++)
+  {
+    if (update && !update[i]) continue;
+    const eb::GridView& v = g->views[i];
+    if (!v.data) return fail(EB_ERR_INVALID_ARGUMENT, std::string(call) + ": instance " + std::to_string(i) + " has no map");
+    if (row_begin && (unsigned long long)row_begin[i] + row_count[i] > v.ysize)
+      return fail(EB_ERR_INVALID_ARGUMENT, std::string(call) + ": rows [" + std::to_string(row_begin[i]) + ", +" +
+                                               std::to_string(row_count[i]) + ") of map " + std::to_string(i) +
+                                               " pass its " + std::to_string(v.ysize) + " rows");
+    n++;
+    const int units = eb::mb_units((int)v.ysize);
+    const eb_controller::KeptKey& k = c->kb_key[i];
+    const bool whole = !row_begin || k.grid != g->serial || k.map != g->map_serial[i] || k.nx != v.xsize ||
+                       k.ny != v.ysize || k.res != v.resolution || units > c->kb_cap[i];
+    if (whole)
+      run[i] = eb::MapKept{ 0, units, 0 };
+    else if (row_count[i] > 0)
+    {
+      const int first = (int)(row_begin[i] / eb::kMbRows), last = (int)((row_begin[i] + row_count[i] - 1) / eb::kMbRows);
+      run[i] = eb::MapKept{ first, last - first + 1, 0 };
+    }
+    work += run[i].count;
+    if (units > cap[i])
+    {
+      cap[i] = units + units / 4;  // a quarter of headroom, as the grid batch's arena
+      grown = true;
+    }
+  }
+  EB_CUDA(cudaSetDevice(c->cfg.device));
+  eb_status st = ensure_per_inst(c);
+  if (st != EB_OK) return st;
+  if (n == B) c->frames_set = true;
+  if (work == 0) return EB_OK;
+  if (work > 0x7fffffffLL) return fail(EB_ERR_INVALID_ARGUMENT, std::string(call) + ": more than 2^31 - 1 units");
+  if ((st = ensure_map_batch(c)) != EB_OK) return st;
+  if (!c->h_mb_kept)
+  {
+    EB_CUDA(cudaHostAlloc(&c->h_mb_kept, sizeof(eb::MapKept) * (size_t)B, cudaHostAllocDefault));
+    EB_CUDA(cudaMalloc(&c->d_mb_kept, sizeof(eb::MapKept) * (size_t)B));
+  }
+  if (grown && (st = kept_relayout(c, cap)) != EB_OK) return st;
+  if (!g->maps_ready)
+  {
+    EB_CUDA(cudaEventCreateWithFlags(&g->maps_ready, cudaEventDisableTiming));
+    EB_CUDA(cudaEventCreateWithFlags(&g->ticked, cudaEventDisableTiming));
+  }
+  EB_CUDA(cudaEventSynchronize(c->mb_staged));  // the previous call's copy out of the pinned descriptors is done
+  int k = 0, u0 = 0;
+  for (int i = 0; i < B; i++)
+  {
+    if (run[i].count == 0) continue;
+    const eb::GridView& v = g->views[i];
+    c->h_mb_desc[k] = eb::MapBatchDesc{ v.data, (int)v.xsize, (int)v.ysize, v.resolution, v.xmin, v.ymin, i, u0 };
+    c->h_mb_kept[k++] = eb::MapKept{ run[i].first, run[i].count, c->kb_slot0[i] };
+    u0 += run[i].count;
+  }
+  EB_CUDA(cudaMemcpyAsync(c->d_mb_desc, c->h_mb_desc, sizeof(eb::MapBatchDesc) * (size_t)k, cudaMemcpyHostToDevice,
+                          c->stream));
+  EB_CUDA(cudaMemcpyAsync(c->d_mb_kept, c->h_mb_kept, sizeof(eb::MapKept) * (size_t)k, cudaMemcpyHostToDevice,
+                          c->stream));
+  EB_CUDA(cudaEventRecord(c->mb_staged, c->stream));  // before the wait below: the next call's sync does not wait for it
+  // after the set and rows calls already enqueued on the grid batch's stream, without a host synchronisation
+  EB_CUDA(cudaEventRecord(g->maps_ready, g->stream));
+  EB_CUDA(cudaStreamWaitEvent(c->stream, g->maps_ready, 0));
+  eb::MapBatchParams p{};
+  p.desc = c->d_mb_desc;
+  p.n = k;
+  p.units = (int)work;
+  p.nb = c->nb;
+  p.slots = c->d_kb;
+  p.arrive = c->d_mb_arrive;
+  p.frames = c->d_frames;
+  p.phik = c->d_phik_b;
+  p.hist = c->d_hist;
+  p.hist_cos = c->d_hist_cos;
+  p.mem_count = c->d_hist_cos ? c->mem_count : 0;
+  p.B = B;
+  p.kept = c->d_mb_kept;
+  const int grid = (int)std::min<long long>(work, c->mb_grid);
+  eb::map_target_batch_kernel<true><<<grid, eb::kMbThreads, eb::kMbSmemBytes, c->stream>>>(p);
+  cudaError_t e = cudaGetLastError();
+  const cudaError_t r = cudaEventRecord(g->ticked, c->stream);  // the grid batch's next set or rows call waits for this
+  if (e == cudaSuccess) e = r;
+  if (e != cudaSuccess)
+  {
+    for (int i = 0; i < B; i++)
+      if (run[i].count > 0) c->kb_key[i] = eb_controller::KeptKey{};
+    return fail(EB_ERR_CUDA, std::string(call) + ": " + cudaGetErrorString(e));
+  }
+  c->launches += 1;
+  for (int i = 0; i < B; i++)
+    if (run[i].count > 0)
+      c->kb_key[i] = eb_controller::KeptKey{ g->serial, g->map_serial[i], g->views[i].xsize, g->views[i].ysize,
+                                             g->views[i].resolution };
   return EB_OK;
 }
 

@@ -18,6 +18,12 @@
 // result does not depend on which unit finished last, or on the other maps of the batch), divides by raw[0], writes
 // the row and the frame record with target_batch_kernel's expressions, and re-derives the instance's replay cosines
 // when its frame key moved.  num_basis > 32 loops over blocks of 32 orders, as elsewhere.
+//
+// KEPT (eb_set_map_targets_from_grid_batch): the slots are the controller's kept blocks, one region of consecutive
+// units per instance that outlives the launch.  The work list holds only the units to recompute (MapKept: one non-empty
+// run of consecutive units per listed map); the arrival count of an instance is the length of its run, and its last
+// unit sums all of the instance's kept blocks in unit order.  A unit's block depends only on its cells and on nx, ny
+// and res, so the row equals the one of a launch over every unit of the map, bit for bit.
 #pragma once
 
 #include "common.cuh"
@@ -43,6 +49,13 @@ struct MapBatchDesc
   int unit0;                 // first work unit of this map
 };
 
+// KEPT: map desc[j] recomputes units [first, first + count) of its map (work items [desc[j].unit0, + count)); its
+// kept blocks are slots [slot0, slot0 + units of the map)
+struct MapKept
+{
+  int first, count, slot0;
+};
+
 struct MapBatchParams
 {
   const MapBatchDesc* desc;  // [n] maps to update, unit0 ascending
@@ -55,6 +68,7 @@ struct MapBatchParams
   double* hist_cos;          // [mem_count][B][2] or null
   long long mem_count;
   int B;
+  const MapKept* kept;       // KEPT: [n] the recomputed units of each map and where its kept blocks live
 };
 
 __host__ __device__ inline int mb_units(int ny) { return (ny + kMbRows - 1) / kMbRows; }
@@ -69,6 +83,7 @@ __device__ __forceinline__ double mb_entropy(int b)
   return -p * log(p) - (1.0 - p) * log(1.0 - p);
 }
 
+template <bool KEPT>
 __global__ void __launch_bounds__(kMbThreads, 3) map_target_batch_kernel(const MapBatchParams p)
 {
   extern __shared__ __align__(16) double mb_smem[];
@@ -94,10 +109,17 @@ __global__ void __launch_bounds__(kMbThreads, 3) map_target_batch_kernel(const M
       else hi = mid - 1;
     }
     const MapBatchDesc d = p.desc[lo];
-    const int r0 = (u - d.unit0) * kMbRows, nrows = min(kMbRows, d.ny - r0), nx = d.nx;
+    int mu = u - d.unit0, su = u;  // unit of the map, slot of the unit
+    if constexpr (KEPT)
+    {
+      const MapKept k = p.kept[lo];
+      mu += k.first;
+      su = k.slot0 + mu;
+    }
+    const int r0 = mu * kMbRows, nrows = min(kMbRows, d.ny - r0), nx = d.nx;
     const double lx = (double)d.nx * d.res, ly = (double)d.ny * d.res;
     const double fx = kPi / lx, fy = kPi / ly;  // basis.cpp:85: cos(k * (PI / l) * x)
-    double* const slot = p.slots + (size_t)u * K;
+    double* const slot = p.slots + (size_t)su * K;
     __syncthreads();  // the previous unit's readers of s_ys / s_t are done
     if (t == 32)
     {
@@ -187,13 +209,19 @@ __global__ void __launch_bounds__(kMbThreads, 3) map_target_batch_kernel(const M
 
     // the last unit of this map to arrive finishes the instance
     const int nunits = mb_units(d.ny);
+    int arrivals = nunits, s0 = d.unit0;
+    if constexpr (KEPT)
+    {
+      arrivals = p.kept[lo].count;
+      s0 = p.kept[lo].slot0;
+    }
     __threadfence();
     __syncthreads();
-    if (t == 0) s_last = atomicAdd(p.arrive + d.inst, 1u) == (unsigned)(nunits - 1);
+    if (t == 0) s_last = atomicAdd(p.arrive + d.inst, 1u) == (unsigned)(arrivals - 1);
     __syncthreads();
     if (!s_last) continue;
     __threadfence();
-    const double* base = p.slots + (size_t)d.unit0 * K;
+    const double* base = p.slots + (size_t)s0 * K;
     double total = 0.0;  // raw[0] = sum(Phi), summed in unit order
     for (int v = 0; v < nunits; v++) total += __ldcg(base + (size_t)v * K);
     double* const row = p.phik + (size_t)d.inst * K;

@@ -368,6 +368,22 @@ eb_status eb_grid_batch_set_maps_dev(eb_grid_batch *g, const signed char *const 
 eb_status eb_grid_batch_set_maps_host(eb_grid_batch *g, const signed char *const *cells, const unsigned *xsize,
                                       const unsigned *ysize, const double *resolution, const double *origin,
                                       const int *update);
+/* eb_grid_batch_set_rows_dev / _host: rows [row_begin[i], row_begin[i] + row_count[i]) of map i <- rows[i], row_count[i]
+ *   x xsize_i int8 cells in GridMap layout (device pointers for _dev, host pointers for _host), for every instance i
+ *   with update[i] != 0 (update NULL: all).  The map must be there already; its geometry, resolution and origin do not
+ *   change (a map that changes shape or origin goes through eb_grid_batch_set_maps_*).  row_begin, row_count and update
+ *   are host arrays of B; a flagged instance with row_count 0, and every unflagged instance, is not read.  One kernel
+ *   launch per call (none when no row is written), after the grid batch's last safe tick or
+ *   eb_set_map_targets_from_grid_batch; _dev is stream-ordered, _host packs the bands into one pinned buffer, copies
+ *   it with one cudaMemcpyAsync and synchronises.  EB_ERR_INVALID_ARGUMENT, before anything is copied or launched, for
+ *   a NULL handle or array, a flagged instance without a map, row_begin + row_count > ysize_i, or a NULL band of a
+ *   flagged instance with row_count > 0.
+ * eb_grid_batch_get_map_host: map i (ysize_i x xsize_i bytes) out of the arena into cells; synchronises. */
+eb_status eb_grid_batch_set_rows_dev(eb_grid_batch *g, const signed char *const *rows_dev, const unsigned *row_begin,
+                                     const unsigned *row_count, const int *update /* B or NULL */);
+eb_status eb_grid_batch_set_rows_host(eb_grid_batch *g, const signed char *const *rows, const unsigned *row_begin,
+                                      const unsigned *row_count, const int *update);
+eb_status eb_grid_batch_get_map_host(const eb_grid_batch *g, int i, signed char *cells);
 eb_status eb_collision_check_batch_host(eb_grid_batch *g, const eb_collision *c, const double *poses, int per, int *hit);
 eb_status eb_collision_check_batch_dev(eb_grid_batch *g, const eb_collision *c, const double *poses_dev, int per,
                                        int *hit_dev);
@@ -479,6 +495,27 @@ eb_status eb_set_map_targets_batch_dev(eb_controller *c, const signed char *cons
 eb_status eb_set_map_targets_batch_host(eb_controller *c, const signed char *const *cells, const unsigned *xsize,
                                         const unsigned *ysize, const double *resolution, const double *origin,
                                         const int *update);
+/* The same targets from the maps of an eb_grid_batch, without a second upload: for every flagged instance i
+ * (update NULL: all) the row, the frame and the replay cosines equal, bit for bit, what eb_set_map_targets_batch_dev
+ * returns for map i's cells, geometry and origin, with the same rules (per-instance mode, unflagged instances not
+ * touched).  row_begin / row_count NULL: whole maps.  Otherwise (host arrays of B) they declare the rows of map i that
+ * changed since this controller last derived instance i from this grid batch: the arrays given to
+ * eb_grid_batch_set_rows_*, or their union over several such calls.  The controller keeps each derived instance's raw
+ * nb x nb block of every 64-row unit of its map, and recomputes only the units that meet the declared rows; the row is
+ * then the sum of all kept blocks in unit order, as in the full call.  An instance is recomputed whole when it has no
+ * kept blocks yet, when they came from another grid batch or from a map of another xsize, ysize or resolution, or when
+ * its map was replaced by eb_grid_batch_set_maps_* since.  A flagged instance with nothing to recompute keeps the row
+ * and frame it was last derived with.
+ * The kept blocks take K doubles per unit: for 4096 maps of 160-640 rows (about 27.6 k units) 22 MB at nb 10, 57 MB at
+ * nb 16, 226 MB at nb 32 and 0.9 GB at nb 64, plus up to a quarter of headroom for a map that grew (its slot then
+ * takes its units and a quarter more, so a growing map rarely moves the blocks).
+ * Stream-ordered on the controller's stream, after the work enqueued on the grid batch's stream, with one kernel
+ * launch (none when no unit needs work); the grid batch's next set or rows call waits for it.
+ * EB_ERR_INVALID_ARGUMENT, before anything is launched: a NULL handle, a grid batch of another B or on another device,
+ * a flagged instance without a map, row_begin + row_count > ysize_i, or only one of row_begin / row_count NULL. */
+eb_status eb_set_map_targets_from_grid_batch(eb_controller *c, eb_grid_batch *g,
+                                             const unsigned *row_begin /* B or NULL */,
+                                             const unsigned *row_count /* B or NULL */, const int *update /* B or NULL */);
 
 /* ---- safe control tick of B robots on B maps -----------------------------------------------------------------------
  * The reference loop's arbitration between the ergodic twist and the safety planner (exploration.hpp:238-247) for a

@@ -81,7 +81,8 @@ class DeviceGridBatch
 {
 public:
   template <class GridT>
-  explicit DeviceGridBatch(const std::vector<GridT>& grids) : batch_(static_cast<unsigned int>(grids.size()))
+  explicit DeviceGridBatch(const std::vector<GridT>& grids)
+    : batch_(static_cast<unsigned int>(grids.size())), xsize_(grids.size(), 0)
   {
     if (grids.empty()) throw std::logic_error("DeviceGridBatch: need at least one grid");
     eb_grid_batch* g = nullptr;
@@ -112,6 +113,33 @@ public:
     }
     check(eb_grid_batch_set_maps_host(h_.get(), cells.data(), xs.data(), ys.data(), res.data(), origin.data(),
                                       upd.data()));
+    for (unsigned int i = 0; i < batch_; i++)
+      if (upd[i]) xsize_[i] = xs[i];
+  }
+
+  /**
+   * @brief rows [row_begin[i], row_begin[i] + n_i) of map i <- bands[i] (n_i x xsize_i cells, GridMap layout) when
+   * (*update)[i] (nullptr: all); shapes and origins do not change.  Pass row_begin and the n_i to setMapTargets.
+   */
+  void updateRows(const std::vector<std::vector<signed char>>& bands, const std::vector<unsigned>& row_begin,
+                  const std::vector<bool>* update = nullptr)
+  {
+    if (bands.size() != batch_ || row_begin.size() != batch_)
+      throw std::logic_error("DeviceGridBatch::updateRows: need B bands and B row_begin");
+    if (update && update->size() != batch_) throw std::logic_error("DeviceGridBatch::updateRows: update needs B flags");
+    std::vector<const signed char*> rows(batch_, nullptr);
+    std::vector<unsigned> count(batch_, 0);
+    std::vector<int> upd(batch_, 1);
+    for (unsigned int i = 0; i < batch_; i++)
+    {
+      if (update) upd[i] = (*update)[i] ? 1 : 0;
+      if (!upd[i] || bands[i].empty()) continue;
+      if (xsize_[i] == 0 || bands[i].size() % xsize_[i] != 0)
+        throw std::logic_error("DeviceGridBatch::updateRows: band " + std::to_string(i) + " is not whole rows of its map");
+      rows[i] = bands[i].data();
+      count[i] = static_cast<unsigned>(bands[i].size() / xsize_[i]);
+    }
+    check(eb_grid_batch_set_rows_host(h_.get(), rows.data(), row_begin.data(), count.data(), upd.data()));
   }
 
   eb_grid_batch* handle() const { return h_.get(); }
@@ -127,6 +155,7 @@ public:
 
 private:
   unsigned int batch_;
+  std::vector<unsigned> xsize_;  // of each map set so far (0: none)
   std::shared_ptr<eb_grid_batch> h_;
 };
 
@@ -331,6 +360,28 @@ std::tuple<arma::mat, std::vector<int>> controlSafe(BatchedErgodicControl<ModelT
                                    val_horizon, nullptr, X.memptr(), nullptr, VB.memptr(), u.memptr(), branch.data(),
                                    nullptr));
   return std::make_tuple(u, branch);
+}
+
+/**
+ * @brief ErgodicControl::setMapTargets of every flagged instance i from map i of grids, without uploading the cells
+ * again: bit for bit the target of map i's cells and geometry.  row_begin / row_count (both or neither; nullptr: whole
+ * maps) declare the rows of map i changed since ctl last derived instance i from grids (what updateRows was given);
+ * only the 64-row units that meet them are recomputed.
+ */
+template <class ModelT>
+void setMapTargets(BatchedErgodicControl<ModelT>& ctl, DeviceGridBatch& grids,
+                   const std::vector<unsigned>* row_begin = nullptr, const std::vector<unsigned>* row_count = nullptr,
+                   const std::vector<bool>* update = nullptr)
+{
+  const unsigned int B = grids.batch();
+  if (ctl.batch() != B) throw std::logic_error("setMapTargets: the controller and the grid batch need the same B");
+  if ((row_begin && row_begin->size() != B) || (row_count && row_count->size() != B) || (update && update->size() != B))
+    throw std::logic_error("setMapTargets: row_begin, row_count and update need B entries");
+  std::vector<int> upd(B, 1);
+  if (update)
+    for (unsigned int i = 0; i < B; i++) upd[i] = (*update)[i] ? 1 : 0;
+  check(eb_set_map_targets_from_grid_batch(ctl.handle(), grids.handle(), row_begin ? row_begin->data() : nullptr,
+                                           row_count ? row_count->data() : nullptr, upd.data()));
 }
 }  // namespace b200
 }  // namespace ergodic_exploration

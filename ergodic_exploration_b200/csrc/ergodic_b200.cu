@@ -46,18 +46,21 @@ eb_status fail(eb_status st, const std::string& msg)
   return st;
 }
 
-#define EB_CUDA(expr)                                                                                   \
-  do                                                                                                    \
-  {                                                                                                     \
-    cudaError_t e__ = (expr);                                                                           \
-    if (e__ != cudaSuccess)                                                                             \
-    {                                                                                                   \
-      const eb_status st__ = (e__ == cudaErrorNoDevice || e__ == cudaErrorInsufficientDriver ||         \
-                              e__ == cudaErrorInvalidDevice) ?                                          \
-                                 EB_ERR_NO_DEVICE :                                                     \
-                                 EB_ERR_CUDA;                                                           \
-      return fail(st__, std::string(#expr) + ": " + cudaGetErrorName(e__) + ": " + cudaGetErrorString(e__)); \
-    }                                                                                                   \
+// a failed runtime call: EB_ERR_NO_DEVICE when there is no usable device, else EB_ERR_CUDA; `what` names the call
+eb_status fail_cuda(cudaError_t e, const std::string& what)
+{
+  const eb_status st = (e == cudaErrorNoDevice || e == cudaErrorInsufficientDriver || e == cudaErrorInvalidDevice) ?
+                           EB_ERR_NO_DEVICE :
+                           EB_ERR_CUDA;
+  return fail(st, what + ": " + cudaGetErrorName(e) + ": " + cudaGetErrorString(e));
+}
+
+#define EB_CUDA(expr)                                   \
+  do                                                    \
+  {                                                     \
+    cudaError_t e__ = (expr);                           \
+    if (e__ != cudaSuccess)                             \
+      return fail_cuda(e__, std::string(#expr));        \
   } while (0)
 
 // NVTX range around a C-ABI call (SURVEY.md section 5: tracing hook)
@@ -67,6 +70,101 @@ struct NvtxRange
   ~NvtxRange() { nvtxRangePop(); }
 };
 #define EB_TRACE(name) NvtxRange nvtx_range__(name)
+
+// the message of a failed allocation of `bytes` for the buffer `name`
+std::string alloc_what(const char* name, const char* call, size_t bytes)
+{
+  return std::string(name) + ": " + call + " of " + std::to_string(bytes) + " bytes";
+}
+
+// A device array of at least `cap` elements, owned: scratch that grows on demand, so a control loop pays no
+// allocation per tick.  Growing frees the old array first (cudaFree synchronises with the launches that still use it)
+// and keeps no contents.  `name` identifies the buffer in the message of a failed allocation.
+template <class T>
+struct DevScratch
+{
+  const char* name;
+  T* p = nullptr;
+  size_t cap = 0;
+  explicit DevScratch(const char* name) : name(name) {}
+  DevScratch(const DevScratch&) = delete;
+  DevScratch& operator=(const DevScratch&) = delete;
+  ~DevScratch() { cudaFree(p); }
+  eb_status reserve(size_t n)
+  {
+    if (n <= cap) return EB_OK;
+    cudaFree(p);
+    p = nullptr;
+    cap = 0;
+    if (const cudaError_t e = cudaMalloc(&p, sizeof(T) * n))
+      return fail_cuda(e, alloc_what(name, "cudaMalloc", sizeof(T) * n));
+    cap = n;
+    return EB_OK;
+  }
+};
+
+// A pinned host array and a device array of the same length, owned: records or cells written on the host and uploaded
+// with one cudaMemcpyAsync.  Grows as DevScratch.
+template <class T>
+struct Pinned
+{
+  const char* name;
+  T* h = nullptr;
+  T* d = nullptr;
+  size_t cap = 0;
+  explicit Pinned(const char* name) : name(name) {}
+  Pinned(const Pinned&) = delete;
+  Pinned& operator=(const Pinned&) = delete;
+  ~Pinned()
+  {
+    cudaFreeHost(h);
+    cudaFree(d);
+  }
+  eb_status reserve(size_t n)
+  {
+    if (n <= cap) return EB_OK;
+    cudaFreeHost(h);
+    cudaFree(d);
+    h = d = nullptr;
+    cap = 0;
+    if (const cudaError_t e = cudaHostAlloc(&h, sizeof(T) * n, cudaHostAllocDefault))
+      return fail_cuda(e, alloc_what(name, "cudaHostAlloc", sizeof(T) * n));
+    if (const cudaError_t e = cudaMalloc(&d, sizeof(T) * n))
+      return fail_cuda(e, alloc_what(name, "cudaMalloc", sizeof(T) * n));
+    cap = n;
+    return EB_OK;
+  }
+};
+
+// Packs src[i] (bytes(i) bytes, 0: nothing to copy) of every instance that `update` flags into `buf` at 16-byte
+// aligned offsets and uploads them with one cudaMemcpyAsync on `stream`; (*dev)[i] is instance i's device copy, or
+// NULL.  The stream is synchronised first, so no earlier copy still reads the buffer.
+template <class Bytes>
+eb_status pack_flagged(Pinned<signed char>& buf, cudaStream_t stream, int B, const int* update,
+                       const signed char* const* src, const Bytes& bytes, std::vector<const signed char*>* dev)
+{
+  std::vector<size_t> off((size_t)B, 0), len((size_t)B, 0);
+  size_t total = 0;
+  for (int i = 0; i < B; i++)
+  {
+    if (update && !update[i]) continue;
+    len[i] = bytes(i);
+    off[i] = total;
+    total += (len[i] + 15) & ~(size_t)15;
+  }
+  EB_CUDA(cudaStreamSynchronize(stream));
+  const eb_status st = buf.reserve(total);
+  if (st != EB_OK) return st;
+  dev->assign((size_t)B, nullptr);
+  for (int i = 0; i < B; i++)
+    if (len[i] > 0)
+    {
+      std::memcpy(buf.h + off[i], src[i], len[i]);
+      (*dev)[i] = buf.d + off[i];
+    }
+  if (total > 0) EB_CUDA(cudaMemcpyAsync(buf.d, buf.h, total, cudaMemcpyHostToDevice, stream));
+  return EB_OK;
+}
 
 // grid.hpp:61-64
 unsigned axis_length(double lower, double upper, double resolution)
@@ -115,7 +213,8 @@ struct eb_phik_plan
   double *d_T = nullptr;                    // stage-1 result [ny][32]
   double *d_parts = nullptr;                // partial 32x32 blocks
   double *d_phik = nullptr, *d_sum = nullptr;  // staging for the _host call
-  double* d_phi_stage = nullptr;               // device copy of the density for the _host call (kept between calls)
+  // device copy of the density for the _host call (kept between calls)
+  DevScratch<double> d_phi_stage{ "eb_phik_plan::d_phi_stage" };
   unsigned int* d_done = nullptr;              // arrival counter of the TMA kernel's fused final sum
   const eb::PhikTmaPeer* peer = nullptr;       // set for the duration of eb_phik_execute_allreduce_dev
   int max_parts = 0;
@@ -358,7 +457,6 @@ void eb_phik_plan_destroy(eb_phik_plan* p)
   cudaFree(p->d_parts);
   cudaFree(p->d_phik);
   cudaFree(p->d_sum);
-  cudaFree(p->d_phi_stage);
   cudaFree(p->d_done);
   for (double* q : p->w_cxt) cudaFree(q);
   for (double* q : p->w_cxtf) cudaFree(q);
@@ -494,11 +592,11 @@ eb_status eb_phik_execute_host(eb_phik_plan* p, const double* phi, double* phik,
   EB_TRACE("eb_phik_execute_host");
   if (!p || !phi || !phik) return fail(EB_ERR_INVALID_ARGUMENT, "eb_phik_execute_host: NULL argument");
   EB_CUDA(cudaSetDevice(p->device));
-  const size_t bytes = sizeof(double) * (size_t)p->nx * p->ny;
-  if (!p->d_phi_stage) EB_CUDA(cudaMalloc(&p->d_phi_stage, bytes));  // once per plan: a map update reuses it
-  double* const d_phi = p->d_phi_stage;
-  cudaError_t e = cudaMemcpyAsync(d_phi, phi, bytes, cudaMemcpyHostToDevice, p->stream);
-  eb_status st = EB_OK;
+  const size_t cells = (size_t)p->nx * p->ny;
+  eb_status st = p->d_phi_stage.reserve(cells);  // once per plan: a map update reuses it
+  if (st != EB_OK) return st;
+  double* const d_phi = p->d_phi_stage.p;
+  cudaError_t e = cudaMemcpyAsync(d_phi, phi, sizeof(double) * cells, cudaMemcpyHostToDevice, p->stream);
   if (e == cudaSuccess) st = eb_phik_execute_dev(p, d_phi, p->d_phik, p->d_sum);
   if (e == cudaSuccess && st == EB_OK)
     e = cudaMemcpyAsync(phik, p->d_phik, sizeof(double) * p->nb * p->nb, cudaMemcpyDeviceToHost, p->stream);
@@ -555,7 +653,8 @@ struct eb_controller
   long long hist_cap = 0, mem_count = 0;
   double *d_phik = nullptr, *d_lamk = nullptr;
   double *d_u0 = nullptr, *d_metric = nullptr, *d_ck = nullptr, *d_x = nullptr;
-  double* d_xt = nullptr;                  // [B][N][3] staging of eb_opt_traj_host (allocated on first use, kept)
+  // [B][N][3] staging of eb_opt_traj_host (allocated on first use, kept)
+  DevScratch<double> d_xt{ "eb_controller::d_xt" };
   double* d_big_scratch = nullptr;         // num_basis > 32: [big_rows][K], one row per resident CTA of solve_kernel_big
   int big_rows = 0;
   int *d_mem_idx_in = nullptr, *d_mem_idx_out = nullptr;
@@ -565,10 +664,8 @@ struct eb_controller
   double map_pos[2] = { 0.0, 0.0 };
   std::vector<double> gauss_mu, gauss_sigma;  // target_
   eb_phik_plan* plan = nullptr;               // cached for the current extent
-  double* d_phi_grid = nullptr;
-  size_t phi_grid_cells = 0;
-  double* d_gauss = nullptr;
-  int gauss_cap = 0;
+  DevScratch<double> d_phi_grid{ "eb_controller::d_phi_grid" };  // the target density on the plan's grid
+  DevScratch<double> d_gauss{ "eb_controller::d_gauss" };  // [6] per Gaussian
   unsigned long long call = 0;
   long long launches = 0;
   bool have_pose = false;
@@ -580,20 +677,17 @@ struct eb_controller
   bool frames_set = false;          // a configure or eb_set_phik_batch_dev has given every instance a frame
   double* d_phik_b = nullptr;       // [B][K]
   double* d_frames = nullptr;       // [B][eb::kFrDoubles]
-  double *d_gmu = nullptr, *d_gsig = nullptr;  // [B][gmax][2]
+  DevScratch<double> d_gmu{ "eb_controller::d_gmu" };  // [B][gmax][2]
+  DevScratch<double> d_gsig{ "eb_controller::d_gsig" };
   int* d_gcount = nullptr;          // [B]
   int gmax = 0;
-  double* d_bounds = nullptr;       // [B][4] staging of eb_control_batch_host
+  DevScratch<double> d_bounds{ "eb_controller::d_bounds" };  // [B][4] staging of eb_control_batch_host
   // map-derived targets per instance (eb_set_map_targets_batch_*, map_target_batch.cuh)
-  eb::MapBatchDesc* h_mb_desc = nullptr;  // [B] pinned: the maps of a call
-  eb::MapBatchDesc* d_mb_desc = nullptr;  // [B]
+  Pinned<eb::MapBatchDesc> mb_desc{ "eb_controller::mb_desc" };  // [B]: the maps of a call
   cudaEvent_t mb_staged = nullptr;        // recorded after the copies out of the pinned buffers
-  double* d_mb_slots = nullptr;           // [units][K] raw blocks
-  long long mb_slot_units = 0;
-  unsigned* d_mb_arrive = nullptr;        // [B] arrival counters (zero between launches)
-  signed char* h_mb_cells = nullptr;      // pinned staging of the _host call's maps
-  signed char* d_mb_cells = nullptr;
-  size_t mb_cells_bytes = 0;
+  DevScratch<double> d_mb_slots{ "eb_controller::d_mb_slots" };  // [units][K] raw blocks
+  DevScratch<unsigned> d_mb_arrive{ "eb_controller::d_mb_arrive" };  // [B] arrival counters (zero between launches)
+  Pinned<signed char> mb_cells{ "eb_controller::mb_cells" };  // staging of the _host call's maps
   int mb_grid = 0;                        // resident CTAs of map_target_batch_kernel on the device
   // kept blocks of eb_set_map_targets_from_grid_batch: instance i's raw block of unit v of its map is slot
   // kb_slot0[i] + v of d_kb (kb_cap[i] slots reserved); kb_key[i] says which map the blocks belong to
@@ -606,12 +700,11 @@ struct eb_controller
   double* d_kb = nullptr;
   std::vector<int> kb_slot0, kb_cap;
   std::vector<KeptKey> kb_key;
-  eb::MapKept* h_mb_kept = nullptr;  // [B] pinned: the recomputed units of a call
-  eb::MapKept* d_mb_kept = nullptr;
+  Pinned<eb::MapKept> mb_kept{ "eb_controller::mb_kept" };  // [B]: the recomputed units of a call
   // safe control tick (eb_control_safe_batch_*, safe_control.cuh)
   int* d_safe_list = nullptr;      // [1 + B]: the count of failing robots, then their indices
-  int* d_safe_branch = nullptr;    // [B] staging of the _host call
-  double* d_safe_vb = nullptr;     // [B][3] staging of the _host call
+  DevScratch<int> d_safe_branch{ "eb_controller::d_safe_branch" };  // [B] staging of the _host call
+  DevScratch<double> d_safe_vb{ "eb_controller::d_safe_vb" };  // [B][3] staging of the _host call
   int safe_grid = 0;               // resident CTAs of dwa_fallback_kernel with this horizon
 
   // device alias of a page-locked host buffer (nullptr for pageable memory);
@@ -912,7 +1005,8 @@ eb_status ensure_per_inst(eb_controller* c)
   EB_CUDA(cudaMalloc(&c->d_phik_b, pb));
   EB_CUDA(cudaMalloc(&c->d_frames, fb));
   EB_CUDA(cudaMalloc(&c->d_gcount, sizeof(int) * (size_t)c->B));
-  EB_CUDA(cudaMalloc(&c->d_bounds, sizeof(double) * 4 * (size_t)c->B));
+  const eb_status st = c->d_bounds.reserve(4 * (size_t)c->B);
+  if (st != EB_OK) return st;
   EB_CUDA(cudaMemsetAsync(c->d_phik_b, 0, pb, c->stream));
   EB_CUDA(cudaMemsetAsync(c->d_frames, 0, fb, c->stream));
   EB_CUDA(cudaMemsetAsync(c->d_gcount, 0, sizeof(int) * (size_t)c->B, c->stream));
@@ -931,8 +1025,8 @@ eb_status target_batch(eb_controller* c, const double* bounds_dev, const double*
   tp.bounds = bounds_dev;
   tp.extent = extent_dev;
   tp.counts = c->d_gcount;
-  tp.mu = c->d_gmu;
-  tp.sigma = c->d_gsig;
+  tp.mu = c->d_gmu.p;
+  tp.sigma = c->d_gsig.p;
   tp.frames = c->d_frames;
   tp.phik = c->d_phik_b;
   tp.rebuilt = rebuilt_dev;
@@ -945,6 +1039,50 @@ eb_status target_batch(eb_controller* c, const double* bounds_dev, const double*
   c->launches += 1;
   c->frames_set = true;
   return EB_OK;
+}
+
+// the _host control calls' uploads of the per-instance bounds ([B][4], when given) and of the replay sample indices
+// (when the solve samples with them); *idx_dev is the device copy of the indices, or NULL
+eb_status upload_bounds_idx(eb_controller* c, const double* bounds, const int* mem_idx, const int** idx_dev)
+{
+  if (bounds)
+    EB_CUDA(cudaMemcpyAsync(c->d_bounds.p, bounds, sizeof(double) * 4 * (size_t)c->B, cudaMemcpyHostToDevice, c->stream));
+  const bool need_idx = mem_idx && c->mem_count > (long long)c->cfg.batch_size;
+  if (need_idx)
+    EB_CUDA(cudaMemcpyAsync(c->d_mem_idx_in, mem_idx, sizeof(int) * (size_t)c->cfg.batch_size * c->B,
+                            cudaMemcpyHostToDevice, c->stream));
+  *idx_dev = need_idx ? c->d_mem_idx_in : nullptr;
+  return EB_OK;
+}
+
+// eb_control_host and eb_control_batch_host after their checks: dev(x, mem_idx, u0, metric) is the _dev call, given
+// device pointers; bounds are uploaded when given
+template <class Dev>
+eb_status control_host(eb_controller* c, const double* bounds, const double* x, const int* mem_idx, double* u0,
+                       double* metric, const Dev& dev)
+{
+  const int* idx = nullptr;
+  eb_status st = upload_bounds_idx(c, bounds, mem_idx, &idx);
+  if (st != EB_OK) return st;
+  // Small batches with page-locked caller buffers: the kernel reads x and writes
+  // u0 / metric in place over PCIe (one launch + one sync, no copy-engine hops).
+  double *xm = nullptr, *um = nullptr, *mm = nullptr;
+  if (c->B <= zero_copy_max_batch())
+  {
+    xm = c->mapped(x);
+    um = xm ? c->mapped(u0) : nullptr;
+    mm = (um && metric) ? c->mapped(metric) : nullptr;
+  }
+  if (xm && um && (!metric || mm))
+  {
+    if ((st = dev(xm, idx, um, mm)) != EB_OK) return st;
+    return check_fault(c);  // synchronises
+  }
+  EB_CUDA(cudaMemcpyAsync(c->d_pose, x, sizeof(double) * 3 * c->B, cudaMemcpyHostToDevice, c->stream));
+  if ((st = dev(c->d_pose, idx, c->d_u0, metric ? c->d_metric : nullptr)) != EB_OK) return st;
+  EB_CUDA(cudaMemcpyAsync(u0, c->d_u0, sizeof(double) * 3 * c->B, cudaMemcpyDeviceToHost, c->stream));
+  if (metric) EB_CUDA(cudaMemcpyAsync(metric, c->d_metric, sizeof(double) * c->B, cudaMemcpyDeviceToHost, c->stream));
+  return check_fault(c);  // synchronises
 }
 }  // namespace
 
@@ -1042,6 +1180,7 @@ void eb_destroy(eb_controller* c)
 {
   if (!c) return;
   cudaSetDevice(c->cfg.device);
+  if (c->mb_staged) cudaEventSynchronize(c->mb_staged);
   cudaFree(c->d_ut[0]);
   cudaFree(c->d_ut[1]);
   cudaFree(c->d_pose);
@@ -1050,38 +1189,21 @@ void eb_destroy(eb_controller* c)
   cudaFree(c->d_phik);
   cudaFree(c->d_lamk);
   cudaFree(c->d_u0);
-  cudaFree(c->d_xt);
   cudaFree(c->d_metric);
   cudaFree(c->d_ck);
   cudaFree(c->d_x);
   cudaFree(c->d_mem_idx_in);
   cudaFree(c->d_mem_idx_out);
   cudaFreeHost(c->h_fault);
-  cudaFree(c->d_phi_grid);
-  cudaFree(c->d_gauss);
   cudaFree(c->d_big_scratch);
   cudaFree(c->d_phik_b);
   cudaFree(c->d_frames);
-  cudaFree(c->d_gmu);
-  cudaFree(c->d_gsig);
   cudaFree(c->d_gcount);
-  cudaFree(c->d_bounds);
-  if (c->mb_staged) cudaEventSynchronize(c->mb_staged);
-  cudaFreeHost(c->h_mb_desc);
-  cudaFree(c->d_mb_desc);
   if (c->mb_staged) cudaEventDestroy(c->mb_staged);
-  cudaFree(c->d_mb_slots);
-  cudaFreeHost(c->h_mb_kept);
-  cudaFree(c->d_mb_kept);
   cudaFree(c->d_kb);
-  cudaFree(c->d_mb_arrive);
-  cudaFreeHost(c->h_mb_cells);
-  cudaFree(c->d_mb_cells);
   cudaFree(c->d_safe_list);
-  cudaFree(c->d_safe_branch);
-  cudaFree(c->d_safe_vb);
   eb_phik_plan_destroy(c->plan);
-  delete c;
+  delete c;  // the staging members free themselves here
 }
 
 eb_status eb_clone(const eb_controller* src, eb_controller** out)
@@ -1143,10 +1265,14 @@ eb_status eb_clone(const eb_controller* src, eb_controller** out)
       return bail(e);
     if (src->gmax > 0)
     {
-      const size_t gb = sizeof(double) * 2 * (size_t)src->gmax * B;
-      if ((e = cudaMalloc(&c->d_gmu, gb)) != cudaSuccess || (e = cudaMalloc(&c->d_gsig, gb)) != cudaSuccess ||
-          (e = cudaMemcpy(c->d_gmu, src->d_gmu, gb, cudaMemcpyDeviceToDevice)) != cudaSuccess ||
-          (e = cudaMemcpy(c->d_gsig, src->d_gsig, gb, cudaMemcpyDeviceToDevice)) != cudaSuccess)
+      const size_t gd = 2 * (size_t)src->gmax * B;
+      if ((st = c->d_gmu.reserve(gd)) != EB_OK || (st = c->d_gsig.reserve(gd)) != EB_OK)
+      {
+        eb_destroy(c);
+        return st;
+      }
+      if ((e = cudaMemcpy(c->d_gmu.p, src->d_gmu.p, sizeof(double) * gd, cudaMemcpyDeviceToDevice)) != cudaSuccess ||
+          (e = cudaMemcpy(c->d_gsig.p, src->d_gsig.p, sizeof(double) * gd, cudaMemcpyDeviceToDevice)) != cudaSuccess)
         return bail(e);
       c->gmax = src->gmax;
     }
@@ -1218,22 +1344,7 @@ eb_status eb_config_target(eb_controller* c, double xmin, double xmax, double ym
   c->plan = plan;
   c->plan->stream = c->stream;
   const size_t cells = (size_t)nx * ny;
-  if (cells > c->phi_grid_cells)
-  {
-    cudaFree(c->d_phi_grid);
-    c->d_phi_grid = nullptr;
-    c->phi_grid_cells = 0;
-    EB_CUDA(cudaMalloc(&c->d_phi_grid, sizeof(double) * cells));
-    c->phi_grid_cells = cells;
-  }
-  if (ng > c->gauss_cap)
-  {
-    cudaFree(c->d_gauss);
-    c->d_gauss = nullptr;
-    c->gauss_cap = 0;
-    EB_CUDA(cudaMalloc(&c->d_gauss, sizeof(double) * 6 * (size_t)ng));
-    c->gauss_cap = ng;
-  }
+  if ((st = c->d_phi_grid.reserve(cells)) != EB_OK || (st = c->d_gauss.reserve(6 * (size_t)ng)) != EB_OK) return st;
   // Gaussian ctor (target.hpp:68-71): cov = diag(sigma^2), cov_inv = inv(cov)
   // (2x2 cofactor inverse); operator() (:91-102) translates the mean.
   std::vector<double> g(6 * (size_t)ng);
@@ -1249,13 +1360,13 @@ eb_status eb_config_target(eb_controller* c, double xmin, double xmax, double ym
     g[6 * i + 4] = -0.0 / det;  // ci(0,1)
     g[6 * i + 5] = a / det;     // ci(1,1)
   }
-  EB_CUDA(cudaMemcpyAsync(c->d_gauss, g.data(), sizeof(double) * g.size(), cudaMemcpyHostToDevice, c->stream));
+  EB_CUDA(cudaMemcpyAsync(c->d_gauss.p, g.data(), sizeof(double) * g.size(), cudaMemcpyHostToDevice, c->stream));
   EB_CUDA(cudaStreamSynchronize(c->stream));  // g is a stack-lifetime buffer
-  eb::target_fill_kernel<<<(unsigned)((cells + 255) / 256), 256, 0, c->stream>>>(ng, c->d_gauss, c->plan->d_xs,
-                                                                                 c->plan->d_ys, nx, ny, c->d_phi_grid);
+  eb::target_fill_kernel<<<(unsigned)((cells + 255) / 256), 256, 0, c->stream>>>(ng, c->d_gauss.p, c->plan->d_xs,
+                                                                                 c->plan->d_ys, nx, ny, c->d_phi_grid.p);
   c->launches += 1;
   EB_CUDA(cudaGetLastError());
-  st = eb_phik_execute_dev(c->plan, c->d_phi_grid, c->d_phik, nullptr);
+  st = eb_phik_execute_dev(c->plan, c->d_phi_grid.p, c->d_phik, nullptr);
   if (st != EB_OK) return st;
   c->lx = mx;  // :382-383
   c->ly = my;
@@ -1486,32 +1597,9 @@ eb_status eb_control_host(eb_controller* c, double xmin, double xmax, double ymi
   if (!c || !x || !u0) return fail(EB_ERR_INVALID_ARGUMENT, "eb_control_host: NULL argument");
   if (c->per_inst) return refuse_per_inst("eb_control_host");
   EB_CUDA(cudaSetDevice(c->cfg.device));
-  const bool need_idx = mem_idx && c->mem_count > (long long)c->cfg.batch_size;
-  if (need_idx)
-    EB_CUDA(cudaMemcpyAsync(c->d_mem_idx_in, mem_idx, sizeof(int) * (size_t)c->cfg.batch_size * c->B,
-                            cudaMemcpyHostToDevice, c->stream));
-  // Small batches with page-locked caller buffers: the kernel reads x and writes
-  // u0 / metric in place over PCIe (one launch + one sync, no copy-engine hops).
-  double *xm = nullptr, *um = nullptr, *mm = nullptr;
-  if (c->B <= zero_copy_max_batch())
-  {
-    xm = c->mapped(x);
-    um = xm ? c->mapped(u0) : nullptr;
-    mm = (um && metric) ? c->mapped(metric) : nullptr;
-  }
-  if (xm && um && (!metric || mm))
-  {
-    eb_status st = eb_control_dev(c, xmin, xmax, ymin, ymax, xm, need_idx ? c->d_mem_idx_in : nullptr, um, mm);
-    if (st != EB_OK) return st;
-    return check_fault(c);  // synchronises
-  }
-  EB_CUDA(cudaMemcpyAsync(c->d_pose, x, sizeof(double) * 3 * c->B, cudaMemcpyHostToDevice, c->stream));
-  eb_status st = eb_control_dev(c, xmin, xmax, ymin, ymax, c->d_pose, need_idx ? c->d_mem_idx_in : nullptr, c->d_u0,
-                                metric ? c->d_metric : nullptr);
-  if (st != EB_OK) return st;
-  EB_CUDA(cudaMemcpyAsync(u0, c->d_u0, sizeof(double) * 3 * c->B, cudaMemcpyDeviceToHost, c->stream));
-  if (metric) EB_CUDA(cudaMemcpyAsync(metric, c->d_metric, sizeof(double) * c->B, cudaMemcpyDeviceToHost, c->stream));
-  return check_fault(c);  // synchronises
+  return control_host(c, nullptr, x, mem_idx, u0, metric, [&](const double* xd, const int* idx, double* ud, double* md) {
+    return eb_control_dev(c, xmin, xmax, ymin, ymax, xd, idx, ud, md);
+  });
 }
 
 eb_status eb_opt_traj_dev(eb_controller* c, double* xt_dev)
@@ -1536,12 +1624,13 @@ eb_status eb_opt_traj_host(eb_controller* c, double* xt)
 {
   if (!c || !xt) return fail(EB_ERR_INVALID_ARGUMENT, "eb_opt_traj_host: NULL argument");
   EB_CUDA(cudaSetDevice(c->cfg.device));
-  const size_t bytes = sizeof(double) * 3 * (size_t)c->N * c->B;
-  if (!c->d_xt) EB_CUDA(cudaMalloc(&c->d_xt, bytes));  // optTraj() runs every tick (exploration.hpp:234): keep it
-  double* const d = c->d_xt;
-  eb_status st = eb_opt_traj_dev(c, d);
+  const size_t n = 3 * (size_t)c->N * c->B;
+  eb_status st = c->d_xt.reserve(n);  // optTraj() runs every tick (exploration.hpp:234): keep it
+  if (st != EB_OK) return st;
+  double* const d = c->d_xt.p;
+  st = eb_opt_traj_dev(c, d);
   cudaError_t e = cudaSuccess;
-  if (st == EB_OK) e = cudaMemcpyAsync(xt, d, bytes, cudaMemcpyDeviceToHost, c->stream);
+  if (st == EB_OK) e = cudaMemcpyAsync(xt, d, sizeof(double) * n, cudaMemcpyDeviceToHost, c->stream);
   if (st == EB_OK && e == cudaSuccess) st = check_fault(c);
   cudaStreamSynchronize(c->stream);
   if (st != EB_OK) return st;
@@ -2057,14 +2146,12 @@ struct eb_grid
   eb::GridView view{};
   signed char* d_data = nullptr;
   cudaStream_t stream = nullptr;
-  double* d_a = nullptr;  // staging for the _host calls: poses / x0
-  double* d_b = nullptr;  // twists
-  double* d_u = nullptr;  // DynamicWindow: optimal twists
-  double* d_cost = nullptr;
-  double* d_ref = nullptr;  // DynamicWindow: reference twists / trajectories
-  size_t ref_cap = 0;
-  int* d_out = nullptr;
-  int cap = 0;
+  DevScratch<double> d_a{ "eb_grid::d_a" };  // staging for the _host calls: poses / x0
+  DevScratch<double> d_b{ "eb_grid::d_b" };  // twists
+  DevScratch<double> d_u{ "eb_grid::d_u" };  // DynamicWindow: optimal twists
+  DevScratch<double> d_cost{ "eb_grid::d_cost" };
+  DevScratch<double> d_ref{ "eb_grid::d_ref" };  // DynamicWindow: reference twists / trajectories
+  DevScratch<int> d_out{ "eb_grid::d_out" };
   long long launches = 0;
   // pre-dilated map for one set of collision radii / threshold (collision_kernels.cuh, inflate_kernel)
   unsigned char* d_inflated = nullptr;
@@ -2200,28 +2287,6 @@ eb_status use_inflated(eb_grid* g, eb::CollisionParams* p, bool build)
   p->pad = g->infl_pad;
   return EB_OK;
 }
-
-// staging of the _host calls (eb_grid, eb_grid_batch): grown on demand, so a control loop pays no allocation per tick
-template <class G>
-eb_status grid_reserve(G* g, int count)
-{
-  if (count <= g->cap) return EB_OK;
-  cudaFree(g->d_a);
-  cudaFree(g->d_b);
-  cudaFree(g->d_u);
-  cudaFree(g->d_cost);
-  cudaFree(g->d_out);
-  g->d_a = g->d_b = g->d_u = g->d_cost = nullptr;
-  g->d_out = nullptr;
-  g->cap = 0;
-  EB_CUDA(cudaMalloc(&g->d_a, sizeof(double) * 3 * (size_t)count));
-  EB_CUDA(cudaMalloc(&g->d_b, sizeof(double) * 3 * (size_t)count));
-  EB_CUDA(cudaMalloc(&g->d_u, sizeof(double) * 3 * (size_t)count));
-  EB_CUDA(cudaMalloc(&g->d_cost, sizeof(double) * (size_t)count));
-  EB_CUDA(cudaMalloc(&g->d_out, sizeof(int) * (size_t)count));
-  g->cap = count;
-  return EB_OK;
-}
 }  // namespace
 
 extern "C" {
@@ -2267,12 +2332,6 @@ void eb_grid_destroy(eb_grid* g)
   cudaFree(g->d_data);
   cudaFree(g->d_inflated);
   cudaFree(g->d_offsets);
-  cudaFree(g->d_a);
-  cudaFree(g->d_b);
-  cudaFree(g->d_u);
-  cudaFree(g->d_cost);
-  cudaFree(g->d_ref);
-  cudaFree(g->d_out);
   if (g->side) cudaStreamDestroy(g->side);
   if (g->ev_ready) cudaEventDestroy(g->ev_ready);
   if (g->ev_side) cudaEventDestroy(g->ev_side);
@@ -2348,12 +2407,12 @@ eb_status eb_collision_check_host(eb_grid* g, const eb_collision* c, const doubl
   if (count > 0 && (!poses || !hit)) return fail(EB_ERR_INVALID_ARGUMENT, "eb_collision_check_host: NULL argument");
   if (count <= 0) return count == 0 ? EB_OK : fail(EB_ERR_INVALID_ARGUMENT, "count < 0");
   EB_CUDA(cudaSetDevice(g->device));
-  eb_status st = grid_reserve(g, count);
+  eb_status st;
+  if ((st = g->d_a.reserve(3 * (size_t)count)) != EB_OK || (st = g->d_out.reserve(count)) != EB_OK) return st;
+  EB_CUDA(cudaMemcpyAsync(g->d_a.p, poses, sizeof(double) * 3 * (size_t)count, cudaMemcpyHostToDevice, g->stream));
+  st = eb_collision_check_dev(g, c, g->d_a.p, count, g->d_out.p);
   if (st != EB_OK) return st;
-  EB_CUDA(cudaMemcpyAsync(g->d_a, poses, sizeof(double) * 3 * (size_t)count, cudaMemcpyHostToDevice, g->stream));
-  st = eb_collision_check_dev(g, c, g->d_a, count, g->d_out);
-  if (st != EB_OK) return st;
-  EB_CUDA(cudaMemcpyAsync(hit, g->d_out, sizeof(int) * (size_t)count, cudaMemcpyDeviceToHost, g->stream));
+  EB_CUDA(cudaMemcpyAsync(hit, g->d_out.p, sizeof(int) * (size_t)count, cudaMemcpyDeviceToHost, g->stream));
   EB_CUDA(cudaStreamSynchronize(g->stream));
   return EB_OK;
 }
@@ -2365,13 +2424,15 @@ eb_status eb_validate_control_host(eb_grid* g, const eb_collision* c, const doub
   if (count > 0 && (!x0 || !u || !valid)) return fail(EB_ERR_INVALID_ARGUMENT, "eb_validate_control_host: NULL argument");
   if (count <= 0) return count == 0 ? EB_OK : fail(EB_ERR_INVALID_ARGUMENT, "count < 0");
   EB_CUDA(cudaSetDevice(g->device));
-  eb_status st = grid_reserve(g, count);
+  eb_status st = g->d_a.reserve(3 * (size_t)count);
+  if (st == EB_OK) st = g->d_b.reserve(3 * (size_t)count);
+  if (st == EB_OK) st = g->d_out.reserve(count);
   if (st != EB_OK) return st;
-  EB_CUDA(cudaMemcpyAsync(g->d_a, x0, sizeof(double) * 3 * (size_t)count, cudaMemcpyHostToDevice, g->stream));
-  EB_CUDA(cudaMemcpyAsync(g->d_b, u, sizeof(double) * 3 * (size_t)count, cudaMemcpyHostToDevice, g->stream));
-  st = eb_validate_control_dev(g, c, g->d_a, g->d_b, count, dt, horizon, g->d_out);
+  EB_CUDA(cudaMemcpyAsync(g->d_a.p, x0, sizeof(double) * 3 * (size_t)count, cudaMemcpyHostToDevice, g->stream));
+  EB_CUDA(cudaMemcpyAsync(g->d_b.p, u, sizeof(double) * 3 * (size_t)count, cudaMemcpyHostToDevice, g->stream));
+  st = eb_validate_control_dev(g, c, g->d_a.p, g->d_b.p, count, dt, horizon, g->d_out.p);
   if (st != EB_OK) return st;
-  EB_CUDA(cudaMemcpyAsync(valid, g->d_out, sizeof(int) * (size_t)count, cudaMemcpyDeviceToHost, g->stream));
+  EB_CUDA(cudaMemcpyAsync(valid, g->d_out.p, sizeof(int) * (size_t)count, cudaMemcpyDeviceToHost, g->stream));
   EB_CUDA(cudaStreamSynchronize(g->stream));
   return EB_OK;
 }
@@ -2512,16 +2573,13 @@ static eb_status dwa_host(eb_grid* g, const eb_collision* c, const eb_dwa* d, co
   if (count == 0) return EB_OK;
   EB_CUDA(cudaSetDevice(g->device));
   // staging buffers live with the grid (grown on demand), so a control loop pays no allocation per tick
-  eb_status st = grid_reserve(g, count);
+  eb_status st = g->d_a.reserve(3 * (size_t)count);
+  if (st == EB_OK) st = g->d_b.reserve(3 * (size_t)count);
+  if (st == EB_OK) st = g->d_u.reserve(3 * (size_t)count);
+  if (st == EB_OK) st = g->d_cost.reserve(count);
+  if (st == EB_OK) st = g->d_out.reserve(count);
+  if (st == EB_OK) st = g->d_ref.reserve(ref_doubles);
   if (st != EB_OK) return st;
-  if (ref_doubles > g->ref_cap)
-  {
-    cudaFree(g->d_ref);
-    g->d_ref = nullptr;
-    g->ref_cap = 0;
-    EB_CUDA(cudaMalloc(&g->d_ref, sizeof(double) * ref_doubles));
-    g->ref_cap = ref_doubles;
-  }
   auto pinned = [](const void* ptr) {
     cudaPointerAttributes a{};
     if (cudaPointerGetAttributes(&a, ptr) != cudaSuccess)
@@ -2535,28 +2593,28 @@ static eb_status dwa_host(eb_grid* g, const eb_collision* c, const eb_dwa* d, co
     // one slice [lo, lo + n) of the batch on the grid's CURRENT stream: H2D, kernel, D2H
     cudaStream_t s = g->stream;
     const size_t o3 = 3 * (size_t)lo;
-    cudaError_t e = cudaMemcpyAsync(g->d_a + o3, x0 + o3, sizeof(double) * 3 * (size_t)n, cudaMemcpyHostToDevice, s);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(g->d_b + o3, vb + o3, sizeof(double) * 3 * (size_t)n, cudaMemcpyHostToDevice, s);
-    const double* dref = g->d_ref;
+    cudaError_t e = cudaMemcpyAsync(g->d_a.p + o3, x0 + o3, sizeof(double) * 3 * (size_t)n, cudaMemcpyHostToDevice, s);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(g->d_b.p + o3, vb + o3, sizeof(double) * 3 * (size_t)n, cudaMemcpyHostToDevice, s);
+    const double* dref = g->d_ref.p;
     if (!traj || per_instance)
     {
       const size_t per = traj ? 3 * (size_t)ncols : 3;  // doubles of reference data per instance
-      dref = g->d_ref + per * (size_t)lo;
+      dref = g->d_ref.p + per * (size_t)lo;
       if (e == cudaSuccess)
-        e = cudaMemcpyAsync(g->d_ref + per * (size_t)lo, ref + per * (size_t)lo, sizeof(double) * per * (size_t)n, cudaMemcpyHostToDevice, s);
+        e = cudaMemcpyAsync(g->d_ref.p + per * (size_t)lo, ref + per * (size_t)lo, sizeof(double) * per * (size_t)n, cudaMemcpyHostToDevice, s);
     }
     else if (copy_shared_ref && e == cudaSuccess)
-      e = cudaMemcpyAsync(g->d_ref, ref, sizeof(double) * ref_doubles, cudaMemcpyHostToDevice, s);
+      e = cudaMemcpyAsync(g->d_ref.p, ref, sizeof(double) * ref_doubles, cudaMemcpyHostToDevice, s);
     if (e != cudaSuccess) return fail(EB_ERR_CUDA, std::string("eb_dwa_control_host: ") + cudaGetErrorString(e));
-    eb_status r = traj ? eb_dwa_control_traj_dev(g, c, d, g->d_a + o3, g->d_b + o3, dref, ncols, per_instance, dt_ref, n,
-                                                 g->d_out + lo, g->d_u + o3, g->d_cost + lo) :
-                         eb_dwa_control_twist_dev(g, c, d, g->d_a + o3, g->d_b + o3, dref, n, g->d_out + lo, g->d_u + o3,
-                                                  g->d_cost + lo);
+    eb_status r = traj ? eb_dwa_control_traj_dev(g, c, d, g->d_a.p + o3, g->d_b.p + o3, dref, ncols, per_instance, dt_ref, n,
+                                                 g->d_out.p + lo, g->d_u.p + o3, g->d_cost.p + lo) :
+                         eb_dwa_control_twist_dev(g, c, d, g->d_a.p + o3, g->d_b.p + o3, dref, n, g->d_out.p + lo, g->d_u.p + o3,
+                                                  g->d_cost.p + lo);
     if (r != EB_OK) return r;
-    e = cudaMemcpyAsync(found + lo, g->d_out + lo, sizeof(int) * (size_t)n, cudaMemcpyDeviceToHost, s);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(u_opt + o3, g->d_u + o3, sizeof(double) * 3 * (size_t)n, cudaMemcpyDeviceToHost, s);
+    e = cudaMemcpyAsync(found + lo, g->d_out.p + lo, sizeof(int) * (size_t)n, cudaMemcpyDeviceToHost, s);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(u_opt + o3, g->d_u.p + o3, sizeof(double) * 3 * (size_t)n, cudaMemcpyDeviceToHost, s);
     if (e == cudaSuccess && min_cost)
-      e = cudaMemcpyAsync(min_cost + lo, g->d_cost + lo, sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, s);
+      e = cudaMemcpyAsync(min_cost + lo, g->d_cost.p + lo, sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, s);
     if (e != cudaSuccess) return fail(EB_ERR_CUDA, std::string("eb_dwa_control_host: ") + cudaGetErrorString(e));
     return EB_OK;
   };
@@ -2644,13 +2702,12 @@ struct eb_grid_batch
   std::vector<eb::GridView> views;
   std::vector<size_t> slot;  // bytes of the arena reserved for each instance's map
   int unmapped = 0;
-  eb::GridView* d_views = nullptr;
+  DevScratch<eb::GridView> d_views{ "eb_grid_batch::d_views" };
   signed char* d_arena = nullptr;
   signed char* d_retired = nullptr;  // the arena before the last relayout, read by that set call's copy kernel
-  // set call: descriptors (pinned, one upload per call) and the _host call's packed cells
-  eb::MapCopy* h_copies = nullptr;
-  eb::MapCopy* d_copies = nullptr;
-  cudaEvent_t staged = nullptr;  // the last upload out of h_copies has been made
+  // set call: descriptors (one upload per call) and the _host call's packed cells
+  Pinned<eb::MapCopy> copies{ "eb_grid_batch::copies" };
+  cudaEvent_t staged = nullptr;  // the last upload out of the pinned records has been made
   // eb_control_safe_batch_*: recorded on the grid batch's stream before a tick (maps_ready) and on the controller's
   // stream after it (ticked); the next set call waits for the last tick before it writes or frees an arena
   cudaEvent_t maps_ready = nullptr;
@@ -2658,20 +2715,13 @@ struct eb_grid_batch
   // eb_set_map_targets_from_grid_batch: this handle (unique per process) and, per map, how often a set call replaced it
   unsigned long long serial = 0;
   std::vector<unsigned long long> map_serial;
-  eb::BandCopy* h_bands = nullptr;  // eb_grid_batch_set_rows_*: pinned band records, uploaded like h_copies
-  eb::BandCopy* d_bands = nullptr;
-  signed char* h_cells = nullptr;
-  signed char* d_cells = nullptr;
-  size_t cells_bytes = 0;
-  // staging of the _host checks (grid_reserve)
-  double* d_a = nullptr;
-  double* d_b = nullptr;
-  double* d_u = nullptr;
-  double* d_cost = nullptr;
-  double* d_ref = nullptr;
-  size_t ref_cap = 0;
-  int* d_out = nullptr;
-  int cap = 0;
+  // eb_grid_batch_set_rows_*: band records, uploaded like the copies
+  Pinned<eb::BandCopy> bands{ "eb_grid_batch::bands" };
+  Pinned<signed char> cells{ "eb_grid_batch::cells" };
+  // staging of the _host checks, as eb_grid's
+  DevScratch<double> d_a{ "eb_grid_batch::d_a" }, d_b{ "eb_grid_batch::d_b" }, d_u{ "eb_grid_batch::d_u" };
+  DevScratch<double> d_cost{ "eb_grid_batch::d_cost" }, d_ref{ "eb_grid_batch::d_ref" };
+  DevScratch<int> d_out{ "eb_grid_batch::d_out" };
 };
 
 namespace
@@ -2688,12 +2738,12 @@ eb_status grid_batch_set(eb_grid_batch* g, const signed char* const* cells, cons
   const int B = g->B;
   EB_CUDA(cudaSetDevice(g->device));
   if (g->ticked) EB_CUDA(cudaStreamWaitEvent(g->stream, g->ticked, 0));  // a safe control tick may still read the maps
-  if (!g->d_views)
+  if (!g->staged)
   {
-    EB_CUDA(cudaMalloc(&g->d_views, sizeof(eb::GridView) * (size_t)B));
-    EB_CUDA(cudaHostAlloc(&g->h_copies, sizeof(eb::MapCopy) * (size_t)B, cudaHostAllocDefault));
-    EB_CUDA(cudaMalloc(&g->d_copies, sizeof(eb::MapCopy) * (size_t)B));
-    EB_CUDA(cudaEventCreateWithFlags(&g->staged, cudaEventDisableTiming));
+    eb_status st = g->d_views.reserve(B);
+    if (st == EB_OK) st = g->copies.reserve(B);
+    if (st != EB_OK) return st;
+    EB_CUDA(cudaEventCreateWithFlags(&g->staged, cudaEventDisableTiming));  // last: it marks the block as complete
   }
   bool relayout = false;
   for (int i = 0; i < B && !relayout; i++)
@@ -2719,7 +2769,7 @@ eb_status grid_batch_set(eb_grid_batch* g, const signed char* const* cells, cons
     }
     EB_CUDA(cudaMalloc(&arena, total));
   }
-  cudaError_t e = cudaEventSynchronize(g->staged);  // the previous call's upload out of h_copies is done
+  cudaError_t e = cudaEventSynchronize(g->staged);  // the previous call's upload out of the pinned records is done
   std::vector<eb::GridView> views = g->views;
   int k = 0;
   size_t off = 0;
@@ -2730,21 +2780,21 @@ eb_status grid_batch_set(eb_grid_batch* g, const signed char* const* cells, cons
     if (!(update && !update[i]))
     {
       views[i] = eb::GridView{ dst, xsize[i], ysize[i], resolution[i], origin[2 * i + 0], origin[2 * i + 1] };
-      g->h_copies[k++] = eb::MapCopy{ cells[i], views[i], i };
+      g->copies.h[k++] = eb::MapCopy{ cells[i], views[i], i };
     }
     else if (relayout && views[i].data)
     {
       const signed char* src = views[i].data;
       views[i].data = dst;
-      g->h_copies[k++] = eb::MapCopy{ src, views[i], i };
+      g->copies.h[k++] = eb::MapCopy{ src, views[i], i };
     }
   }
   if (e == cudaSuccess)
-    e = cudaMemcpyAsync(g->d_copies, g->h_copies, sizeof(eb::MapCopy) * (size_t)k, cudaMemcpyHostToDevice, g->stream);
+    e = cudaMemcpyAsync(g->copies.d, g->copies.h, sizeof(eb::MapCopy) * (size_t)k, cudaMemcpyHostToDevice, g->stream);
   if (e == cudaSuccess) e = cudaEventRecord(g->staged, g->stream);
   if (e == cudaSuccess)
   {
-    eb::map_copy_kernel<<<k, 256, 0, g->stream>>>(g->d_copies, g->d_views);
+    eb::map_copy_kernel<<<k, 256, 0, g->stream>>>(g->copies.d, g->d_views.p);
     e = cudaGetLastError();
   }
   if (e != cudaSuccess)
@@ -2803,7 +2853,7 @@ eb_status grid_batch_params(const eb_grid_batch* g, const eb_collision* c, int p
     return fail(EB_ERR_INVALID_ARGUMENT, "eb_grid_batch: " + std::to_string(g->unmapped) + " instance(s) have no map yet");
   p->occupied_threshold = c->occupied_threshold;
   p->B = per * g->B;
-  *m = eb::MapSet{ g->d_views, per, c->boundary_radius, c->boundary_radius + c->obstacle_threshold, c->search_radius };
+  *m = eb::MapSet{ g->d_views.p, per, c->boundary_radius, c->boundary_radius + c->obstacle_threshold, c->search_radius };
   return EB_OK;
 }
 
@@ -2855,25 +2905,12 @@ void eb_grid_batch_destroy(eb_grid_batch* g)
   cudaSetDevice(g->device);
   if (g->staged) cudaEventSynchronize(g->staged);
   if (g->ticked) cudaEventSynchronize(g->ticked);
-  cudaFree(g->d_views);
   cudaFree(g->d_arena);
   cudaFree(g->d_retired);
-  cudaFreeHost(g->h_copies);
-  cudaFree(g->d_copies);
-  cudaFreeHost(g->h_bands);
-  cudaFree(g->d_bands);
-  cudaFreeHost(g->h_cells);
-  cudaFree(g->d_cells);
-  cudaFree(g->d_a);
-  cudaFree(g->d_b);
-  cudaFree(g->d_u);
-  cudaFree(g->d_cost);
-  cudaFree(g->d_ref);
-  cudaFree(g->d_out);
   if (g->staged) cudaEventDestroy(g->staged);
   if (g->maps_ready) cudaEventDestroy(g->maps_ready);
   if (g->ticked) cudaEventDestroy(g->ticked);
-  delete g;
+  delete g;  // the staging members free themselves here
 }
 
 eb_status eb_grid_batch_set_stream(eb_grid_batch* g, void* s)
@@ -2905,36 +2942,10 @@ eb_status eb_grid_batch_set_maps_host(eb_grid_batch* g, const signed char* const
   int n = 0;
   eb_status st = grid_batch_check_maps(g, cells, xsize, ysize, resolution, origin, update, "eb_grid_batch_set_maps_host", &n);
   if (st != EB_OK || n == 0) return st;
-  // the flagged maps are packed into one pinned buffer (16-byte aligned offsets) and copied with one cudaMemcpyAsync
-  std::vector<size_t> off((size_t)g->B, 0);
-  size_t total = 0;
-  for (int i = 0; i < g->B; i++)
-  {
-    if (update && !update[i]) continue;
-    off[i] = total;
-    total += ((size_t)xsize[i] * ysize[i] + 15) & ~(size_t)15;
-  }
   EB_CUDA(cudaSetDevice(g->device));
-  EB_CUDA(cudaStreamSynchronize(g->stream));  // no earlier copy still reads the staging buffers
-  if (total > g->cells_bytes)
-  {
-    cudaFreeHost(g->h_cells);
-    cudaFree(g->d_cells);
-    g->h_cells = nullptr;
-    g->d_cells = nullptr;
-    g->cells_bytes = 0;
-    EB_CUDA(cudaHostAlloc(&g->h_cells, total, cudaHostAllocDefault));
-    EB_CUDA(cudaMalloc(&g->d_cells, total));
-    g->cells_bytes = total;
-  }
-  std::vector<const signed char*> dptr((size_t)g->B, nullptr);
-  for (int i = 0; i < g->B; i++)
-    if (!(update && !update[i]))
-    {
-      std::memcpy(g->h_cells + off[i], cells[i], (size_t)xsize[i] * ysize[i]);
-      dptr[i] = g->d_cells + off[i];
-    }
-  EB_CUDA(cudaMemcpyAsync(g->d_cells, g->h_cells, total, cudaMemcpyHostToDevice, g->stream));
+  std::vector<const signed char*> dptr;
+  st = pack_flagged(g->cells, g->stream, g->B, update, cells, [&](int i) { return (size_t)xsize[i] * ysize[i]; }, &dptr);
+  if (st != EB_OK) return st;
   st = grid_batch_set(g, dptr.data(), xsize, ysize, resolution, origin, update, n);
   if (st != EB_OK) return st;
   EB_CUDA(cudaStreamSynchronize(g->stream));
@@ -2973,11 +2984,8 @@ eb_status grid_batch_set_rows(eb_grid_batch* g, const signed char* const* rows, 
 {
   if (n == 0) return EB_OK;
   EB_CUDA(cudaSetDevice(g->device));
-  if (!g->h_bands)
-  {
-    EB_CUDA(cudaHostAlloc(&g->h_bands, sizeof(eb::BandCopy) * (size_t)g->B, cudaHostAllocDefault));
-    EB_CUDA(cudaMalloc(&g->d_bands, sizeof(eb::BandCopy) * (size_t)g->B));
-  }
+  const eb_status st = g->bands.reserve(g->B);
+  if (st != EB_OK) return st;
   EB_CUDA(cudaEventSynchronize(g->staged));  // the previous upload out of the pinned records is done
   int k = 0;
   for (int i = 0; i < g->B; i++)
@@ -2985,13 +2993,13 @@ eb_status grid_batch_set_rows(eb_grid_batch* g, const signed char* const* rows, 
     if ((update && !update[i]) || row_count[i] == 0) continue;
     const eb::GridView& v = g->views[i];
     signed char* dst = const_cast<signed char*>(v.data) + (size_t)row_begin[i] * v.xsize;
-    g->h_bands[k++] = eb::BandCopy{ rows[i], dst, (size_t)row_count[i] * v.xsize };
+    g->bands.h[k++] = eb::BandCopy{ rows[i], dst, (size_t)row_count[i] * v.xsize };
   }
   // the records go up before the wait for the last tick, so the next call's wait on `staged` does not wait for it
-  EB_CUDA(cudaMemcpyAsync(g->d_bands, g->h_bands, sizeof(eb::BandCopy) * (size_t)k, cudaMemcpyHostToDevice, g->stream));
+  EB_CUDA(cudaMemcpyAsync(g->bands.d, g->bands.h, sizeof(eb::BandCopy) * (size_t)k, cudaMemcpyHostToDevice, g->stream));
   EB_CUDA(cudaEventRecord(g->staged, g->stream));
   if (g->ticked) EB_CUDA(cudaStreamWaitEvent(g->stream, g->ticked, 0));  // a tick or target call may still read the maps
-  eb::band_copy_kernel<<<k, 256, 0, g->stream>>>(g->d_bands);
+  eb::band_copy_kernel<<<k, 256, 0, g->stream>>>(g->bands.d);
   EB_CUDA(cudaGetLastError());
   g->launches += 1;
   return EB_OK;
@@ -3017,37 +3025,12 @@ eb_status eb_grid_batch_set_rows_host(eb_grid_batch* g, const signed char* const
   int n = 0;
   eb_status st = grid_batch_check_rows(g, rows, row_begin, row_count, update, "eb_grid_batch_set_rows_host", &n);
   if (st != EB_OK || n == 0) return st;
-  // the bands are packed into the set call's pinned buffer (16-byte aligned offsets) and copied with one
-  // cudaMemcpyAsync
-  std::vector<size_t> off((size_t)g->B, 0);
-  size_t total = 0;
-  for (int i = 0; i < g->B; i++)
-  {
-    if ((update && !update[i]) || row_count[i] == 0) continue;
-    off[i] = total;
-    total += ((size_t)row_count[i] * g->views[i].xsize + 15) & ~(size_t)15;
-  }
+  // the bands go through the set call's pinned buffer
   EB_CUDA(cudaSetDevice(g->device));
-  EB_CUDA(cudaStreamSynchronize(g->stream));  // no earlier copy still reads the staging buffers
-  if (total > g->cells_bytes)
-  {
-    cudaFreeHost(g->h_cells);
-    cudaFree(g->d_cells);
-    g->h_cells = nullptr;
-    g->d_cells = nullptr;
-    g->cells_bytes = 0;
-    EB_CUDA(cudaHostAlloc(&g->h_cells, total, cudaHostAllocDefault));
-    EB_CUDA(cudaMalloc(&g->d_cells, total));
-    g->cells_bytes = total;
-  }
-  std::vector<const signed char*> dptr((size_t)g->B, nullptr);
-  for (int i = 0; i < g->B; i++)
-    if (!(update && !update[i]) && row_count[i] > 0)
-    {
-      std::memcpy(g->h_cells + off[i], rows[i], (size_t)row_count[i] * g->views[i].xsize);
-      dptr[i] = g->d_cells + off[i];
-    }
-  EB_CUDA(cudaMemcpyAsync(g->d_cells, g->h_cells, total, cudaMemcpyHostToDevice, g->stream));
+  std::vector<const signed char*> dptr;
+  st = pack_flagged(g->cells, g->stream, g->B, update, rows,
+                    [&](int i) { return (size_t)row_count[i] * g->views[i].xsize; }, &dptr);
+  if (st != EB_OK) return st;
   st = grid_batch_set_rows(g, dptr.data(), row_begin, row_count, update, n);
   if (st != EB_OK) return st;
   EB_CUDA(cudaStreamSynchronize(g->stream));
@@ -3117,12 +3100,11 @@ eb_status eb_collision_check_batch_host(eb_grid_batch* g, const eb_collision* c,
   if (!poses || !hit) return fail(EB_ERR_INVALID_ARGUMENT, "eb_collision_check_batch_host: NULL argument");
   const int count = p.B;
   EB_CUDA(cudaSetDevice(g->device));
-  st = grid_reserve(g, count);
+  if ((st = g->d_a.reserve(3 * (size_t)count)) != EB_OK || (st = g->d_out.reserve(count)) != EB_OK) return st;
+  EB_CUDA(cudaMemcpyAsync(g->d_a.p, poses, sizeof(double) * 3 * (size_t)count, cudaMemcpyHostToDevice, g->stream));
+  st = eb_collision_check_batch_dev(g, c, g->d_a.p, per, g->d_out.p);
   if (st != EB_OK) return st;
-  EB_CUDA(cudaMemcpyAsync(g->d_a, poses, sizeof(double) * 3 * (size_t)count, cudaMemcpyHostToDevice, g->stream));
-  st = eb_collision_check_batch_dev(g, c, g->d_a, per, g->d_out);
-  if (st != EB_OK) return st;
-  EB_CUDA(cudaMemcpyAsync(hit, g->d_out, sizeof(int) * (size_t)count, cudaMemcpyDeviceToHost, g->stream));
+  EB_CUDA(cudaMemcpyAsync(hit, g->d_out.p, sizeof(int) * (size_t)count, cudaMemcpyDeviceToHost, g->stream));
   EB_CUDA(cudaStreamSynchronize(g->stream));
   return EB_OK;
 }
@@ -3137,13 +3119,15 @@ eb_status eb_validate_control_batch_host(eb_grid_batch* g, const eb_collision* c
   if (!x0 || !u || !valid || dt == 0.0) return fail(EB_ERR_INVALID_ARGUMENT, "eb_validate_control_batch_host: bad arguments");
   const int count = p.B;
   EB_CUDA(cudaSetDevice(g->device));
-  st = grid_reserve(g, count);
+  st = g->d_a.reserve(3 * (size_t)count);
+  if (st == EB_OK) st = g->d_b.reserve(3 * (size_t)count);
+  if (st == EB_OK) st = g->d_out.reserve(count);
   if (st != EB_OK) return st;
-  EB_CUDA(cudaMemcpyAsync(g->d_a, x0, sizeof(double) * 3 * (size_t)count, cudaMemcpyHostToDevice, g->stream));
-  EB_CUDA(cudaMemcpyAsync(g->d_b, u, sizeof(double) * 3 * (size_t)count, cudaMemcpyHostToDevice, g->stream));
-  st = eb_validate_control_batch_dev(g, c, g->d_a, g->d_b, per, dt, horizon, g->d_out);
+  EB_CUDA(cudaMemcpyAsync(g->d_a.p, x0, sizeof(double) * 3 * (size_t)count, cudaMemcpyHostToDevice, g->stream));
+  EB_CUDA(cudaMemcpyAsync(g->d_b.p, u, sizeof(double) * 3 * (size_t)count, cudaMemcpyHostToDevice, g->stream));
+  st = eb_validate_control_batch_dev(g, c, g->d_a.p, g->d_b.p, per, dt, horizon, g->d_out.p);
   if (st != EB_OK) return st;
-  EB_CUDA(cudaMemcpyAsync(valid, g->d_out, sizeof(int) * (size_t)count, cudaMemcpyDeviceToHost, g->stream));
+  EB_CUDA(cudaMemcpyAsync(valid, g->d_out.p, sizeof(int) * (size_t)count, cudaMemcpyDeviceToHost, g->stream));
   EB_CUDA(cudaStreamSynchronize(g->stream));
   return EB_OK;
 }
@@ -3200,26 +3184,23 @@ static eb_status dwa_batch_host(eb_grid_batch* g, const eb_collision* c, const e
   const int B = g->B;
   const size_t ref_doubles = traj ? 3 * (size_t)ncols * (per_instance ? (size_t)B : 1) : 3 * (size_t)B;
   EB_CUDA(cudaSetDevice(g->device));
-  eb_status st = grid_reserve(g, B);
+  eb_status st = g->d_a.reserve(3 * (size_t)B);
+  if (st == EB_OK) st = g->d_b.reserve(3 * (size_t)B);
+  if (st == EB_OK) st = g->d_u.reserve(3 * (size_t)B);
+  if (st == EB_OK) st = g->d_cost.reserve(B);
+  if (st == EB_OK) st = g->d_out.reserve(B);
+  if (st == EB_OK) st = g->d_ref.reserve(ref_doubles);
   if (st != EB_OK) return st;
-  if (ref_doubles > g->ref_cap)
-  {
-    cudaFree(g->d_ref);
-    g->d_ref = nullptr;
-    g->ref_cap = 0;
-    EB_CUDA(cudaMalloc(&g->d_ref, sizeof(double) * ref_doubles));
-    g->ref_cap = ref_doubles;
-  }
-  EB_CUDA(cudaMemcpyAsync(g->d_a, x0, sizeof(double) * 3 * (size_t)B, cudaMemcpyHostToDevice, g->stream));
-  EB_CUDA(cudaMemcpyAsync(g->d_b, vb, sizeof(double) * 3 * (size_t)B, cudaMemcpyHostToDevice, g->stream));
-  EB_CUDA(cudaMemcpyAsync(g->d_ref, ref, sizeof(double) * ref_doubles, cudaMemcpyHostToDevice, g->stream));
-  st = traj ? eb_dwa_control_traj_batch_dev(g, c, d, g->d_a, g->d_b, g->d_ref, ncols, per_instance, dt_ref, g->d_out,
-                                            g->d_u, g->d_cost) :
-              eb_dwa_control_twist_batch_dev(g, c, d, g->d_a, g->d_b, g->d_ref, g->d_out, g->d_u, g->d_cost);
+  EB_CUDA(cudaMemcpyAsync(g->d_a.p, x0, sizeof(double) * 3 * (size_t)B, cudaMemcpyHostToDevice, g->stream));
+  EB_CUDA(cudaMemcpyAsync(g->d_b.p, vb, sizeof(double) * 3 * (size_t)B, cudaMemcpyHostToDevice, g->stream));
+  EB_CUDA(cudaMemcpyAsync(g->d_ref.p, ref, sizeof(double) * ref_doubles, cudaMemcpyHostToDevice, g->stream));
+  st = traj ? eb_dwa_control_traj_batch_dev(g, c, d, g->d_a.p, g->d_b.p, g->d_ref.p, ncols, per_instance, dt_ref,
+                                            g->d_out.p, g->d_u.p, g->d_cost.p) :
+              eb_dwa_control_twist_batch_dev(g, c, d, g->d_a.p, g->d_b.p, g->d_ref.p, g->d_out.p, g->d_u.p, g->d_cost.p);
   if (st != EB_OK) return st;
-  EB_CUDA(cudaMemcpyAsync(found, g->d_out, sizeof(int) * (size_t)B, cudaMemcpyDeviceToHost, g->stream));
-  EB_CUDA(cudaMemcpyAsync(u_opt, g->d_u, sizeof(double) * 3 * (size_t)B, cudaMemcpyDeviceToHost, g->stream));
-  if (min_cost) EB_CUDA(cudaMemcpyAsync(min_cost, g->d_cost, sizeof(double) * (size_t)B, cudaMemcpyDeviceToHost, g->stream));
+  EB_CUDA(cudaMemcpyAsync(found, g->d_out.p, sizeof(int) * (size_t)B, cudaMemcpyDeviceToHost, g->stream));
+  EB_CUDA(cudaMemcpyAsync(u_opt, g->d_u.p, sizeof(double) * 3 * (size_t)B, cudaMemcpyDeviceToHost, g->stream));
+  if (min_cost) EB_CUDA(cudaMemcpyAsync(min_cost, g->d_cost.p, sizeof(double) * (size_t)B, cudaMemcpyDeviceToHost, g->stream));
   EB_CUDA(cudaStreamSynchronize(g->stream));
   return EB_OK;
 }
@@ -3398,10 +3379,11 @@ struct eb_map_target
   cudaStream_t stream = nullptr;
   eb_phik_plan* plan = nullptr;
   double* d_lut = nullptr;       // entropy of the 256 int8 patterns
-  double* d_phi = nullptr;       // un-normalised density [ysize][xsize]: written by the two-kernel route or on demand
+  // un-normalised density [ysize][xsize]: written by the two-kernel route or on demand
+  DevScratch<double> d_phi{ "eb_map_target::d_phi" };
   const signed char* last_cells = nullptr;  // device cells of the last execute (must stay alive for a later density request)
   bool density_valid = false;    // d_phi holds the density of last_cells
-  signed char* d_cells = nullptr;  // staging for the _host call
+  DevScratch<signed char> d_cells{ "eb_map_target::d_cells" };  // staging for the _host call
   double *d_phik = nullptr, *d_sum = nullptr;
   long long launches = 0;
 };
@@ -3462,8 +3444,6 @@ void eb_map_target_destroy(eb_map_target* m)
   cudaSetDevice(m->device);
   eb_phik_plan_destroy(m->plan);
   cudaFree(m->d_lut);
-  cudaFree(m->d_phi);
-  cudaFree(m->d_cells);
   cudaFree(m->d_phik);
   cudaFree(m->d_sum);
   delete m;
@@ -3482,7 +3462,7 @@ double* eb_map_target_density_dev(eb_map_target* m)
 {
   // the fused execute never writes the density: materialise it from the last execute's cells on demand
   if (!m || cudaSetDevice(m->device) != cudaSuccess || map_density(m) != EB_OK) return nullptr;
-  return m->d_phi;
+  return m->d_phi.p;
 }
 
 eb_status eb_map_target_extent(const eb_map_target* m, double* lx, double* ly)
@@ -3499,11 +3479,12 @@ static eb_status map_density(eb_map_target* m)
   if (m->density_valid) return EB_OK;
   if (!m->last_cells) return fail(EB_ERR_INVALID_ARGUMENT, "map target: no execute yet");
   const long long cells = (long long)m->xsize * m->ysize;
-  if (!m->d_phi) EB_CUDA(cudaMalloc(&m->d_phi, sizeof(double) * (size_t)cells));
+  const eb_status st = m->d_phi.reserve((size_t)cells);
+  if (st != EB_OK) return st;
   int sms = 148;
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, m->device);
   const int grid = (int)std::min<long long>((cells / 512 + 7) / 8 + 1, (long long)sms * 8);  // 8 warps per CTA, 512 cells per warp iteration
-  eb::entropy_density_kernel<<<grid, 256, 0, m->stream>>>(m->last_cells, cells, m->d_lut, m->d_phi);
+  eb::entropy_density_kernel<<<grid, 256, 0, m->stream>>>(m->last_cells, cells, m->d_lut, m->d_phi.p);
   m->launches += 1;
   EB_CUDA(cudaGetLastError());
   m->density_valid = true;
@@ -3534,7 +3515,7 @@ eb_status eb_map_target_execute_dev(eb_map_target* m, const signed char* cells_d
   }
   const eb_status st = map_density(m);
   if (st != EB_OK) return st;
-  return eb_phik_execute_dev(m->plan, m->d_phi, phik_dev, phi_sum_dev);
+  return eb_phik_execute_dev(m->plan, m->d_phi.p, phik_dev, phi_sum_dev);
 }
 
 eb_status eb_map_target_execute_host(eb_map_target* m, const signed char* cells, double* phik, double* phi_sum)
@@ -3543,9 +3524,10 @@ eb_status eb_map_target_execute_host(eb_map_target* m, const signed char* cells,
   if (!m || !cells || !phik) return fail(EB_ERR_INVALID_ARGUMENT, "eb_map_target_execute_host: NULL argument");
   EB_CUDA(cudaSetDevice(m->device));
   const size_t n = (size_t)m->xsize * m->ysize;
-  if (!m->d_cells) EB_CUDA(cudaMalloc(&m->d_cells, n));
-  EB_CUDA(cudaMemcpyAsync(m->d_cells, cells, n, cudaMemcpyHostToDevice, m->stream));
-  eb_status st = eb_map_target_execute_dev(m, m->d_cells, m->d_phik, m->d_sum);
+  eb_status st = m->d_cells.reserve(n);
+  if (st != EB_OK) return st;
+  EB_CUDA(cudaMemcpyAsync(m->d_cells.p, cells, n, cudaMemcpyHostToDevice, m->stream));
+  st = eb_map_target_execute_dev(m, m->d_cells.p, m->d_phik, m->d_sum);
   if (st != EB_OK) return st;
   EB_CUDA(cudaMemcpyAsync(phik, m->d_phik, sizeof(double) * m->nb * m->nb, cudaMemcpyDeviceToHost, m->stream));
   if (phi_sum) EB_CUDA(cudaMemcpyAsync(phi_sum, m->d_sum, sizeof(double), cudaMemcpyDeviceToHost, m->stream));
@@ -3583,23 +3565,16 @@ eb_status eb_set_target_gaussians_batch(eb_controller* c, int max_n, const int* 
   EB_CUDA(cudaSetDevice(c->cfg.device));
   eb_status st = ensure_per_inst(c);
   if (st != EB_OK) return st;
-  if (max_n > c->gmax)
-  {
-    cudaFree(c->d_gmu);
-    cudaFree(c->d_gsig);
-    c->d_gmu = c->d_gsig = nullptr;
-    c->gmax = 0;
-    const size_t gb = sizeof(double) * 2 * (size_t)max_n * c->B;
-    EB_CUDA(cudaMalloc(&c->d_gmu, gb));
-    EB_CUDA(cudaMalloc(&c->d_gsig, gb));
-  }
+  const size_t gd = 2 * (size_t)max_n * c->B;
+  if (gd > c->d_gmu.cap || gd > c->d_gsig.cap) c->gmax = 0;  // rows of neither buffer until both have grown
+  if ((st = c->d_gmu.reserve(gd)) != EB_OK || (st = c->d_gsig.reserve(gd)) != EB_OK) return st;
   c->gmax = std::max(c->gmax, max_n);
   // the caller's [B][max_n][2] rows into the [B][gmax][2] buffers
   const size_t row = sizeof(double) * 2 * (size_t)max_n, pitch = sizeof(double) * 2 * (size_t)c->gmax;
   if (max_n > 0)
   {
-    EB_CUDA(cudaMemcpy2DAsync(c->d_gmu, pitch, mu, row, row, c->B, cudaMemcpyHostToDevice, c->stream));
-    EB_CUDA(cudaMemcpy2DAsync(c->d_gsig, pitch, sigma, row, row, c->B, cudaMemcpyHostToDevice, c->stream));
+    EB_CUDA(cudaMemcpy2DAsync(c->d_gmu.p, pitch, mu, row, row, c->B, cudaMemcpyHostToDevice, c->stream));
+    EB_CUDA(cudaMemcpy2DAsync(c->d_gsig.p, pitch, sigma, row, row, c->B, cudaMemcpyHostToDevice, c->stream));
   }
   EB_CUDA(cudaMemcpyAsync(c->d_gcount, counts, sizeof(int) * (size_t)c->B, cudaMemcpyHostToDevice, c->stream));
   EB_CUDA(cudaStreamSynchronize(c->stream));  // the caller's buffers may go once this returns
@@ -3657,19 +3632,19 @@ eb_status map_targets_check(const eb_controller* c, const signed char* const* ce
 // the descriptors, arrival counters and resident grid of map_target_batch_kernel, allocated at the first call
 eb_status ensure_map_batch(eb_controller* c)
 {
-  if (c->h_mb_desc) return EB_OK;
+  if (c->mb_staged) return EB_OK;
   const int B = c->B;
-  EB_CUDA(cudaHostAlloc(&c->h_mb_desc, sizeof(eb::MapBatchDesc) * (size_t)B, cudaHostAllocDefault));
-  EB_CUDA(cudaMalloc(&c->d_mb_desc, sizeof(eb::MapBatchDesc) * (size_t)B));
-  EB_CUDA(cudaMalloc(&c->d_mb_arrive, sizeof(unsigned) * (size_t)B));
-  EB_CUDA(cudaMemset(c->d_mb_arrive, 0, sizeof(unsigned) * (size_t)B));
-  EB_CUDA(cudaEventCreateWithFlags(&c->mb_staged, cudaEventDisableTiming));
+  eb_status st = c->mb_desc.reserve(B);
+  if (st == EB_OK) st = c->d_mb_arrive.reserve(B);
+  if (st != EB_OK) return st;
+  EB_CUDA(cudaMemset(c->d_mb_arrive.p, 0, sizeof(unsigned) * (size_t)B));
   for (auto kernel : { eb::map_target_batch_kernel<false>, eb::map_target_batch_kernel<true> })
     EB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)eb::kMbSmemBytes));
   int per_sm = 0, sms = 0;
   EB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, eb::map_target_batch_kernel<false>, eb::kMbThreads,
                                                         eb::kMbSmemBytes));
   EB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->cfg.device));
+  EB_CUDA(cudaEventCreateWithFlags(&c->mb_staged, cudaEventDisableTiming));  // last: it marks the block as complete
   c->mb_grid = std::max(1, per_sm * sms);
   return EB_OK;
 }
@@ -3690,20 +3665,14 @@ eb_status map_targets_batch(eb_controller* c, const signed char* const* cells, c
   if (n == B) c->frames_set = true;
   if (n == 0) return EB_OK;
   if ((st = ensure_map_batch(c)) != EB_OK) return st;
-  if (units > c->mb_slot_units)
-  {
-    cudaFree(c->d_mb_slots);  // synchronises with earlier launches that use it
-    c->d_mb_slots = nullptr;
-    c->mb_slot_units = 0;
-    EB_CUDA(cudaMalloc(&c->d_mb_slots, sizeof(double) * (size_t)c->K * (size_t)units));
-    c->mb_slot_units = units;
-  }
+  // growing frees the old blocks first: that synchronises with earlier launches that use them
+  if ((st = c->d_mb_slots.reserve((size_t)c->K * (size_t)units)) != EB_OK) return st;
   EB_CUDA(cudaEventSynchronize(c->mb_staged));  // the previous call's copy out of the pinned descriptors is done
   int k = 0, u0 = 0;
   for (int i = 0; i < B; i++)
   {
     if (update && !update[i]) continue;
-    eb::MapBatchDesc& d = c->h_mb_desc[k++];
+    eb::MapBatchDesc& d = c->mb_desc.h[k++];
     d.cells = cells[i];
     d.nx = (int)xsize[i];
     d.ny = (int)ysize[i];
@@ -3714,16 +3683,16 @@ eb_status map_targets_batch(eb_controller* c, const signed char* const* cells, c
     d.unit0 = u0;
     u0 += eb::mb_units(d.ny);
   }
-  EB_CUDA(cudaMemcpyAsync(c->d_mb_desc, c->h_mb_desc, sizeof(eb::MapBatchDesc) * (size_t)n, cudaMemcpyHostToDevice,
+  EB_CUDA(cudaMemcpyAsync(c->mb_desc.d, c->mb_desc.h, sizeof(eb::MapBatchDesc) * (size_t)n, cudaMemcpyHostToDevice,
                           c->stream));
   EB_CUDA(cudaEventRecord(c->mb_staged, c->stream));
   eb::MapBatchParams p{};
-  p.desc = c->d_mb_desc;
+  p.desc = c->mb_desc.d;
   p.n = n;
   p.units = (int)units;
   p.nb = c->nb;
-  p.slots = c->d_mb_slots;
-  p.arrive = c->d_mb_arrive;
+  p.slots = c->d_mb_slots.p;
+  p.arrive = c->d_mb_arrive.p;
   p.frames = c->d_frames;
   p.phik = c->d_phik_b;
   p.hist = c->d_hist;
@@ -3761,37 +3730,11 @@ eb_status eb_set_map_targets_batch_host(eb_controller* c, const signed char* con
   long long units = 0;
   eb_status st = map_targets_check(c, cells, xsize, ysize, resolution, update, call, &n, &units);
   if (st != EB_OK) return st;
-  // the flagged maps are packed into one pinned buffer (16-byte aligned offsets) and copied with one cudaMemcpyAsync
-  std::vector<size_t> off((size_t)c->B, 0);
-  size_t total = 0;
-  for (int i = 0; i < c->B; i++)
-  {
-    if (update && !update[i]) continue;
-    off[i] = total;
-    total += ((size_t)xsize[i] * ysize[i] + 15) & ~(size_t)15;
-  }
   EB_CUDA(cudaSetDevice(c->cfg.device));
-  EB_CUDA(cudaStreamSynchronize(c->stream));  // no earlier copy still reads the staging buffers
-  if (total > c->mb_cells_bytes)
-  {
-    cudaFreeHost(c->h_mb_cells);
-    cudaFree(c->d_mb_cells);
-    c->h_mb_cells = nullptr;
-    c->d_mb_cells = nullptr;
-    c->mb_cells_bytes = 0;
-    EB_CUDA(cudaHostAlloc(&c->h_mb_cells, total, cudaHostAllocDefault));
-    EB_CUDA(cudaMalloc(&c->d_mb_cells, total));
-    c->mb_cells_bytes = total;
-  }
-  std::vector<const signed char*> dptr((size_t)c->B, nullptr);
-  for (int i = 0; i < c->B; i++)
-    if (!(update && !update[i]))
-    {
-      std::memcpy(c->h_mb_cells + off[i], cells[i], (size_t)xsize[i] * ysize[i]);
-      dptr[i] = c->d_mb_cells + off[i];
-    }
-  if (total > 0)
-    EB_CUDA(cudaMemcpyAsync(c->d_mb_cells, c->h_mb_cells, total, cudaMemcpyHostToDevice, c->stream));
+  std::vector<const signed char*> dptr;
+  st = pack_flagged(c->mb_cells, c->stream, c->B, update, cells, [&](int i) { return (size_t)xsize[i] * ysize[i]; },
+                    &dptr);
+  if (st != EB_OK) return st;
   st = map_targets_batch(c, dptr.data(), xsize, ysize, resolution, origin, update, call);
   if (st != EB_OK) return st;
   EB_CUDA(cudaStreamSynchronize(c->stream));
@@ -3913,11 +3856,7 @@ eb_status eb_set_map_targets_from_grid_batch(eb_controller* c, eb_grid_batch* g,
   if (work == 0) return EB_OK;
   if (work > 0x7fffffffLL) return fail(EB_ERR_INVALID_ARGUMENT, std::string(call) + ": more than 2^31 - 1 units");
   if ((st = ensure_map_batch(c)) != EB_OK) return st;
-  if (!c->h_mb_kept)
-  {
-    EB_CUDA(cudaHostAlloc(&c->h_mb_kept, sizeof(eb::MapKept) * (size_t)B, cudaHostAllocDefault));
-    EB_CUDA(cudaMalloc(&c->d_mb_kept, sizeof(eb::MapKept) * (size_t)B));
-  }
+  if ((st = c->mb_kept.reserve(B)) != EB_OK) return st;
   if (grown && (st = kept_relayout(c, cap)) != EB_OK) return st;
   if (!g->maps_ready)
   {
@@ -3930,32 +3869,32 @@ eb_status eb_set_map_targets_from_grid_batch(eb_controller* c, eb_grid_batch* g,
   {
     if (run[i].count == 0) continue;
     const eb::GridView& v = g->views[i];
-    c->h_mb_desc[k] = eb::MapBatchDesc{ v.data, (int)v.xsize, (int)v.ysize, v.resolution, v.xmin, v.ymin, i, u0 };
-    c->h_mb_kept[k++] = eb::MapKept{ run[i].first, run[i].count, c->kb_slot0[i] };
+    c->mb_desc.h[k] = eb::MapBatchDesc{ v.data, (int)v.xsize, (int)v.ysize, v.resolution, v.xmin, v.ymin, i, u0 };
+    c->mb_kept.h[k++] = eb::MapKept{ run[i].first, run[i].count, c->kb_slot0[i] };
     u0 += run[i].count;
   }
-  EB_CUDA(cudaMemcpyAsync(c->d_mb_desc, c->h_mb_desc, sizeof(eb::MapBatchDesc) * (size_t)k, cudaMemcpyHostToDevice,
+  EB_CUDA(cudaMemcpyAsync(c->mb_desc.d, c->mb_desc.h, sizeof(eb::MapBatchDesc) * (size_t)k, cudaMemcpyHostToDevice,
                           c->stream));
-  EB_CUDA(cudaMemcpyAsync(c->d_mb_kept, c->h_mb_kept, sizeof(eb::MapKept) * (size_t)k, cudaMemcpyHostToDevice,
+  EB_CUDA(cudaMemcpyAsync(c->mb_kept.d, c->mb_kept.h, sizeof(eb::MapKept) * (size_t)k, cudaMemcpyHostToDevice,
                           c->stream));
   EB_CUDA(cudaEventRecord(c->mb_staged, c->stream));  // before the wait below: the next call's sync does not wait for it
   // after the set and rows calls already enqueued on the grid batch's stream, without a host synchronisation
   EB_CUDA(cudaEventRecord(g->maps_ready, g->stream));
   EB_CUDA(cudaStreamWaitEvent(c->stream, g->maps_ready, 0));
   eb::MapBatchParams p{};
-  p.desc = c->d_mb_desc;
+  p.desc = c->mb_desc.d;
   p.n = k;
   p.units = (int)work;
   p.nb = c->nb;
   p.slots = c->d_kb;
-  p.arrive = c->d_mb_arrive;
+  p.arrive = c->d_mb_arrive.p;
   p.frames = c->d_frames;
   p.phik = c->d_phik_b;
   p.hist = c->d_hist;
   p.hist_cos = c->d_hist_cos;
   p.mem_count = c->d_hist_cos ? c->mem_count : 0;
   p.B = B;
-  p.kept = c->d_mb_kept;
+  p.kept = c->mb_kept.d;
   const int grid = (int)std::min<long long>(work, c->mb_grid);
   eb::map_target_batch_kernel<true><<<grid, eb::kMbThreads, eb::kMbSmemBytes, c->stream>>>(p);
   cudaError_t e = cudaGetLastError();
@@ -4011,35 +3950,12 @@ eb_status eb_control_batch_host(eb_controller* c, const double* bounds, const do
   if (!bounds && !c->frames_set)
     return fail(EB_ERR_INVALID_ARGUMENT, "eb_control_batch_host: bounds NULL before any frame was configured");
   EB_CUDA(cudaSetDevice(c->cfg.device));
-  eb_status st = ensure_per_inst(c);
+  const eb_status st = ensure_per_inst(c);
   if (st != EB_OK) return st;
-  if (bounds)
-    EB_CUDA(cudaMemcpyAsync(c->d_bounds, bounds, sizeof(double) * 4 * (size_t)c->B, cudaMemcpyHostToDevice, c->stream));
-  const double* bd = bounds ? c->d_bounds : nullptr;
-  const bool need_idx = mem_idx && c->mem_count > (long long)c->cfg.batch_size;
-  if (need_idx)
-    EB_CUDA(cudaMemcpyAsync(c->d_mem_idx_in, mem_idx, sizeof(int) * (size_t)c->cfg.batch_size * c->B,
-                            cudaMemcpyHostToDevice, c->stream));
-  // as eb_control_host: page-locked caller buffers of a small batch are read / written in place
-  double *xm = nullptr, *um = nullptr, *mm = nullptr;
-  if (c->B <= zero_copy_max_batch())
-  {
-    xm = c->mapped(x);
-    um = xm ? c->mapped(u0) : nullptr;
-    mm = (um && metric) ? c->mapped(metric) : nullptr;
-  }
-  if (xm && um && (!metric || mm))
-  {
-    st = eb_control_batch_dev(c, bd, xm, need_idx ? c->d_mem_idx_in : nullptr, um, mm);
-    if (st != EB_OK) return st;
-    return check_fault(c);  // synchronises
-  }
-  EB_CUDA(cudaMemcpyAsync(c->d_pose, x, sizeof(double) * 3 * c->B, cudaMemcpyHostToDevice, c->stream));
-  st = eb_control_batch_dev(c, bd, c->d_pose, need_idx ? c->d_mem_idx_in : nullptr, c->d_u0, metric ? c->d_metric : nullptr);
-  if (st != EB_OK) return st;
-  EB_CUDA(cudaMemcpyAsync(u0, c->d_u0, sizeof(double) * 3 * c->B, cudaMemcpyDeviceToHost, c->stream));
-  if (metric) EB_CUDA(cudaMemcpyAsync(metric, c->d_metric, sizeof(double) * c->B, cudaMemcpyDeviceToHost, c->stream));
-  return check_fault(c);  // synchronises
+  const double* bd = bounds ? c->d_bounds.p : nullptr;
+  return control_host(c, bounds, x, mem_idx, u0, metric, [&](const double* xd, const int* idx, double* ud, double* md) {
+    return eb_control_batch_dev(c, bd, xd, idx, ud, md);
+  });
 }
 
 }  // extern "C"
@@ -4077,8 +3993,9 @@ eb_status ensure_safe(eb_controller* c)
 {
   if (c->d_safe_list) return EB_OK;
   const size_t B = (size_t)c->B;
-  EB_CUDA(cudaMalloc(&c->d_safe_branch, sizeof(int) * B));
-  EB_CUDA(cudaMalloc(&c->d_safe_vb, sizeof(double) * 3 * B));
+  eb_status st = c->d_safe_branch.reserve(B);
+  if (st == EB_OK) st = c->d_safe_vb.reserve(3 * B);
+  if (st != EB_OK) return st;
   const bool omni = c->cfg.model == EB_MODEL_OMNI;
   auto kernel = omni ? eb::dwa_fallback_kernel<eb::kModelOmni, false> : eb::dwa_fallback_kernel<eb::kModelSimpleCart, false>;
   auto publishing = omni ? eb::dwa_fallback_kernel<eb::kModelOmni, true> : eb::dwa_fallback_kernel<eb::kModelSimpleCart, true>;
@@ -4259,19 +4176,15 @@ eb_status eb_control_safe_batch_host(eb_controller* c, eb_grid_batch* g, const e
   EB_CUDA(cudaSetDevice(c->cfg.device));
   if ((st = ensure_safe(c)) != EB_OK) return st;
   const size_t B = (size_t)c->B;
-  if (bounds) EB_CUDA(cudaMemcpyAsync(c->d_bounds, bounds, sizeof(double) * 4 * B, cudaMemcpyHostToDevice, c->stream));
-  const bool need_idx = mem_idx && c->mem_count > (long long)c->cfg.batch_size;
-  if (need_idx)
-    EB_CUDA(cudaMemcpyAsync(c->d_mem_idx_in, mem_idx, sizeof(int) * (size_t)c->cfg.batch_size * B,
-                            cudaMemcpyHostToDevice, c->stream));
+  const int* idx = nullptr;
+  if ((st = upload_bounds_idx(c, bounds, mem_idx, &idx)) != EB_OK) return st;
   EB_CUDA(cudaMemcpyAsync(c->d_pose, x, sizeof(double) * 3 * B, cudaMemcpyHostToDevice, c->stream));
-  EB_CUDA(cudaMemcpyAsync(c->d_safe_vb, vb, sizeof(double) * 3 * B, cudaMemcpyHostToDevice, c->stream));
-  st = eb_control_safe_batch_dev(c, g, col, dwa, val_dt, val_horizon, bounds ? c->d_bounds : nullptr, c->d_pose,
-                                 need_idx ? c->d_mem_idx_in : nullptr, c->d_safe_vb, c->d_u0, c->d_safe_branch,
-                                 metric ? c->d_metric : nullptr);
+  EB_CUDA(cudaMemcpyAsync(c->d_safe_vb.p, vb, sizeof(double) * 3 * B, cudaMemcpyHostToDevice, c->stream));
+  st = eb_control_safe_batch_dev(c, g, col, dwa, val_dt, val_horizon, bounds ? c->d_bounds.p : nullptr, c->d_pose, idx,
+                                 c->d_safe_vb.p, c->d_u0, c->d_safe_branch.p, metric ? c->d_metric : nullptr);
   if (st != EB_OK) return st;
   EB_CUDA(cudaMemcpyAsync(u, c->d_u0, sizeof(double) * 3 * B, cudaMemcpyDeviceToHost, c->stream));
-  EB_CUDA(cudaMemcpyAsync(branch, c->d_safe_branch, sizeof(int) * B, cudaMemcpyDeviceToHost, c->stream));
+  EB_CUDA(cudaMemcpyAsync(branch, c->d_safe_branch.p, sizeof(int) * B, cudaMemcpyDeviceToHost, c->stream));
   if (metric) EB_CUDA(cudaMemcpyAsync(metric, c->d_metric, sizeof(double) * B, cudaMemcpyDeviceToHost, c->stream));
   return check_fault(c);  // synchronises
 }
